@@ -6,6 +6,7 @@ and track-pairs/sec).
     python bench.py --impl reference --steps K --warmup W    # the CPU path on the host cores, same config
     python bench.py --config 2|3|4 [--steps K]               # per-family lines of BASELINE configs 2 / 3 / 4
     python bench.py --single-pair                            # config 1: latency of one pair
+    python bench.py --steps K --dump-outputs DIR             # config 5, plus the last timed step's results as DIR/*.npy
 
 A step = one full analysis (strip → slice → gate → pitch → tempo src → prior → tempo nc → hop-64
 IBI pass → bootstraps → result assembly) of a batch of synthetic track pairs of BASELINE config 5
@@ -173,6 +174,43 @@ def audio_seconds(n_pairs: float, pair_sec: float) -> float:
     return n_pairs * pair_sec * (1.0 + NC_SEC_PER_SRC_SEC)
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, results, pair_ids, prefix: str = "") -> None:
+    """Write what the analysis handed its caller, one float64 .npy per field, so that two builds can be compared output
+    for output: the per-pair record (status, tempo / pitch / IBI ratios and CIs, window counts, median BPMs; see
+    parallel.result_record), the analysed durations, and the per-window tempo and per-chunk pitch lists padded with NaN
+    (None and failed pairs are NaN too).  `pair_index` names the pair of every row; above DUMP_MAX_BYTES the rows are a
+    fixed, seeded sample of the pairs."""
+    from nightcore_analyzer import parallel as npar
+    ok = [None if r is None or isinstance(r, Exception) else r for r in results]
+    nan = float("nan")
+
+    def padded(name):
+        rows = [[] if r is None else (getattr(r, name) or []) for r in ok]
+        a = np.full((len(rows), max((len(x) for x in rows), default=0)), nan)
+        for i, x in enumerate(rows):
+            a[i, :len(x)] = [nan if v is None else v for v in x]
+        return a
+
+    arrays = {"pair_index": np.asarray(pair_ids, dtype=np.float64),
+              "records": npar.records_of(results),
+              "durations": np.array([[nan, nan] if r is None else
+                                     [nan if r.nc_duration is None else r.nc_duration,
+                                      nan if r.src_duration is None else r.src_duration] for r in ok]).reshape(-1, 2)}
+    for name in ("src_tempos_raw", "nc_tempos_raw", "src_pitches_raw", "nc_pitches_raw"):
+        arrays[name] = padded(name)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        n = len(ok)
+        keep = np.sort(np.random.default_rng(0).choice(n, int(n * DUMP_MAX_BYTES / total), replace=False))
+        arrays = {k: a[keep] for k, a in arrays.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), a)
+
+
 def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
@@ -326,7 +364,7 @@ def run_gpu(args):
     if args.no_pageable:
         ms_page, windows_p = None, 0
     else:
-        ms_page, _, stats_p = time_e2e(pairs_np, 1, max(1, min(args.steps, 2)))
+        ms_page, _, stats_p = time_e2e(pairs_np, 1, args.steps)
         windows_p = stats_p["windows"]
 
     # ---- max over ranks, totals over ranks
@@ -401,6 +439,9 @@ def run_gpu(args):
                                     "pairs_per_sec": n / wall, "audio_sec_per_sec": audio_seconds(n / wall, args.pair_sec),
                                     "sample": arm.sample_text() + f"; one step, {wall:.1f} s wall"}
         print(json.dumps(line), flush=True)
+    if args.dump_outputs:
+        # `res` is the last timed step of the resident path, the one `value` measures
+        dump_outputs(args.dump_outputs, res, my_ids, f"rank{rank}_" if world > 1 else "")
     if world > 1:
         dist.destroy_process_group()
 
@@ -560,7 +601,13 @@ def main():
     ap.add_argument("--cpu-procs", type=int, default=0)
     ap.add_argument("--family-pairs", type=int, default=0, help="pairs of the --config 3 / 4 family lines")
     ap.add_argument("--single-pair", action="store_true", help="config 1: latency of one pair through pipeline.run_arrays")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step as DIR/<name>.npy (config 5 GPU run)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.single_pair or args.impl != "graft" or args.config != 5):
+        ap.error("--dump-outputs applies to the config 5 GPU run")
     if args.single_pair:
         return run_single_pair(args)
     if args.impl == "reference":

@@ -1,7 +1,6 @@
 """The reference's own control flow (its io/tempo/pitch/xcorr/consensus/pipeline modules run UNMODIFIED over the
 librosa shim, tests/golden/make_pipeline_golden.py → tests/golden/pipeline_golden.json) against
-  * the CPU oracle port (oracle/pipeline_port.py)            — CPU test, pins the port to the reference's flow;
-  * the reference modules re-run live when /root/reference exists — CPU test, build container only;
+  * the CPU oracle port (oracle/pipeline_port.py)            — CPU tests, pin the port to the reference's flow;
   * the CUDA product (nightcore_analyzer)                    — GPU tests, through the drop-in API.
 Integer-derived outputs (quantised BPMs, chunk Hz, bootstrap ratios/CIs, IBI ratio) are compared bit-exact via
 float.hex; the xcorr quality (float32 cosine) within 1e-5."""
@@ -69,17 +68,15 @@ def test_port_xcorr_and_align_match_reference_flow(g):
     assert off == unhex(g["align_D"]["offset_sec"]) and float(speed) == unhex(g["align_D"]["speed"])
 
 
-def test_golden_is_reproducible_from_the_reference(g):
-    """Build container only: re-run the reference's estimate_pitch_chroma over the shim and compare with the file."""
-    from oracle import reference_shim
-    if not reference_shim.reference_available():
-        pytest.skip("/root/reference is not present on this machine")
-    ref = reference_shim.load_reference()
+def test_port_pitch_chroma_matches_reference_flow(g):
+    """The reference's estimate_pitch_chroma, as stored in the golden file, against the port's chunk-wise chroma lags
+    and shift bootstrap on the same inputs."""
     src3 = synth.synth(3000, 75.0, SR, bpm=112.0)
     nc3 = synth.synth(3000, 60.0, SR, bpm=112.0, speed=1.25, pitch_mult=1.25 * 2.0 ** (1.5 / 12))
-    s_hz, n_hz, point, ci, n_chunks = ref.pitch.estimate_pitch_chroma(src3, nc3, SR)
+    s_hz, n_hz, point, ci, n_chunks, _ = port.estimate_pitch_chroma(src3, nc3, SR)
     B = g["pitch_B"]
     assert n_hz == [unhex(v) for v in B["nc_hz"]] and point == unhex(B["point_st"]) and n_chunks == B["n_chunks"]
+    assert s_hz == [unhex(v) for v in B["src_hz"]]
     assert tuple(ci) == tuple(unhex(v) for v in B["ci_st"])
 
 
