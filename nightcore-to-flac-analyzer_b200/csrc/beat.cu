@@ -5,8 +5,7 @@
 // One CTA per envelope.  All arithmetic is float64 and this file is compiled with -fmad=false so
 // that sums and products round exactly like the CPU restatement (oracle/csrc/oracle_native.c).
 // The DP is sequential in time, but frame i only looks back to [i-2·fpb, i-round(fpb/2)], so
-// round(fpb/2) consecutive frames are independent: they form one wavefront, one thread each.
-#include <stdlib.h>
+// round(fpb/2) consecutive frames are independent: they form one wavefront, computed in parallel.
 #include "ncfa_common.cuh"
 
 namespace ncfa {
@@ -201,9 +200,7 @@ __global__ void __launch_bounds__(256) beat_score_kernel(const int32_t *__restri
         atomicMax(reinterpret_cast<unsigned long long *>(base + 3 * (size_t)env_stride + 2 * K), f64_to_ordered(lmax));
 }
 
-// MONO = true (default): the DP exploits that the best predecessor moves monotonically with the frame — see the
-// comment at the wavefront loop; MONO = false is the full scan of every candidate (NCFA_BEAT_DP=scan, cross-check).
-template <bool MONO>
+// The DP exploits that the best predecessor moves monotonically with the frame — see the comment at the wavefront loop.
 __global__ void beat_track_kernel(const float *__restrict__ onset, const int64_t *__restrict__ onset_off,
                                   const int32_t *__restrict__ env_len, int env_stride, const int32_t *__restrict__ lag,
                                   double *__restrict__ ws_f64, int32_t *__restrict__ ws_i32, int max_fpb,
@@ -259,175 +256,84 @@ __global__ void beat_track_kernel(const float *__restrict__ onset, const int64_t
         first = block_reduce(first, sh_i, [](int a, int b) { return a < b ? a : b; });
     }
 
-    if constexpr (MONO) {
-        // ---- DP over wavefronts of `near` independent frames, with a MONOTONE ARGMAX search.
-        // score(i, loc) = cum[loc] − pen[i − loc], pen(d) = 100·ln²(d / fpb) is strictly convex for d < e·fpb, and the
-        // search window ends at d = 2·fpb.  For loc2 < loc1 the exact scores satisfy
-        //     score(i, loc2) + score(i+1, loc1) − score(i, loc1) − score(i+1, loc2) = Σ_{d} pen''(d) >= 15 / fpb² (> 3e-5 here),
-        // an inverse-Monge gap that is five orders of magnitude above the rounding of the float64 scores (half an ulp of
-        // cum, < 1e-10 for any envelope length that fits the workspace) — so the winning predecessor (maximum score, ties
-        // to the nearest = largest loc, librosa's rule) of frame i+1 is never farther back than the one of frame i, for
-        // the COMPUTED values too.  Hence: every S-th frame of the wavefront (and its last frame) is an anchor and gets
-        // the full scan, one warp each; a frame between two anchors only scans [best(anchor before), best(anchor after)]
-        // — typically a handful of candidates instead of 1.5·fpb.  Same maxima, same tie rule, same float64 values as
-        // the full scan; ~5x fewer evaluations.
-        constexpr int S = 8;
-        int *wloc = reinterpret_cast<int *>(pen + (far - near + 1) + 1);  // best predecessor of every frame of the wavefront
-        const int lane = tid & 31, warp = tid >> 5, nwarps = nt >> 5;
-        constexpr int L = 4;
-        const int ngroups = nt / L, grp = tid / L, sub = tid % L;
-        for (int basei = 0; basei < N; basei += near) {
-            const int nf = min(near, N - basei);
-            const int na = (nf - 1) / S + 1 + (((nf - 1) % S) ? 1 : 0);
-            // phase A: anchors, one warp per anchor
-            for (int a = warp; a < na; a += nwarps) {
-                const int j = min(a * S, nf - 1);
-                const int i = basei + j;
-                const double lsi = (lane == 0) ? ls[i] : 0.0;
-                double best = -INFINITY;
-                int bl = -1;
-                const int lo = max(0, i - far);
-                for (int loc = i - near - lane; loc >= lo; loc -= 32) {  // nearest first: strict > keeps the lane's nearest maximum
+    // ---- DP over wavefronts of `near` independent frames, with a MONOTONE ARGMAX search.
+    // score(i, loc) = cum[loc] − pen[i − loc], pen(d) = 100·ln²(d / fpb) is strictly convex for d < e·fpb, and the
+    // search window ends at d = 2·fpb.  For loc2 < loc1 the exact scores satisfy
+    //     score(i, loc2) + score(i+1, loc1) − score(i, loc1) − score(i+1, loc2) = Σ_{d} pen''(d) >= 15 / fpb² (> 3e-5 here),
+    // an inverse-Monge gap that is five orders of magnitude above the rounding of the float64 scores (half an ulp of
+    // cum, < 1e-10 for any envelope length that fits the workspace) — so the winning predecessor (maximum score, ties
+    // to the nearest = largest loc, librosa's rule) of frame i+1 is never farther back than the one of frame i, for
+    // the COMPUTED values too.  Hence: every S-th frame of the wavefront (and its last frame) is an anchor and gets
+    // the full scan, one warp each; a frame between two anchors only scans [best(anchor before), best(anchor after)]
+    // — typically a handful of candidates instead of 1.5·fpb.  Same maxima, same tie rule, same float64 values as
+    // the full scan; ~5x fewer evaluations.
+    constexpr int S = 8;
+    int *wloc = reinterpret_cast<int *>(pen + (far - near + 1) + 1);  // best predecessor of every frame of the wavefront
+    const int lane = tid & 31, warp = tid >> 5, nwarps = nt >> 5;
+    constexpr int L = 4;
+    const int ngroups = nt / L, grp = tid / L, sub = tid % L;
+    for (int basei = 0; basei < N; basei += near) {
+        const int nf = min(near, N - basei);
+        const int na = (nf - 1) / S + 1 + (((nf - 1) % S) ? 1 : 0);
+        // phase A: anchors, one warp per anchor
+        for (int a = warp; a < na; a += nwarps) {
+            const int j = min(a * S, nf - 1);
+            const int i = basei + j;
+            const double lsi = (lane == 0) ? ls[i] : 0.0;
+            double best = -INFINITY;
+            int bl = -1;
+            const int lo = max(0, i - far);
+            for (int loc = i - near - lane; loc >= lo; loc -= 32) {  // nearest first: strict > keeps the lane's nearest maximum
+                const double sc = cring[loc & rmask] - pen[i - loc - near];
+                if (sc > best) {
+                    best = sc;
+                    bl = loc;
+                }
+            }
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) {
+                const double ob = __shfl_xor_sync(0xffffffffu, best, o);
+                const int ol = __shfl_xor_sync(0xffffffffu, bl, o);
+                if (ol >= 0 && (bl < 0 || ob > best || (ob == best && ol > bl))) {
+                    best = ob;
+                    bl = ol;
+                }
+            }
+            if (lane == 0) {
+                const double c = (bl >= 0) ? lsi + best : lsi;
+                cum[i] = c;
+                cring[i & rmask] = c;  // frames of this wavefront never alias the ones being read: ring >= far + near
+                backlink[i] = (i < first) ? -1 : bl;
+                wloc[j] = bl;
+            }
+        }
+        __syncthreads();
+        // phase B: the frames between anchors, a group of L lanes each, over the interval the anchors leave
+        const int n_between = (nf - 1) - ((nf - 1 + S - 1) / S);  // j in (0, nf−1) with j % S != 0
+        const int rounds = (n_between + ngroups - 1) / ngroups;
+        for (int r = 0; r < rounds; ++r) {  // warp-uniform trip count: every lane takes part in the shuffles
+            const int g = r * ngroups + grp;
+            const int j = (g / (S - 1)) * S + 1 + g % (S - 1);
+            const bool active = g < n_between && j < nf - 1;
+            const int i = basei + j;
+            double best = -INFINITY;
+            int bl = -1;
+            const double lsi = (active && sub == 0) ? ls[i] : 0.0;
+            if (active) {
+                const int ja = (j / S) * S, jb = min(ja + S, nf - 1);
+                const int A = wloc[ja], B = wloc[jb];
+                int lo = max(0, i - far), hi = i - near;
+                if (A >= 0) lo = max(lo, A);
+                if (B >= 0) hi = min(hi, B);  // B < 0: the later anchor has no predecessor at all, then neither has i (hi < 0)
+                for (int loc = hi - sub; loc >= lo; loc -= L) {
                     const double sc = cring[loc & rmask] - pen[i - loc - near];
                     if (sc > best) {
                         best = sc;
                         bl = loc;
                     }
                 }
+            }
 #pragma unroll
-                for (int o = 16; o > 0; o >>= 1) {
-                    const double ob = __shfl_xor_sync(0xffffffffu, best, o);
-                    const int ol = __shfl_xor_sync(0xffffffffu, bl, o);
-                    if (ol >= 0 && (bl < 0 || ob > best || (ob == best && ol > bl))) {
-                        best = ob;
-                        bl = ol;
-                    }
-                }
-                if (lane == 0) {
-                    const double c = (bl >= 0) ? lsi + best : lsi;
-                    cum[i] = c;
-                    cring[i & rmask] = c;  // frames of this wavefront never alias the ones being read: ring >= far + near
-                    backlink[i] = (i < first) ? -1 : bl;
-                    wloc[j] = bl;
-                }
-            }
-            __syncthreads();
-            // phase B: the frames between anchors, a group of L lanes each, over the interval the anchors leave
-            const int n_between = (nf - 1) - ((nf - 1 + S - 1) / S);  // j in (0, nf−1) with j % S != 0
-            const int rounds = (n_between + ngroups - 1) / ngroups;
-            for (int r = 0; r < rounds; ++r) {  // warp-uniform trip count: every lane takes part in the shuffles
-                const int g = r * ngroups + grp;
-                const int j = (g / (S - 1)) * S + 1 + g % (S - 1);
-                const bool active = g < n_between && j < nf - 1;
-                const int i = basei + j;
-                double best = -INFINITY;
-                int bl = -1;
-                const double lsi = (active && sub == 0) ? ls[i] : 0.0;
-                if (active) {
-                    const int ja = (j / S) * S, jb = min(ja + S, nf - 1);
-                    const int A = wloc[ja], B = wloc[jb];
-                    int lo = max(0, i - far), hi = i - near;
-                    if (A >= 0) lo = max(lo, A);
-                    if (B >= 0) hi = min(hi, B);  // B < 0: the later anchor has no predecessor at all, then neither has i (hi < 0)
-                    for (int loc = hi - sub; loc >= lo; loc -= L) {
-                        const double sc = cring[loc & rmask] - pen[i - loc - near];
-                        if (sc > best) {
-                            best = sc;
-                            bl = loc;
-                        }
-                    }
-                }
-#pragma unroll
-                for (int o = L >> 1; o > 0; o >>= 1) {
-                    const double ob = __shfl_xor_sync(0xffffffffu, best, o);
-                    const int ol = __shfl_xor_sync(0xffffffffu, bl, o);
-                    if (ol >= 0 && (bl < 0 || ob > best || (ob == best && ol > bl))) {
-                        best = ob;
-                        bl = ol;
-                    }
-                }
-                if (active && sub == 0) {
-                    const double c = (bl >= 0) ? lsi + best : lsi;
-                    cum[i] = c;
-                    cring[i & rmask] = c;
-                    backlink[i] = (i < first) ? -1 : bl;
-                }
-            }
-            __syncthreads();
-        }
-    } else {
-    // ---- DP over wavefronts of `near` independent frames.  A frame is owned by a group of L lanes (L = largest power
-    // of two with near·L <= blockDim, at most 32) that share the scan over the predecessors loc = i−near … i−2·fpb
-    // (nearest first).  librosa keeps the first strict maximum in that order; the lane-local strict > plus the
-    // (score, larger loc) reduction reproduces it exactly.
-    int L = 1;
-    while (L < 32 && near * (2 * L) <= nt) L *= 2;
-    const int ngroups = nt / L, grp = tid / L, sub = tid % L;
-    const int rounds = (near + ngroups - 1) / ngroups;
-    for (int basei = 0; basei < N; basei += near) {
-        for (int r = 0; r < rounds; ++r) {  // warp-uniform trip count: every lane takes part in the shuffles
-            const int j = r * ngroups + grp;
-            const int i = basei + j;
-            const bool active = j < near && i < N;
-            double best = -INFINITY;
-            int bl = -1;
-            const double lsi = (active && sub == 0) ? ls[i] : 0.0;  // issued before the scan hides its latency
-            if (active) {
-                int lo = i - far;
-                if (lo < 0) lo = 0;
-                // element k of this lane: loc = first − L·k (nearest first), score = cring[loc] − pen[sub + L·k].
-                // The scan keeps only the running maximum and WHERE a group of four produced it (three max + one
-                // compare per four elements instead of a compare-and-select per element); the winning group is
-                // re-read at the end to find its first (nearest) element equal to the maximum — the scores are
-                // recomputed from the same operands, so the comparison is exact.
-                const int first_loc = i - near - sub;
-                const int n_el = first_loc >= lo ? (first_loc - lo) / L + 1 : 0;
-                int kbest = -1, wbest = 1;
-                if (n_el > 0) {
-                    const int idx0 = first_loc & rmask;
-                    int n1 = idx0 / L + 1;  // elements before the ring index wraps
-                    if (n1 > n_el) n1 = n_el;
-                    const double *pp = pen + sub;
-                    const double *cp = cring + idx0;
-                    int k = 0;
-#pragma unroll 1
-                    for (int part = 0; part < 2; ++part) {
-                        const int kend = part == 0 ? n1 : n_el;
-                        for (; k + 4 <= kend; k += 4) {
-                            const double s0 = cp[0] - pp[0];
-                            const double s1 = cp[-L] - pp[L];
-                            const double s2 = cp[-2 * L] - pp[2 * L];
-                            const double s3 = cp[-3 * L] - pp[3 * L];
-                            const double m = fmax(fmax(s0, s1), fmax(s2, s3));
-                            if (m > best) {
-                                best = m;
-                                kbest = k;
-                                wbest = 4;
-                            }
-                            cp -= 4 * L;
-                            pp += 4 * L;
-                        }
-                        for (; k < kend; ++k) {
-                            const double sc = cp[0] - pp[0];
-                            if (sc > best) {
-                                best = sc;
-                                kbest = k;
-                                wbest = 1;
-                            }
-                            cp -= L;
-                            pp += L;
-                        }
-                        cp += ring;  // the remaining elements sit one ring length higher
-                    }
-                    for (int kk = kbest; kk < kbest + wbest; ++kk) {
-                        const int loc = first_loc - L * kk;
-                        if (cring[loc & rmask] - pen[sub + L * kk] == best) {
-                            bl = loc;
-                            break;
-                        }
-                    }
-                }
-            }
             for (int o = L >> 1; o > 0; o >>= 1) {
                 const double ob = __shfl_xor_sync(0xffffffffu, best, o);
                 const int ol = __shfl_xor_sync(0xffffffffu, bl, o);
@@ -439,13 +345,11 @@ __global__ void beat_track_kernel(const float *__restrict__ onset, const int64_t
             if (active && sub == 0) {
                 const double c = (bl >= 0) ? lsi + best : lsi;
                 cum[i] = c;
-                cring[i & rmask] = c;  // frames of this wavefront never alias the ones being read: ring >= far + near
+                cring[i & rmask] = c;
                 backlink[i] = (i < first) ? -1 : bl;
             }
         }
         __syncthreads();
-    }
-
     }
 
     // ---- last beat: last local max of cumscore with cumscore >= ½·median(local-max scores)
@@ -554,20 +458,12 @@ extern "C" int ncfa_beat_track_batched(const float *d_onset, const int64_t *d_on
     double *wf = (double *)d_workspace;
     int32_t *wi = (int32_t *)((char *)d_workspace +
                               align_up((size_t)n_seg * beat_f64_per_seg(max_env_len, max_lag) * 8, 256));
-    static const int long_threads = [] {
-        const char *e = getenv("NCFA_BEAT_THREADS");  // experiments only
-        const int v = e ? atoi(e) : 0;
-        return (v == 256 || v == 512 || v == 1024) ? v : 512;  // measured: 9.9 ms (512) vs 11.1 (1024) vs 12.5 (256) per 250 pairs
-    }();
-    const int threads = max_env_len <= 2048 ? 64 : long_threads;
+    // long envelopes: measured on B200, 9.9 ms (512 threads) vs 11.1 (1024) vs 12.5 (256) per 250 pairs
+    const int threads = max_env_len <= 2048 ? 64 : 512;
     const int ring = beat_ring(max_lag);
     // reduction scratch | score ring | transition penalties | best predecessor per frame of a wavefront (ints)
     const size_t smem = ((size_t)threads + ring + (3 * (size_t)max_lag / 2 + 4) + ((size_t)max_lag / 4 + 4)) * sizeof(double);
-    static const bool mono = [] {
-        const char *e = getenv("NCFA_BEAT_DP");  // "scan": the full scan of every candidate (cross-check)
-        return !(e && strcmp(e, "scan") == 0);
-    }();
-    int rc = ensure_dynamic_smem(mono ? (const void *)beat_track_kernel<true> : (const void *)beat_track_kernel<false>, smem);
+    int rc = ensure_dynamic_smem((const void *)beat_track_kernel, smem);
     if (rc) return rc;
     {
         ProfScope _p("beat_prep_kernel", (cudaStream_t)stream);
@@ -588,14 +484,9 @@ extern "C" int ncfa_beat_track_batched(const float *d_onset, const int64_t *d_on
     NCFA_LAUNCH_OK("beat_score_kernel");
     {
         ProfScope _p(max_env_len <= 2048 ? "beat_track_kernel" : "beat_track_kernel[long]", (cudaStream_t)stream);
-        if (mono)
-            beat_track_kernel<true><<<n_seg, threads, smem, (cudaStream_t)stream>>>(d_onset, d_onset_off, d_env_len,
-                                                                                     max_env_len, d_lag, wf, wi, max_lag,
-                                                                                     d_beats, max_beats, d_n_beats, ring);
-        else
-            beat_track_kernel<false><<<n_seg, threads, smem, (cudaStream_t)stream>>>(d_onset, d_onset_off, d_env_len,
-                                                                                      max_env_len, d_lag, wf, wi, max_lag,
-                                                                                      d_beats, max_beats, d_n_beats, ring);
+        beat_track_kernel<<<n_seg, threads, smem, (cudaStream_t)stream>>>(d_onset, d_onset_off, d_env_len, max_env_len,
+                                                                          d_lag, wf, wi, max_lag, d_beats, max_beats,
+                                                                          d_n_beats, ring);
     }
     NCFA_LAUNCH_OK("beat_track_kernel");
     return NCFA_OK;

@@ -7,15 +7,14 @@
 //   tuning_pick_kernel    median magnitude over the segment (radix select) → histogram of the peaks at
 //                         or above it → first fullest bin = tuning index j, tuning = −0.5 + j/100
 //   decimate2_kernel      2:1 decimation ×√2 between octaves (127-tap Kaiser half-band, float64 sums)
-//   cqt_chroma_kernel     per octave: the 36 CQT responses of every frame as ONE real contraction
-//                         C[72 × frames] = K[72 × 1024] · X[1024 × frames],  X[n][t] = y_oct[t·hop_oct + n − 512]
+//   cqt_tc_kernel         per octave: the 36 CQT responses of every frame as ONE real contraction on the tensor
+//                         cores, C[72 × frames] = K[72 × 1024] · X[1024 × frames],  X[n][t] = y_oct[t·hop_oct + n − 512]
 //                         (K = sparsified FFT-domain basis ∘ DFT, folded on the host in float64 — the same
 //                         linear map as rectangular-window STFT followed by the sparse basis product),
 //                         then |·|, fold 252 → 12 chroma, inf-norm per frame, partial sums over frames
 //   chroma_mean_kernel    partial sums → mean chroma float64[12] per segment
 //   cyclic_xcorr_kernel   argmax_k dot(src, roll(nc, −k)) wrapped to (−n/2, n/2]
 #include <cmath>
-#include <cstdlib>
 #include <cstring>
 #include <algorithm>
 #include <complex>
@@ -37,9 +36,10 @@ constexpr int kHbTaps = 127;
 constexpr int kPeakStride = 180;  // ≥ max local maxima among the 358 candidate bins (179)
 
 struct ChromaTables {
-    const float *K;     // [100][1024][72]  K[j][n][r]: r < 36 real part of bin r, r ≥ 36 imaginary part of bin r−36
     const double *hb;   // [127] half-band taps
-    const float *Bimg;  // [100][32 k-tiles][hi, lo][80 rows × 32 k] tf32 split of K as swizzle-128B shared-memory images
+    // [100][32 k-tiles][hi, lo][80 rows × 32 k] tf32 split of K as swizzle-128B shared-memory images, where
+    // K[j][n][r] (tuning j, [100][1024][72]): r < 36 real part of bin r, r ≥ 36 imaginary part of bin r−36
+    const float *Bimg;
 };
 
 constexpr int kTcN = 80;                          // MMA N: 72 rows of K + 8 zero rows (N % 16 == 0 for M = 128)
@@ -201,14 +201,6 @@ static void build_halfband(std::vector<double> &h) {
 // them as constant-bank operands (no shared-memory load per tap)
 __constant__ double c_hb_even[64];
 __constant__ double c_hb_mid;
-__constant__ float c_hbf_even[64];
-__constant__ float c_hbf_mid;
-template <typename acc_t> __device__ __forceinline__ acc_t hb_even_tap(int m);
-template <> __device__ __forceinline__ double hb_even_tap<double>(int m) { return c_hb_even[m]; }
-template <> __device__ __forceinline__ float hb_even_tap<float>(int m) { return c_hbf_even[m]; }
-template <typename acc_t> __device__ __forceinline__ acc_t hb_mid_tap();
-template <> __device__ __forceinline__ double hb_mid_tap<double>() { return c_hb_mid; }
-template <> __device__ __forceinline__ float hb_mid_tap<float>() { return c_hbf_mid; }
 
 static std::mutex g_hb_mu;
 static std::map<int, const double *> g_hb;
@@ -228,17 +220,10 @@ int get_halfband_device(const double **out) {
     NCFA_CUDA_OK(cudaMemcpy(dh, h.data(), h.size() * sizeof(double), cudaMemcpyHostToDevice));
     {
         double ev[64];
-        float evf[64];
-        for (int m = 0; m < 64; ++m) {
-            ev[m] = h[2 * m];
-            evf[m] = (float)h[2 * m];
-        }
+        for (int m = 0; m < 64; ++m) ev[m] = h[2 * m];
         const double mid = h[(kHbTaps - 1) / 2];
-        const float midf = (float)mid;
         NCFA_CUDA_OK(cudaMemcpyToSymbol(c_hb_even, ev, sizeof(ev)));
         NCFA_CUDA_OK(cudaMemcpyToSymbol(c_hb_mid, &mid, sizeof(mid)));
-        NCFA_CUDA_OK(cudaMemcpyToSymbol(c_hbf_even, evf, sizeof(evf)));
-        NCFA_CUDA_OK(cudaMemcpyToSymbol(c_hbf_mid, &midf, sizeof(midf)));
     }
     g_hb[dev] = dh;
     *out = dh;
@@ -266,9 +251,6 @@ static int get_chroma_tables(int sr, ChromaTables *out) {
         memcpy(all.data() + (size_t)j * kCqtNfft * kCqtRows, one.data(), one.size() * sizeof(float));
     }
     ChromaTables t;
-    float *dK = nullptr;
-    NCFA_CUDA_OK(cudaMalloc(&dK, all.size() * sizeof(float)));
-    NCFA_CUDA_OK(cudaMemcpy(dK, all.data(), all.size() * sizeof(float), cudaMemcpyHostToDevice));
     {
         int rc = get_halfband_device(&t.hb);
         if (rc) return rc;
@@ -283,7 +265,6 @@ static int get_chroma_tables(int sr, ChromaTables *out) {
         NCFA_CUDA_OK(cudaMemcpy(dB, img.data(), img.size() * sizeof(float), cudaMemcpyHostToDevice));
         t.Bimg = dB;
     }
-    t.K = dK;
     g_chroma_tables[key] = t;
     *out = t;
     return NCFA_OK;
@@ -493,14 +474,13 @@ __global__ void __launch_bounds__(256) tuning_pick_kernel(const int32_t *__restr
 //     out[t] = h[63]·xe[t] + Σ_{m<64} h[2m]·xo[t + m − 32],   xe[j] = in[2j], xo[j] = in[2j+1].
 // A CTA de-interleaves its input span into xe / xo in shared memory; each thread produces 4 consecutive outputs
 // from a 67-sample register window (17 conflict-free LDS.128), float64 accumulation.
-// Accumulation type: float64 like the oracle.  A float32 variant (NCFA_DECIMATE=f32) was measured: 10.6 -> 8.3 ms per
+// Accumulation type: float64 like the oracle.  A float32 variant was measured: 10.6 -> 8.3 ms per
 // 250 pairs only — the kernel is paced by its strided staging loads, not by the FP64 pipe — so the exact sums stay.
 // ncu (profiles/r2f_ncu_summary.md, 4 outputs per thread): XU pipe 61 % — the float → double conversions of the register
 // window, 17.75 per output — next to FP64 54 %.  Eight outputs per thread share a 71-sample window: 9.9 conversions per
 // output, and the kernel is left with its 64 float64 FMAs per output.
 constexpr int kDecPerThread = 8;
 constexpr int kDecOutPerCta = 256 * kDecPerThread;
-template <typename acc_t>
 __global__ void __launch_bounds__(256) decimate2_kernel(const float *__restrict__ audio,
                                                         const int64_t *__restrict__ seg_off,
                                                         const int32_t *__restrict__ seg_len, int level,
@@ -538,30 +518,30 @@ __global__ void __launch_bounds__(256) decimate2_kernel(const float *__restrict_
     }
     __syncthreads();
     const int t = kDecPerThread * threadIdx.x;  // outputs o0 + t .. o0 + t + 7 use xo[t .. t + 70]
-    acc_t w[72];
+    double w[72];
 #pragma unroll
     for (int j = 0; j < 18; ++j) {
         const float4 v = *reinterpret_cast<const float4 *>(xo + t + 4 * j);
-        w[4 * j] = (acc_t)v.x;
-        w[4 * j + 1] = (acc_t)v.y;
-        w[4 * j + 2] = (acc_t)v.z;
-        w[4 * j + 3] = (acc_t)v.w;
+        w[4 * j] = (double)v.x;
+        w[4 * j + 1] = (double)v.y;
+        w[4 * j + 2] = (double)v.z;
+        w[4 * j + 3] = (double)v.w;
     }
-    acc_t a[kDecPerThread];
+    double a[kDecPerThread];
     {
         const float4 e0 = *reinterpret_cast<const float4 *>(xe + t);
         const float4 e1 = *reinterpret_cast<const float4 *>(xe + t + 4);
-        const acc_t hm = hb_mid_tap<acc_t>();
-        a[0] = hm * (acc_t)e0.x, a[1] = hm * (acc_t)e0.y, a[2] = hm * (acc_t)e0.z, a[3] = hm * (acc_t)e0.w;
-        a[4] = hm * (acc_t)e1.x, a[5] = hm * (acc_t)e1.y, a[6] = hm * (acc_t)e1.z, a[7] = hm * (acc_t)e1.w;
+        const double hm = c_hb_mid;
+        a[0] = hm * (double)e0.x, a[1] = hm * (double)e0.y, a[2] = hm * (double)e0.z, a[3] = hm * (double)e0.w;
+        a[4] = hm * (double)e1.x, a[5] = hm * (double)e1.y, a[6] = hm * (double)e1.z, a[7] = hm * (double)e1.w;
     }
 #pragma unroll
     for (int m = 0; m < 64; ++m) {  // ascending m per output, as before: the sums round identically
-        const acc_t hm = hb_even_tap<acc_t>(m);  // compile-time index: a constant-bank operand of the FMAs
+        const double hm = c_hb_even[m];  // compile-time index: a constant-bank operand of the FMAs
 #pragma unroll
         for (int u = 0; u < kDecPerThread; ++u) a[u] = fma(hm, w[m + u], a[u]);
     }
-    const acc_t r2 = (acc_t)1.4142135623730951;
+    const double r2 = 1.4142135623730951;
     const int o = o0 + t;
     if (o + kDecPerThread - 1 < n_out && (reinterpret_cast<uintptr_t>(out + o) & 15u) == 0) {  // level offsets: multiples of 4 floats
         *reinterpret_cast<float4 *>(out + o) =
@@ -575,19 +555,8 @@ __global__ void __launch_bounds__(256) decimate2_kernel(const float *__restrict_
     }
 }
 
-static bool decimate_f64() {
-    static const bool v = [] {
-        const char *e = getenv("NCFA_DECIMATE");
-        return !(e && strcmp(e, "f32") == 0);
-    }();
-    return v;
-}
-
 // ------------------------------------------------------------------------------------------------ CQT → chroma
-constexpr int kCqtTF = 32;                                   // frames per CTA
-constexpr int kCqtKT = 32;                                   // n (time-sample) tile of the contraction
-constexpr int kCqtThreads = 160;                             // 18 row groups × 8 frame groups = 144 active
-constexpr int kCqtSpanMax = (kCqtTF - 1) * 512 + kCqtNfft;   // widest sample span (octave 0)
+constexpr int kPartialTF = 32;  // frames per tile of the partial[] stride (the workspace is sized in 32-frame tiles)
 
 // |re + i·im| as np.abs(complex64) gives it (hypot): re² + im² underflows in float32 below ~1e-19, and a frame whose only
 // content is that small (the tail of a decayed note reaching the lowest octave of an otherwise digitally silent stretch)
@@ -599,152 +568,12 @@ __device__ __forceinline__ float cabs_f32(float re, float im) {
     return sqrtf(as * as + bs * bs) * 0x1p-96f;
 }
 
-struct CqtSmem {
-    float sig[kCqtSpanMax + kCqtTF + kCqtNfft / 8 + 8];  // skewed: sample s lives at s + (s >> log2 hop)
-    float kt[kCqtKT][kCqtRows];                          // K tile, n-major
-    float c[kCqtRows][kCqtTF + 1];                       // responses of the current octave
-    float chroma[kChroma][kCqtTF];                       // summed over octaves
-};
-
-template <int L2HOP>
-__device__ __forceinline__ void cqt_octave(CqtSmem &sm, const float *__restrict__ y, int len, int t0,
-                                           const float *__restrict__ Kj, int tid) {
-    constexpr int HOP = 1 << L2HOP;
-    constexpr int SPAN = (kCqtTF - 1) * HOP + kCqtNfft;
-    // ---- stage the sample span of this octave (centred frames: frame t starts at t·hop − 512)
-    const int64_t pos0 = (int64_t)t0 * HOP - kCqtNfft / 2;
-    for (int s = tid; s < SPAN; s += kCqtThreads) {
-        const int64_t p = pos0 + s;
-        sm.sig[s + (s >> L2HOP)] = (p >= 0 && p < len) ? __ldg(y + p) : 0.0f;
-    }
-    const int ty = tid >> 3, tx = tid & 7;  // rows 4ty..4ty+3, frames tx + 8c
-    const bool active = ty < kCqtRows / 4;
-    float acc[4][4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) acc[i][j] = 0.0f;
-    int fbase[4];
-#pragma unroll
-    for (int c = 0; c < 4; ++c) fbase[c] = (tx + 8 * c) * (HOP + 1);
-    // register prefetch of the K tile: 32×72 floats = 576 float4, ≤ 4 per thread
-    constexpr int kT4 = kCqtKT * kCqtRows / 4;
-    float4 pre[4];
-    const float4 *Kg = reinterpret_cast<const float4 *>(Kj);
-#pragma unroll
-    for (int q = 0; q < 4; ++q) {
-        const int idx = tid + q * kCqtThreads;
-        pre[q] = idx < kT4 ? __ldg(Kg + idx) : make_float4(0, 0, 0, 0);
-    }
-    for (int n0 = 0; n0 < kCqtNfft; n0 += kCqtKT) {
-        __syncthreads();  // previous tile consumed (and, first time, the span is staged)
-        float4 *kt4 = reinterpret_cast<float4 *>(&sm.kt[0][0]);
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-            const int idx = tid + q * kCqtThreads;
-            if (idx < kT4) kt4[idx] = pre[q];
-        }
-        __syncthreads();
-        if (n0 + kCqtKT < kCqtNfft) {
-            const float4 *Kn = Kg + (size_t)(n0 + kCqtKT) * kCqtRows / 4;
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-                const int idx = tid + q * kCqtThreads;
-                pre[q] = idx < kT4 ? __ldg(Kn + idx) : make_float4(0, 0, 0, 0);
-            }
-        }
-        if (active) {
-#pragma unroll
-            for (int nn = 0; nn < kCqtKT; ++nn) {
-                const int n = n0 + nn;
-                const float4 kv = *reinterpret_cast<const float4 *>(&sm.kt[nn][4 * ty]);
-                const int o = n + (n >> L2HOP);
-                float x[4];
-#pragma unroll
-                for (int c = 0; c < 4; ++c) x[c] = sm.sig[fbase[c] + o];
-#pragma unroll
-                for (int c = 0; c < 4; ++c) {
-                    acc[0][c] = fmaf(kv.x, x[c], acc[0][c]);
-                    acc[1][c] = fmaf(kv.y, x[c], acc[1][c]);
-                    acc[2][c] = fmaf(kv.z, x[c], acc[2][c]);
-                    acc[3][c] = fmaf(kv.w, x[c], acc[3][c]);
-                }
-            }
-        }
-    }
-    if (active) {
-#pragma unroll
-        for (int i = 0; i < 4; ++i)
-#pragma unroll
-            for (int c = 0; c < 4; ++c) sm.c[4 * ty + i][tx + 8 * c] = acc[i][c];
-    }
-    __syncthreads();
-    // ---- |response| and fold: bin b feeds chroma ((b + 1) mod 36) / 3  (cq_to_chroma: 3 bins per semitone, rolled −1)
-    for (int i = tid; i < kChroma * kCqtTF; i += kCqtThreads) {
-        const int ch = i / kCqtTF, t = i % kCqtTF;
-        float s = 0.0f;
-#pragma unroll
-        for (int q = 0; q < 3; ++q) {
-            const int b = (3 * ch - 1 + q + kCqtBins) % kCqtBins;
-            const float re = sm.c[b][t], im = sm.c[kCqtBins + b][t];
-            s += cabs_f32(re, im);
-        }
-        sm.chroma[ch][t] += s;
-    }
-    // the next octave's first __syncthreads orders these reads before sm.c / sm.sig are rewritten
-}
-
 struct PyrOffsets {
     size_t off[kOctaves + 1];  // float offset of level o (1..6) inside a segment's pyramid; off[7] = stride
 };
 
-__global__ void __launch_bounds__(kCqtThreads) cqt_chroma_kernel(const float *__restrict__ audio,
-                                                                 const int64_t *__restrict__ seg_off,
-                                                                 const int32_t *__restrict__ seg_len,
-                                                                 const float *__restrict__ pyr, PyrOffsets po,
-                                                                 const int32_t *__restrict__ tuning_idx,
-                                                                 const float *__restrict__ Kall, int tile_stride,
-                                                                 double *__restrict__ partial) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    CqtSmem &sm = *reinterpret_cast<CqtSmem *>(smem_raw);
-    const int seg = blockIdx.y;
-    const int n = seg_len[seg];
-    const int n_frames = cqt_frames(n);
-    const int t0 = blockIdx.x * kCqtTF;
-    if (t0 >= n_frames) return;
-    const int tid = threadIdx.x;
-    int tj = tuning_idx[seg];
-    tj = tj < 0 ? 0 : (tj >= kNTunings ? kNTunings - 1 : tj);
-    const float *Kj = Kall + (size_t)tj * kCqtNfft * kCqtRows;
-    for (int i = tid; i < kChroma * kCqtTF; i += kCqtThreads) (&sm.chroma[0][0])[i] = 0.0f;
-    const float *pseg = pyr + (size_t)seg * po.off[kOctaves];
-    cqt_octave<9>(sm, audio + seg_off[seg], n, t0, Kj, tid);
-    cqt_octave<8>(sm, pseg + po.off[1], level_len(n, 1), t0, Kj, tid);
-    cqt_octave<7>(sm, pseg + po.off[2], level_len(n, 2), t0, Kj, tid);
-    cqt_octave<6>(sm, pseg + po.off[3], level_len(n, 3), t0, Kj, tid);
-    cqt_octave<5>(sm, pseg + po.off[4], level_len(n, 4), t0, Kj, tid);
-    cqt_octave<4>(sm, pseg + po.off[5], level_len(n, 5), t0, Kj, tid);
-    cqt_octave<3>(sm, pseg + po.off[6], level_len(n, 6), t0, Kj, tid);
-    __syncthreads();
-    // ---- librosa.util.normalize(norm=inf) per frame, then the tile's sum over frames (float64)
-    if (tid < 32) {
-        const int t = tid;
-        const bool valid = (t0 + t) < n_frames;
-        float mx = 0.0f;
-#pragma unroll
-        for (int ch = 0; ch < kChroma; ++ch) mx = fmaxf(mx, sm.chroma[ch][t]);
-        const double len = (mx < 1.17549435e-38f) ? 1.0 : (double)mx;
-#pragma unroll
-        for (int ch = 0; ch < kChroma; ++ch) {
-            double v = valid ? (double)sm.chroma[ch][t] / len : 0.0;
-            v = warp_sum(v);
-            if (t == 0) partial[((size_t)seg * tile_stride + blockIdx.x) * kChroma + ch] = v;
-        }
-    }
-}
-
 // ------------------------------------------------------------------------------------------------ CQT on tcgen05
-// Same contraction on the 5th-generation tensor cores:  D[128 frames × 80] (+)= A[128 × 8]·B[80 × 8]^T, kind::tf32,
+// The contraction on the 5th-generation tensor cores:  D[128 frames × 80] (+)= A[128 × 8]·B[80 × 8]^T, kind::tf32,
 // with the 3×TF32 split  x = hi + lo  (hi = x truncated to tf32, lo = x − hi exactly):  A·B ≈ Ah·Bh + Al·Bh + Ah·Bl.
 //   A (the Hankel matrix of frames) is never materialised in memory: the frame warps stage the rows of a k-tile in shared
 //     memory with coalesced cp.async copies (64 contiguous bytes of eight rows per instruction; L1/L2 serve the overlap
@@ -755,57 +584,38 @@ __global__ void __launch_bounds__(kCqtThreads) cqt_chroma_kernel(const float *__
 //   D lives in TMEM; the epilogue is tcgen05.ld → |re + i·im| → fold to 12 chroma.
 // Warp roles (320 threads): warps 0-7 frame warps (A producer + epilogue; warp w serves rows 32·(w & 3) … +31 — its TMEM
 // lane quarter — and column half q = w >> 2 of every k-tile), warp 8 MMA issuer and TMEM allocator, warp 9 B loader.
-// Pipeline shape (struct TcOne / TcTwo below): the default is TWO CTAs per SM, each with 2 A stages, 2 B images, one
-// accumulator and 256 TMEM columns; NCFA_CQT_IMPL=tc1 selects one CTA per SM with 5 A stages, 5 B images and two
-// accumulators (epilogue of octave o−1 overlapped with the MMAs of octave o+1).
+// Pipeline shape: TWO CTAs per SM, each with a shallow pipeline (2 A stages in TMEM, 2 B images in shared memory, one
+// accumulator, 256 TMEM columns, 100 KB of shared memory).  Timing experiments (profiles/r2l_cqt_debug.log) showed that
+// with A traffic, B traffic AND the MMAs all switched off, a deep one-CTA-per-SM pipeline (5 stages, two accumulators,
+// 512 TMEM columns) still took 12.3 of its 13.4 ms: what paces the kernel is the latency of one CTA's serial producer →
+// MMA → release chain, with two or three warps per scheduler to hide it.  A second resident CTA overlaps two such chains
+// on the same tensor pipe: 13.4 -> 9.8 ms per 1750 chunks on B200 (profiles/r2m).  (A k-tile-major variant that fetched
+// every B image once per four octaves — 3.5x less bulk-copy traffic — measured exactly the same 13.4 ms as the
+// octave-major order and was dropped: B traffic is not the limiter either.)
 constexpr int kTcFrames = 128;
 constexpr int kTcQ = 2;                                  // column splits of a k-tile row (threads per frame row)
 constexpr int kTcVals = kTcKT / kTcQ;                    // samples per thread per k-tile (16)
 constexpr int kTcFrameWarps = 4 * kTcQ;
 constexpr int kTcThreads = (kTcFrameWarps + 2) * 32;     // 320
-constexpr int kTcAStages = 5;                           // deep shape (TcOne); the default TcTwo uses 2
-constexpr int kTcBStages = kTcAStages;                   // A and B share the stage index and ONE release barrier per stage
+constexpr int kTcMinBlocks = 2;                          // resident CTAs per SM
+constexpr int kTcStages = 2;                             // A stages (TMEM) = B stages (shared memory): A and B share the
+                                                         // stage index and ONE release barrier per stage
 constexpr int kTcACols = 2 * kTcKT;                      // hi + lo columns of one A stage
 constexpr int kTcAccN = kTcN;                            // accumulator columns (80: 36 real, 36 imaginary, 8 pad)
-constexpr int kTcAPre = 4;                               // k-tiles of A rows in flight (cp.async ring in shared memory)
+constexpr int kTcTmemCols = 256;                         // half of the SM's TMEM per CTA
+constexpr int kTcAPre = 3;                               // k-tiles of A rows in flight (cp.async ring in shared memory)
 constexpr int kTcAPlane = kTcFrames + 1;                 // float4 per chunk plane of the A staging ring
 
-template <int BST, int PRE = kTcAPre>
-struct TcSmemT {
-    alignas(1024) unsigned char b[BST][kTcBStageBytes];
-    float4 arow[PRE][8 * kTcAPlane];  // [slot][16-byte chunk · kTcAPlane + frame]: the odd plane stride keeps both the
+struct TcSmem {
+    alignas(1024) unsigned char b[kTcStages][kTcBStageBytes];
+    float4 arow[kTcAPre][8 * kTcAPlane];  // [slot][16-byte chunk · kTcAPlane + frame]: the odd plane stride keeps both the
                                           // (8 rows × 4 chunks) cp.async writes and the per-row LDS.128 reads conflict free
     float chroma_part[kTcFrames][16];    // [frame][4·q + j]: partial chroma (3q + j) mod 12 of column quarter q
-    alignas(8) uint64_t full_a[kTcAStages], empty_a[kTcAStages], full_b[kTcBStages], empty_b[kTcBStages];
-    uint64_t acc_full[2], acc_empty[2];
+    alignas(8) uint64_t full_a[kTcStages], empty_a[kTcStages], full_b[kTcStages], empty_b[kTcStages];
+    uint64_t acc_full, acc_empty;
     uint32_t tmem_base;
     double red[4][kChroma];
 };
-using TcSmem = TcSmemT<kTcBStages>;
-
-// Pipeline shape of the octave-major kernel.  One: a deep pipeline that owns the SM (5 A stages in TMEM, 5 B images in
-// shared memory, two accumulators, all 512 TMEM columns).  Two: TWO CTAs per SM, each with a shallow pipeline (2 A stages,
-// 2 B images, one accumulator, 256 TMEM columns, 107 KB of shared memory).  The timing experiments (NCFA_TC_DEBUG,
-// profiles/r2l_cqt_debug.log) show that with A traffic, B traffic AND the MMAs all switched off the kernel still takes
-// 12.3 of its 13.4 ms: what paces it is the latency of one CTA's serial producer → MMA → release chain, with two or three
-// warps per scheduler to hide it.  A second resident CTA overlaps two such chains on the same tensor pipe: 13.4 -> 9.8 ms
-// per 1750 chunks (profiles/r2m).  (A k-tile-major variant that fetched every B image once per four octaves — 3.5x less
-// bulk-copy traffic — measured exactly the same 13.4 ms as the octave-major order and was dropped: B traffic is not the
-// limiter either.)
-struct TcOne {
-    static constexpr int kA = kTcAStages, kB = kTcBStages, kAcc = 2, kTmem = 512, kMinBlocks = 1, kPre = kTcAPre;
-};
-struct TcTwo {
-    static constexpr int kA = 2, kB = 2, kAcc = 1, kTmem = 256, kMinBlocks = 2, kPre = 3;   // 100 KB of shared memory per CTA
-};
-
-__device__ __forceinline__ void tc_load_row8(const float *__restrict__ y, int64_t pos, int len, float (&x)[8]) {
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-        const int64_t q = pos + i;
-        x[i] = (q >= 0 && q < len) ? __ldg(y + q) : 0.0f;
-    }
-}
 
 // Epilogue share of column quarter Q: CQT bins b = 9Q … 9Q+8 of this thread's frame.  Accumulator columns: b (real part)
 // and 36+b (imaginary part).  Bin b feeds chroma ((b + 1) mod 36) / 3, i.e.
@@ -839,25 +649,20 @@ __device__ __forceinline__ void tc_epilogue_quarter(uint32_t acc_addr, float (&p
     }
 }
 
-// DBG = false is the production instantiation (the timing-experiment switches compile away); DBG = true honours `dbg`.
-template <bool DBG, typename CFG>
-__global__ void __launch_bounds__(kTcThreads, CFG::kMinBlocks) cqt_tc_kernel(const float *__restrict__ audio,
-                                                               const int64_t *__restrict__ seg_off,
-                                                               const int32_t *__restrict__ seg_len,
-                                                               const float *__restrict__ pyr, PyrOffsets po,
-                                                               const int32_t *__restrict__ tuning_idx,
-                                                               const float *__restrict__ Bimg, int tile_stride,
-                                                               double *__restrict__ partial, int dbg_arg) {
+__global__ void __launch_bounds__(kTcThreads, kTcMinBlocks) cqt_tc_kernel(const float *__restrict__ audio,
+                                                                         const int64_t *__restrict__ seg_off,
+                                                                         const int32_t *__restrict__ seg_len,
+                                                                         const float *__restrict__ pyr, PyrOffsets po,
+                                                                         const int32_t *__restrict__ tuning_idx,
+                                                                         const float *__restrict__ Bimg, int tile_stride,
+                                                                         double *__restrict__ partial) {
     using namespace tc05;
-    const int dbg = DBG ? dbg_arg : 0;
     extern __shared__ __align__(1024) unsigned char smem_raw[];
-    using Smem = TcSmemT<CFG::kB, CFG::kPre>;
-    constexpr int kPre = CFG::kPre;
-    Smem &sm = *reinterpret_cast<Smem *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-    constexpr int kAS = CFG::kA, kBS = CFG::kB;           // A stages (TMEM), B stages (shared memory); equal: one release barrier
-    static_assert(kAS == kBS, "A and B stages share the release barrier");
+    TcSmem &sm = *reinterpret_cast<TcSmem *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
+    constexpr int kPre = kTcAPre;
+    constexpr int kAS = kTcStages, kBS = kTcStages;  // A stages (TMEM), B stages (shared memory)
     constexpr int kAccCol0 = kAS * kTcACols;
-    static_assert(kAccCol0 + CFG::kAcc * kTcAccN <= CFG::kTmem, "TMEM budget");
+    static_assert(kAccCol0 + kTcAccN <= kTcTmemCols, "TMEM budget");
     const int seg = blockIdx.y;
     const int n = seg_len[seg];
     const int n_frames = cqt_frames(n);
@@ -874,13 +679,11 @@ __global__ void __launch_bounds__(kTcThreads, CFG::kMinBlocks) cqt_tc_kernel(con
             mbar_init(&sm.full_b[i], 1);
             mbar_init(&sm.empty_b[i], 1);
         }
-        for (int i = 0; i < 2; ++i) {
-            mbar_init(&sm.acc_full[i], 1);
-            mbar_init(&sm.acc_empty[i], kTcFrameWarps);
-        }
+        mbar_init(&sm.acc_full, 1);
+        mbar_init(&sm.acc_empty, kTcFrameWarps);
         fence_mbar_init();
     }
-    if (warp == kTcFrameWarps) tmem_alloc(&sm.tmem_base, CFG::kTmem);
+    if (warp == kTcFrameWarps) tmem_alloc(&sm.tmem_base, kTcTmemCols);
     fence_before_sync();
     __syncthreads();
     fence_after_sync();
@@ -908,10 +711,9 @@ __global__ void __launch_bounds__(kTcThreads, CFG::kMinBlocks) cqt_tc_kernel(con
             for (int j = 0; j < 4; ++j) part[a][j] = 0.0f;
 
         auto epilogue = [&](int o) {
-            const int buf = CFG::kAcc == 2 ? (o & 1) : 0;
-            mbar_wait_warp(&sm.acc_full[buf], (uint32_t)(CFG::kAcc == 2 ? (o >> 1) & 1 : o & 1), 100);
+            mbar_wait_warp(&sm.acc_full, (uint32_t)(o & 1), 100);
             fence_after_sync();
-            const uint32_t acc = tmem + lane_base + (uint32_t)(kAccCol0 + buf * kTcAccN);
+            const uint32_t acc = tmem + lane_base + (uint32_t)kAccCol0;
 #pragma unroll
             for (int a = 0; a < kQPer; ++a) {
                 switch (q * kQPer + a) {  // warp-uniform
@@ -923,14 +725,14 @@ __global__ void __launch_bounds__(kTcThreads, CFG::kMinBlocks) cqt_tc_kernel(con
             }
             fence_before_sync();
             __syncwarp();
-            if (lane == 0) mbar_arrive(&sm.acc_empty[buf]);
+            if (lane == 0) mbar_arrive(&sm.acc_empty);
         };
 
         // A rows stream through a cp.async ring (kPre k-tiles ahead, flat over octaves × k-tiles): thread (f, q) owns
         // kTcVals consecutive samples (kTcVals/4 16-byte chunks) of row f in every k-tile.  Zero padding outside [0, len)
         // comes from the src-size (zfill) form — row starts are multiples of 4 samples, so a chunk never straddles 0.
         // The per-tile address arithmetic is kept to a handful of 32-bit operations: this instruction stream, not the
-        // MMAs or the memory system, is what paces the kernel (NCFA_TC_DEBUG timing experiments).
+        // MMAs or the memory system, is what paces the kernel (timing experiments, profiles/r2l_cqt_debug.log).
         // The global side of the copies is coalesced: per cp.async instruction the warp's lanes (r8 = lane >> 2, c = lane & 3)
         // fetch the four 16-byte chunks (column half q) of EIGHT rows — 64 contiguous bytes per row — instead of one
         // chunk of 32 different rows (32 different cache lines per instruction at the upper octaves: the L1 tag stage,
@@ -968,8 +770,7 @@ __global__ void __launch_bounds__(kTcThreads, CFG::kMinBlocks) cqt_tc_kernel(con
                 ybase = ylev + row0;
             }
             const uint32_t slot_u32 = arow_u32 + (uint32_t)(it % kPre) * kSlotBytes + slot_off;
-            if (DBG && (dbg & 2)) {  // timing experiment: no A traffic
-            } else if (oct_fast) {
+            if (oct_fast) {
                 const float *src = ybase + kt * kTcKT;
 #pragma unroll
                 for (int j = 0; j < 4; ++j)
@@ -1038,7 +839,7 @@ __global__ void __launch_bounds__(kTcThreads, CFG::kMinBlocks) cqt_tc_kernel(con
             }
             __syncwarp();  // all lanes have read the slot before other lanes re-fill it (issue() of the next iteration)
             if (pending) {  // publish the PREVIOUS tile: its tcgen05.st had a whole iteration to land
-                if (!(DBG && (dbg & 8))) wait_st();
+                wait_st();
                 fence_before_sync();
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&sm.full_a[(it - 1) % kAS]);
@@ -1050,21 +851,14 @@ __global__ void __launch_bounds__(kTcThreads, CFG::kMinBlocks) cqt_tc_kernel(con
             tmem_st_vals(a0 + kTcKT, l);
             pending = true;
             if (kt == kKTiles - 1) {  // octave boundary (and the very last tile): publish before the epilogue
-                if (!(DBG && (dbg & 8))) wait_st();
+                wait_st();
                 fence_before_sync();
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&sm.full_a[st]);
                 pending = false;
-                // two accumulators: octave o−1 is read while the MMAs of octave o+1 run; one accumulator: the MMAs of
-                // the next octave wait for this read, so it has to happen right here
-                if (CFG::kAcc == 2) {
-                    if (o > 0) epilogue(o - 1);
-                } else {
-                    epilogue(o);
-                }
+                epilogue(o);  // one accumulator: the MMAs of the next octave wait for this read
             }
         }
-        if (CFG::kAcc == 2) epilogue(kOctaves - 1);
 
         // ---- combine the four column quarters of every frame, librosa.util.normalize(norm=inf) per frame, then the
         // tile's sum over frames (float64)
@@ -1102,10 +896,9 @@ __global__ void __launch_bounds__(kTcThreads, CFG::kMinBlocks) cqt_tc_kernel(con
         // ===================== MMA issuer (warp-uniform control flow, one elected lane issues) =====================
         constexpr uint32_t idesc = idesc_tf32(kTcFrames, kTcN);  // M 128 × N 80 × K 8
         for (int o = 0; o < kOctaves; ++o) {
-            const int buf = CFG::kAcc == 2 ? (o & 1) : 0;
-            mbar_wait_warp(&sm.acc_empty[buf], (uint32_t)((CFG::kAcc == 2 ? (o >> 1) & 1 : o & 1) ^ 1));
+            mbar_wait_warp(&sm.acc_empty, (uint32_t)((o & 1) ^ 1));
             fence_after_sync();
-            const uint32_t d = tmem + (uint32_t)(kAccCol0 + buf * kTcAccN);
+            const uint32_t d = tmem + (uint32_t)kAccCol0;
             for (int kt = 0; kt < kKTiles; ++kt) {
                 const int it = o * kKTiles + kt;
                 const int sa = it % kAS, sb = it % kBS;
@@ -1119,14 +912,13 @@ __global__ void __launch_bounds__(kTcThreads, CFG::kMinBlocks) cqt_tc_kernel(con
 #pragma unroll
                     for (int k = 0; k < kTcKT / 8; ++k) {
                         const uint64_t adv = (uint64_t)((k * 8 * 4) >> 4);  // 32 bytes per K = 8 step inside the swizzle row
-                        if (DBG && (dbg & 4)) continue;  // timing experiment: no MMAs
                         mma_tf32_ts(d, ah + 8 * k, bh + adv, idesc, (kt | k) != 0);  // 3×TF32: Ah·Bh + Al·Bh + Ah·Bl
                         mma_tf32_ts(d, al + 8 * k, bh + adv, idesc, 1);
                         mma_tf32_ts(d, ah + 8 * k, bl + adv, idesc, 1);
                     }
                     commit(&sm.empty_a[sa]);  // frees the A stage (TMEM) and the B stage (shared memory) of this tile together:
                                               // tcgen05.commit is the scarce operation of this pipeline, one per tile
-                    if (kt == kKTiles - 1) commit(&sm.acc_full[buf]);
+                    if (kt == kKTiles - 1) commit(&sm.acc_full);
                 }
                 __syncwarp();
             }
@@ -1138,12 +930,8 @@ __global__ void __launch_bounds__(kTcThreads, CFG::kMinBlocks) cqt_tc_kernel(con
             const int sb = it % kBS, kt = ((it % kKTiles) + kshift) & (kKTiles - 1);
             mbar_wait_warp(&sm.empty_a[sb], (uint32_t)(((it / kBS) & 1) ^ 1), 100);
             if (elect_one()) {
-                if (DBG && (dbg & 1) && it >= kBS) {  // timing experiment: no B traffic after the first ring fill
-                    mbar_arrive(&sm.full_b[sb]);
-                } else {
-                    mbar_arrive_expect_tx(&sm.full_b[sb], kTcBStageBytes);
-                    bulk_g2s(sm.b[sb], src + (size_t)kt * kTcBStageBytes, kTcBStageBytes, &sm.full_b[sb]);
-                }
+                mbar_arrive_expect_tx(&sm.full_b[sb], kTcBStageBytes);
+                bulk_g2s(sm.b[sb], src + (size_t)kt * kTcBStageBytes, kTcBStageBytes, &sm.full_b[sb]);
             }
             __syncwarp();
         }
@@ -1152,7 +940,7 @@ __global__ void __launch_bounds__(kTcThreads, CFG::kMinBlocks) cqt_tc_kernel(con
     __syncthreads();
     if (warp == kTcFrameWarps) {
         fence_after_sync();
-        tmem_dealloc(tmem, CFG::kTmem);
+        tmem_dealloc(tmem, kTcTmemCols);
     }
 }
 
@@ -1256,7 +1044,7 @@ extern "C" int ncfa_tuning_estimate_batched(const float *d_audio, const int64_t 
     return NCFA_OK;
 }
 
-static int chroma_tiles(int max_seg_len) { return (cqt_frames(max_seg_len) + kCqtTF - 1) / kCqtTF; }
+static int chroma_tiles(int max_seg_len) { return (cqt_frames(max_seg_len) + kPartialTF - 1) / kPartialTF; }
 
 extern "C" size_t ncfa_chroma_workspace_bytes(int n_seg, int max_seg_len) {
     if (n_seg <= 0 || max_seg_len < 0) return 0;
@@ -1292,58 +1080,22 @@ extern "C" int ncfa_chroma_mean_batched(const float *d_audio, const int64_t *d_s
         if (n_out <= 0) continue;
         ProfScope _p("decimate2_kernel", st);
         dim3 g((n_out + kDecOutPerCta - 1) / kDecOutPerCta, n_seg);
-        if (decimate_f64())
-            decimate2_kernel<double><<<g, 256, 0, st>>>(d_audio, d_seg_off, d_seg_len, level, pyr, stride,
-                                                        level >= 2 ? po.off[level - 1] : 0, po.off[level], ct.hb);
-        else
-            decimate2_kernel<float><<<g, 256, 0, st>>>(d_audio, d_seg_off, d_seg_len, level, pyr, stride,
-                                                       level >= 2 ? po.off[level - 1] : 0, po.off[level], ct.hb);
+        decimate2_kernel<<<g, 256, 0, st>>>(d_audio, d_seg_off, d_seg_len, level, pyr, stride,
+                                            level >= 2 ? po.off[level - 1] : 0, po.off[level], ct.hb);
         NCFA_LAUNCH_OK("decimate2_kernel");
     }
-    // NCFA_CQT_IMPL=simt selects the CUDA-core contraction (kept as the cross-check of the tensor-core kernel)
-    static int use_tc = -1;
-    if (use_tc < 0) {
-        const char *e = getenv("NCFA_CQT_IMPL");
-        use_tc = (e && strcmp(e, "simt") == 0) ? 0 : 1;
-    }
-    if ((rc = ensure_dynamic_smem((const void *)cqt_chroma_kernel, sizeof(CqtSmem)))) return rc;
-    if ((rc = ensure_dynamic_smem((const void *)cqt_tc_kernel<false, TcOne>, sizeof(TcSmem) + 1024))) return rc;
-    if ((rc = ensure_dynamic_smem((const void *)cqt_tc_kernel<true, TcOne>, sizeof(TcSmem) + 1024))) return rc;
-    if ((rc = ensure_dynamic_smem((const void *)cqt_tc_kernel<false, TcTwo>, sizeof(TcSmemT<TcTwo::kB, TcTwo::kPre>) + 1024))) return rc;
-    const int tiles = chroma_tiles(max_seg_len);  // partial[] stride (sized for the 32-frame tiles of the SIMT kernel)
-    if (use_tc) {
+    if ((rc = ensure_dynamic_smem((const void *)cqt_tc_kernel, sizeof(TcSmem) + 1024))) return rc;
+    const int tiles = chroma_tiles(max_seg_len);  // partial[] stride
+    {
         ProfScope _p("cqt_tc_kernel", st);
         dim3 g((cqt_frames(max_seg_len) + kTcFrames - 1) / kTcFrames, n_seg);
-        static int dbg = -1;
-        if (dbg < 0) {
-            const char *e = getenv("NCFA_TC_DEBUG");  // timing experiments only (results are wrong when non-zero)
-            dbg = e ? atoi(e) : 0;
-        }
-        static int impl = -1;  // 0: two shallow CTAs per SM (default), 1: one deep CTA per SM
-        if (impl < 0) {
-            const char *e = getenv("NCFA_CQT_IMPL");  // "tc1": the one-CTA-per-SM pipeline shape (before/after, cross-check)
-            impl = (e && strcmp(e, "tc1") == 0) ? 1 : 0;
-        }
-        if (dbg)
-            cqt_tc_kernel<true, TcOne><<<g, kTcThreads, sizeof(TcSmem) + 1024, st>>>(d_audio, d_seg_off, d_seg_len, pyr, po,
-                                                                                     d_tuning_idx, ct.Bimg, tiles, partial, dbg);
-        else if (impl == 1)
-            cqt_tc_kernel<false, TcOne><<<g, kTcThreads, sizeof(TcSmem) + 1024, st>>>(d_audio, d_seg_off, d_seg_len, pyr, po,
-                                                                                      d_tuning_idx, ct.Bimg, tiles, partial, 0);
-        else
-            cqt_tc_kernel<false, TcTwo><<<g, kTcThreads, sizeof(TcSmemT<TcTwo::kB, TcTwo::kPre>) + 1024, st>>>(
-                d_audio, d_seg_off, d_seg_len, pyr, po, d_tuning_idx, ct.Bimg, tiles, partial, 0);
-        NCFA_LAUNCH_OK("cqt_tc_kernel");
-    } else {
-        ProfScope _p("cqt_chroma_kernel", st);
-        dim3 g(tiles, n_seg);
-        cqt_chroma_kernel<<<g, kCqtThreads, sizeof(CqtSmem), st>>>(d_audio, d_seg_off, d_seg_len, pyr, po, d_tuning_idx,
-                                                                    ct.K, tiles, partial);
-        NCFA_LAUNCH_OK("cqt_chroma_kernel");
+        cqt_tc_kernel<<<g, kTcThreads, sizeof(TcSmem) + 1024, st>>>(d_audio, d_seg_off, d_seg_len, pyr, po, d_tuning_idx,
+                                                                   ct.Bimg, tiles, partial);
     }
+    NCFA_LAUNCH_OK("cqt_tc_kernel");
     {
         ProfScope _p("chroma_mean_kernel", st);
-        chroma_mean_kernel<<<n_seg, 32, 0, st>>>(d_seg_len, tiles, use_tc ? kTcFrames : kCqtTF, partial, d_chroma);
+        chroma_mean_kernel<<<n_seg, 32, 0, st>>>(d_seg_len, tiles, kTcFrames, partial, d_chroma);
     }
     NCFA_LAUNCH_OK("chroma_mean_kernel");
     return NCFA_OK;

@@ -93,7 +93,7 @@ static int upload(const std::vector<T> &h, const T **d) {
 }
 
 // Host side of the Slaney mel bank (librosa.filters.mel(htk=False, norm='slaney'), SURVEY Appendix A.2): packed
-// band-major weights plus the lane-transposed, bank-conflict-free copy of the warp-per-frame kernels.
+// band-major weights, and from them the lane-transposed, bank-conflict-free copy the onset kernel reads.
 struct MelHost {
     std::vector<float> w;          // packed non-zero weights, band-major
     std::vector<int> start, bin0;  // [129], [128]
@@ -229,7 +229,7 @@ int get_tables(int sr, Tables *out) {
         return NCFA_OK;
     }
     NCFA_REQUIRE(sr >= 2000 && sr <= 768000, "sample rate out of range");
-    const int n_fft = NCFA_N_FFT, n_mels = NCFA_N_MELS;
+    const int n_fft = NCFA_N_FFT;
     const double PI = 3.14159265358979323846;
     std::vector<float> hann(n_fft);
     for (int i = 0; i < n_fft; ++i) hann[i] = (float)(0.5 - 0.5 * cos(2.0 * PI * i / n_fft));
@@ -248,8 +248,6 @@ int get_tables(int sr, Tables *out) {
         const int mrc = build_mel_host(sr, &mh);
         if (mrc) return mrc;
     }
-    std::vector<float> &w = mh.w;
-    std::vector<int> &start = mh.start, &bin0 = mh.bin0;
     DeviceTables dt;
     int rc;
     for (int q = 0; q < 4; ++q) {
@@ -259,49 +257,9 @@ int get_tables(int sr, Tables *out) {
     dt.t.mel_wt_rows = mh.rows;
     if ((rc = upload(mh.wt, &dt.t.mel_wt))) return rc;
     if ((rc = upload(mh.lb, &dt.t.mel_lane_bin0))) return rc;
-    // band-major float4 copy + the split of the bands over the 16 warps of the tile kernel
-    {
-        std::vector<float4> w4;
-        std::vector<int> start4(n_mels + 1);
-        for (int m = 0; m < n_mels; ++m) {
-            start4[m] = (int)w4.size();
-            for (int i = start[m]; i < start[m + 1]; i += 4) {
-                float q[4] = {0.f, 0.f, 0.f, 0.f};
-                for (int j = 0; j < 4 && i + j < start[m + 1]; ++j) q[j] = w[i + j];
-                w4.push_back(make_float4(q[0], q[1], q[2], q[3]));
-            }
-            if (bin0[m] + 4 * ((int)w4.size() - start4[m]) > 1028) {
-                set_error("mel band %d reaches past the padded power tile at sr=%d", m, sr);
-                return NCFA_E_OVERFLOW;
-            }
-        }
-        start4[n_mels] = (int)w4.size();
-        if (w4.empty()) w4.push_back(make_float4(0.f, 0.f, 0.f, 0.f));
-        // cost of a band in the mel phase ~ 4 per float4 group + a fixed epilogue; contiguous split into 16 parts
-        auto cost = [&](int m) { return 4 * (start4[m + 1] - start4[m]) + 8; };
-        long total = 0;
-        for (int m = 0; m < n_mels; ++m) total += cost(m);
-        int m = 0;
-        long acc = 0;
-        for (int wp = 0; wp < 16; ++wp) {
-            dt.t.mel_warp_band[wp] = m;
-            const long target = total * (wp + 1) / 16;
-            while (m < n_mels && acc + cost(m) / 2 <= target) {
-                acc += cost(m);
-                ++m;
-            }
-        }
-        dt.t.mel_warp_band[16] = n_mels;
-        if ((rc = upload(w4, &dt.t.mel_w4))) return rc;
-        if ((rc = upload(start4, &dt.t.mel_start4))) return rc;
-    }
     if ((rc = upload(hann, &dt.t.hann))) return rc;
     if ((rc = upload(tw1024, &dt.t.tw1024))) return rc;
     if ((rc = upload(tw2048, &dt.t.tw2048))) return rc;
-    if ((rc = upload(w, &dt.t.mel_w))) return rc;
-    if ((rc = upload(start, &dt.t.mel_start))) return rc;
-    if ((rc = upload(bin0, &dt.t.mel_bin0))) return rc;
-    dt.t.mel_nnz = (int)w.size();
     dt.t.sr = sr;
     g_tables[key] = dt;
     *out = dt.t;

@@ -74,22 +74,12 @@ struct Tables {
     const float *hann;        // [2048] periodic Hann, float32(float64 value)
     const float2 *tw1024;     // [32][32]: tw[k1*32 + n2] = exp(-2πi·k1·n2/1024)
     const float2 *tw2048;     // [32]: exp(-2πi·l/2048), l = lane
-    const float *mel_w;       // packed non-zero weights, band-major
-    const int *mel_start;     // [129] start of band m in mel_w
-    const int *mel_bin0;      // [128] first FFT bin of band m
-    int mel_nnz;
     int sr;
-    // lane-transposed mel bank for the warp-per-frame kernels: lane l owns bands l, 63−l, 64+l, 127−l (group q = 0..3);
+    // lane-transposed mel bank of the onset kernel: lane l owns bands l, 63−l, 64+l, 127−l (group q = 0..3);
     // mel_wt[(mel_qoff[q] + i)·32 + l] = i-th weight of that band (0 beyond its support), i < mel_qw[q]
     const float *mel_wt;
     const int *mel_lane_bin0;  // [4][32] first FFT bin of the band of (q, lane)
     int mel_qoff[4], mel_qw[4], mel_wt_rows;
-    // band-major bank for the tile kernel (stft_onset.cu): band m = float4 groups [mel_start4[m], mel_start4[m+1]) of
-    // mel_w4, first weight at bin mel_bin0[m], zero padded to a multiple of four; warp w of the 16 owns the bands
-    // [mel_warp_band[w], mel_warp_band[w+1]) (balanced by weight count)
-    const float4 *mel_w4;
-    const int *mel_start4;    // [129]
-    int mel_warp_band[17];
 };
 __host__ __device__ inline int mel_band_of(int q, int lane) {
     return q == 0 ? lane : (q == 1 ? 63 - lane : (q == 2 ? 64 + lane : 127 - lane));

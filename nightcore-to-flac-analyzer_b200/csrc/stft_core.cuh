@@ -258,123 +258,4 @@ __device__ __forceinline__ void warp_power_spectrum_global2(const float *__restr
     warp_power_spectrum_regs2(a, b, tw, scra, scrb, twl, lane);
 }
 
-// ---- tile variant (stft_onset.cu): the power spectrum of a frame becomes one COLUMN of a CTA-wide [bin][frame] tile
-// (row stride kPStride floats) so that a later phase can walk bins with lane = frame.  The per-warp transpose tile holds
-// one float per element (real parts, then imaginary parts through the same 4.2 KB) to leave room for the power tile.
-constexpr int kPStride = 33;   // floats per bin row of the power tile (32 frames + 1: stores of one frame hit 32 banks)
-constexpr int kPRows = 1028;   // 1025 bins + rows that only ever meet zero mel weights
-
-template <int K2>
-struct PostStageTile {
-    // same arithmetic as PostStage; bin k of this frame goes to pcol[k * kPStride]
-    static __device__ __forceinline__ void run(const cf (&v)[32], int lane, cf twl, float *pcol) {
-        cf zk = v[br5(K2)];
-        cf own = v[br5((32 - K2) & 31)];
-        cf snd = v[br5(31 - K2)];
-        int src = (32 - lane) & 31;
-        cf p;
-        p.x = __shfl_sync(0xffffffffu, snd.x, src);
-        p.y = __shfl_sync(0xffffffffu, snd.y, src);
-        if (lane == 0) p = own;
-        cf e = cscale(cadd_conj(zk, p), 0.5f);            // ½(Z[k] + conj Z[N−k])
-        cf o = cscale(cmul_mi(csub_conj(zk, p)), 0.5f);   // (Z[k] − conj Z[N−k]) / (2i)
-        cf w = mul_w64<K2>(twl);  // W_2048^(lane + 32·K2)
-        cf wo = cmul(o, w);
-        cf x = cadd(e, wo);
-        cf y = csub(e, wo);
-        pcol[(lane + 32 * K2) * kPStride] = x.x * x.x + x.y * x.y;
-        pcol[(1024 - lane - 32 * K2) * kPStride] = y.x * y.x + y.y * y.y;
-        if constexpr (K2 + 1 < 16) PostStageTile<K2 + 1>::run(v, lane, twl, pcol);
-        if constexpr (K2 == 0) {
-            if (lane == 0) {
-                cf z = v[br5(16)];
-                pcol[512 * kPStride] = z.x * z.x + z.y * z.y;
-            }
-        }
-    }
-};
-
-// v as in warp_power_spectrum_regs; scr: per-warp scratch of 32*kScrStride floats; pcol: this frame's column of the tile
-__device__ __forceinline__ void warp_power_spectrum_regs_tile(cf (&v)[32], const float2 *tw, float *scr, float *pcol,
-                                                              cf twl, int lane) {
-    fft32_dif(v);
-#pragma unroll
-    for (int k1 = 0; k1 < 32; ++k1) {
-        float2 t = tw[k1 * 32 + lane];
-        v[br5(k1)] = cmul(v[br5(k1)], cf{t.x, t.y});
-    }
-#pragma unroll
-    for (int k1 = 0; k1 < 32; ++k1) scr[k1 * kScrStride + lane] = v[br5(k1)].x;
-    __syncwarp();
-#pragma unroll
-    for (int n2 = 0; n2 < 32; ++n2) v[n2].x = scr[lane * kScrStride + n2];  // the old real parts are dead
-    __syncwarp();
-    // imaginary parts still sit where the first FFT left them: slot br5(k1) holds bin k1
-    // (v[n2].x above overwrote only .x components)
-#pragma unroll
-    for (int k1 = 0; k1 < 32; ++k1) scr[k1 * kScrStride + lane] = v[br5(k1)].y;
-    __syncwarp();
-#pragma unroll
-    for (int n2 = 0; n2 < 32; ++n2) v[n2].y = scr[lane * kScrStride + n2];
-    __syncwarp();
-    fft32_dif(v);
-    PostStageTile<0>::run(v, lane, twl, pcol);
-}
-
-__device__ __forceinline__ void warp_power_spectrum_global_tile(const float *__restrict__ src, int64_t pos, int len,
-                                                                const float *hann, const float2 *tw, float *scr,
-                                                                float *pcol, cf twl, int lane) {
-    cf v[32];
-    const bool inside = pos >= 0 && pos + 2048 <= (int64_t)len;
-    const float *fr = src + pos;
-    if (inside && ((reinterpret_cast<uintptr_t>(fr) & 7u) == 0)) {
-#pragma unroll
-        for (int n1 = 0; n1 < 32; ++n1) {
-            const float2 xs = __ldg(reinterpret_cast<const float2 *>(fr + 64 * n1 + 2 * lane));
-            const float2 ws = *reinterpret_cast<const float2 *>(hann + 64 * n1 + 2 * lane);
-            v[n1] = cmul_elem(cf{xs.x, xs.y}, cf{ws.x, ws.y});
-        }
-    } else {
-#pragma unroll
-        for (int n1 = 0; n1 < 32; ++n1) {
-            const int64_t p = pos + 64 * n1 + 2 * lane;
-            const float x0 = (p >= 0 && p < len) ? __ldg(src + p) : 0.0f;
-            const float x1 = (p + 1 >= 0 && p + 1 < len) ? __ldg(src + p + 1) : 0.0f;
-            const float2 ws = *reinterpret_cast<const float2 *>(hann + 64 * n1 + 2 * lane);
-            v[n1] = cmul_elem(cf{x0, x1}, cf{ws.x, ws.y});
-        }
-    }
-    warp_power_spectrum_regs_tile(v, tw, scr, pcol, twl, lane);
-}
-
-// fr: 2048 samples (shared), hann: 2048 (shared), tw: [32][32] W_1024 twiddles (shared),
-// scr: per-warp scratch of 32*kScrStride float2; on return its first 1025 floats hold |X[k]|^2.
-__device__ __forceinline__ void warp_power_spectrum(const float *fr, const float *hann, const float2 *tw, float2 *scr,
-                                                    cf twl, int lane) {
-    cf v[32];
-#pragma unroll
-    for (int n1 = 0; n1 < 32; ++n1) {
-        float2 xs = *reinterpret_cast<const float2 *>(fr + 64 * n1 + 2 * lane);
-        float2 ws = *reinterpret_cast<const float2 *>(hann + 64 * n1 + 2 * lane);
-        v[n1] = cmul_elem(cf{xs.x, xs.y}, cf{ws.x, ws.y});
-    }
-    fft32_dif(v);
-#pragma unroll
-    for (int k1 = 0; k1 < 32; ++k1) {
-        float2 t = tw[k1 * 32 + lane];
-        cf y = cmul(v[br5(k1)], cf{t.x, t.y});
-        scr[k1 * kScrStride + lane] = make_float2(y.x, y.y);
-    }
-    __syncwarp();
-#pragma unroll
-    for (int n2 = 0; n2 < 32; ++n2) {
-        float2 t = scr[lane * kScrStride + n2];
-        v[n2] = cf{t.x, t.y};
-    }
-    __syncwarp();
-    fft32_dif(v);
-    PostStage<0>::run(v, lane, twl, reinterpret_cast<float *>(scr));
-    __syncwarp();
-}
-
 }  // namespace ncfa

@@ -4,94 +4,23 @@
 // Replaces librosa.onset.onset_strength as called at tempo.py:44 (hop 512, one 10 s window per
 // segment) and tempo.py:158 (hop 64, whole track per segment).  SURVEY.md Appendix A.1/A.2.
 //
-// Kernel 1 layout: persistent CTAs, one per SM, 16 warps each; the constant tables (Hann, W_1024 twiddles,
-// lane-transposed mel bank) are staged in shared memory once per CTA.  **One warp = one frame**: the warp
-// loads its 2048 samples straight from global memory (coalesced float2; consecutive frames are handled by
-// the 16 warps of one SM at the same time, so L1 serves the 97 % overlap at hop 64), packs them as 1024
-// complex values (lane n2 holds z[32·n1+n2] in registers), runs a 32-point FFT over n1, multiplies by
-// W_1024^(n2·k1), transposes through a padded per-warp shared tile, runs the second 32-point FFT and
-// un-packs the real spectrum with one shuffle per complex value.  The power spectrum goes through the
-// same per-warp tile into the sparse mel projection (lane owns bands l, 63−l, 64+l, 127−l; weights are
-// stored lane-transposed so the reads are bank-conflict free).  No block-level synchronisation in the loop.
-#include <stdlib.h>
+// Kernel 1 layout: persistent CTAs, one per SM; the constant tables (Hann, W_1024 twiddles, lane-transposed mel bank)
+// are staged in shared memory once per CTA.  **One warp = one pair of frames** (2p, 2p+1) of a segment: the warp loads
+// their samples straight from global memory (coalesced float2; consecutive pairs are handled by the warps of one SM at
+// the same time, so L1 serves the 97 % overlap at hop 64), packs each frame as 1024 complex values (lane n2 holds
+// z[32·n1+n2] in registers), runs a 32-point FFT over n1, multiplies by W_1024^(n2·k1), transposes through a padded
+// per-warp shared tile, runs the second 32-point FFT and un-packs the real spectrum with one shuffle per complex value
+// (stft_core.cuh: warp_power_spectrum_global2).  Both frames go through one instruction stream: the Hann window, the
+// W_1024 twiddles, W_2048^k and the mel weights are read from shared memory once per pair, and at hop 64 the two frames
+// share 31 of their 32 register loads.  The power spectra go through the same per-warp tiles into the sparse mel
+// projection (lane owns bands l, 63−l, 64+l, 127−l; weights are stored lane-transposed so the reads are bank-conflict
+// free).  No block-level synchronisation in the loop.  Measured on B200 (round 1/2, profiles/): the pair form needs ~340
+// shared-memory/L1 wavefronts per frame against 510 for one frame per warp, and its wider register budget removes the
+// spills of that form; a CTA-wide tile form (lane = frame in the mel phase) was 7–19 % slower and latency bound.
 #include "stft_core.cuh"
 
 namespace ncfa {
 
-constexpr int kWarps = 20;
-constexpr int kThreads = kWarps * 32;
-constexpr int kMelRowsMax = 128;
-
-struct OnsetSmem {
-    float hann[2048];
-    float2 tw[1024];
-    float melwt[kMelRowsMax * 32];
-    int lane_bin0[4 * 32];
-    float2 scr[kWarps][32 * kScrStride];
-};
-
-__global__ void __launch_bounds__(kThreads, 1) stft_logmel_kernel(const float *__restrict__ audio,
-                                                                  const int64_t *__restrict__ seg_off,
-                                                                  const int32_t *__restrict__ seg_len, int n_seg,
-                                                                  int hop, int frame_stride, Tables tb,
-                                                                  float *__restrict__ S, unsigned *__restrict__ seg_max) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    OnsetSmem &sm = *reinterpret_cast<OnsetSmem *>(smem_raw);
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    for (int i = tid; i < 2048; i += kThreads) sm.hann[i] = tb.hann[i];
-    for (int i = tid; i < 1024; i += kThreads) sm.tw[i] = tb.tw1024[i];
-    for (int i = tid; i < tb.mel_wt_rows * 32; i += kThreads) sm.melwt[i] = tb.mel_wt[i];
-    for (int i = tid; i < 4 * 32; i += kThreads) sm.lane_bin0[i] = tb.mel_lane_bin0[i];
-    __syncthreads();
-
-    const cf twl = cf{tb.tw2048[lane].x, tb.tw2048[lane].y};
-    float2 *scr = sm.scr[warp];
-    const float *pw = reinterpret_cast<const float *>(scr);
-    int b0[4];
-#pragma unroll
-    for (int q = 0; q < 4; ++q) b0[q] = sm.lane_bin0[q * 32 + lane];
-    const int64_t total = (int64_t)n_seg * frame_stride;
-    int cur_seg = -1;
-    float cur_max = -INFINITY;
-    // items (seg, frame) are dealt in groups of kWarps consecutive frames per CTA
-    for (int64_t item = (int64_t)blockIdx.x * kWarps + warp; item < total; item += (int64_t)gridDim.x * kWarps) {
-        const int seg = (int)(item / frame_stride);
-        const int frame = (int)(item - (int64_t)seg * frame_stride);
-        const int len = seg_len[seg];
-        if (frame >= 1 + len / hop) continue;
-        if (seg != cur_seg) {
-            if (cur_seg >= 0 && lane == 0) atomicMax(seg_max + cur_seg, float_to_ordered(cur_max));
-            cur_seg = seg;
-            cur_max = -INFINITY;
-        }
-        warp_power_spectrum_global(audio + seg_off[seg], (int64_t)frame * hop - 1024, len, sm.hann, sm.tw, scr, twl, lane);
-
-        float *Sout = S + ((size_t)seg * frame_stride + frame) * NCFA_N_MELS;
-        float vmax = -INFINITY;
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-            const float *wt = sm.melwt + (size_t)tb.mel_qoff[q] * 32 + lane;
-            const float *pk = pw + b0[q];
-            const int nw = tb.mel_qw[q];
-            float acc = 0.0f;
-            for (int i = 0; i < nw; ++i) acc = fmaf(wt[i * 32], pk[i], acc);  // zero weights beyond the band's support
-            const float db = 10.0f * log10f(fmaxf(1e-10f, acc));
-            Sout[mel_band_of(q, lane)] = db;
-            vmax = fmaxf(vmax, db);
-        }
-        cur_max = fmaxf(cur_max, warp_max(vmax));
-        __syncwarp();
-    }
-    if (cur_seg >= 0 && lane == 0) atomicMax(seg_max + cur_seg, float_to_ordered(cur_max));
-}
-
-// ---- two frames per warp (the default form) ---------------------------------------------------------------------------
-// Same decomposition, but a warp owns the PAIR of frames (2p, 2p+1) of a segment and runs both through one instruction
-// stream (stft_core.cuh: warp_power_spectrum_global2): the Hann window, the W_1024 twiddles, W_2048^k and the mel
-// weights are read from shared memory once per pair, at hop 64 the two frames share 31 of their 32 register loads, and
-// the wider register budget (10 warps per SM instead of 20) removes the spills of the one-frame form.  Per frame:
-// ~340 shared-memory/L1 wavefronts instead of 510.  The per-frame arithmetic is unchanged, so the log-mel values — and
-// everything downstream — are bit-identical to the one-frame form (NCFA_STFT_IMPL=warp1, kept as a cross-check).
 constexpr int kWarps2Max = 12;  // 168 registers per thread × 384 threads fill the register file
 constexpr size_t kScrBytes2 = 2 * 32 * kScrStride * sizeof(float2);  // two transpose tiles per warp
 
@@ -222,152 +151,6 @@ __global__ void __launch_bounds__(256) flux_kernel(const float *__restrict__ S, 
     }
 }
 
-// ---- tile form (cross-check) ------------------------------------------------------------------------------------------
-// The warp-per-frame kernel above spends more shared-memory wavefronts in the mel projection (lane-dependent, bank
-// conflicting reads of the power spectrum) than in the FFT.  Here a CTA of 16 warps works on a TILE of 32 consecutive
-// frames of one segment in two phases:
-//   1. FFT phase: warp w transforms frames w and w+16 of the tile; the power spectrum of frame f becomes column f of
-//      a shared [1028 bins][33] tile (same arithmetic as above; transposes go through a 4.2 KB per-warp float tile,
-//      real then imaginary parts, to make room);
-//   2. mel phase: lane = frame, warp w owns a contiguous group of mel bands (balanced by weight count); the weights
-//      are warp-uniform float4 loads, the power reads are conflict free — 1 shared wavefront + 1 FFMA per
-//      (band, bin) pair for 32 frames at once, i.e. 63 of each per frame instead of ~360 wavefronts.
-// The log-mel scratch is tile-major, S[tile][band][32 frames] (coalesced stores here, coalesced loads in the flux
-// kernel).  Sums run in the same order as in the warp form, so both produce the same onset envelope bit for bit.
-constexpr int kTileWarps = 16;
-constexpr int kTileThreads = kTileWarps * 32;
-constexpr int kTileFrames = 32;
-
-struct TileSmem {
-    float hann[2048];
-    float2 tw[1024];
-    float scr[kTileWarps][32 * kScrStride];
-    float P[kPRows * kPStride];
-};
-
-__global__ void __launch_bounds__(kTileThreads, 1) stft_logmel_tile_kernel(const float *__restrict__ audio,
-                                                                           const int64_t *__restrict__ seg_off,
-                                                                           const int32_t *__restrict__ seg_len,
-                                                                           int n_seg, int hop, int tiles_per_seg,
-                                                                           Tables tb, float *__restrict__ S,
-                                                                           unsigned *__restrict__ seg_max) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    TileSmem &sm = *reinterpret_cast<TileSmem *>(smem_raw);
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    for (int i = tid; i < 2048; i += kTileThreads) sm.hann[i] = tb.hann[i];
-    for (int i = tid; i < 1024; i += kTileThreads) sm.tw[i] = tb.tw1024[i];
-    for (int i = tid; i < kPRows * kPStride; i += kTileThreads) sm.P[i] = 0.0f;  // padding rows must stay finite
-    __syncthreads();
-
-    const cf twl = cf{tb.tw2048[lane].x, tb.tw2048[lane].y};
-    const int mb0 = tb.mel_warp_band[warp], mb1 = tb.mel_warp_band[warp + 1];
-    const int total = n_seg * tiles_per_seg;
-    int cur_seg = -1;
-    float cur_max = -INFINITY;
-    for (int tile = blockIdx.x; tile < total; tile += gridDim.x) {
-        const int seg = tile / tiles_per_seg;
-        const int f0 = (tile - seg * tiles_per_seg) * kTileFrames;
-        const int len = seg_len[seg];
-        const int n_frames = 1 + len / hop;
-        if (f0 >= n_frames) continue;  // CTA-uniform
-        const float *src = audio + seg_off[seg];
-#pragma unroll 1
-        for (int r = 0; r < kTileFrames / kTileWarps; ++r) {
-            const int f = warp + kTileWarps * r;
-            if (f0 + f < n_frames)
-                warp_power_spectrum_global_tile(src, (int64_t)(f0 + f) * hop - 1024, len, sm.hann, sm.tw, sm.scr[warp],
-                                                sm.P + f, twl, lane);
-        }
-        __syncthreads();
-        if (seg != cur_seg) {
-            if (cur_seg >= 0 && lane == 0) atomicMax(seg_max + cur_seg, float_to_ordered(cur_max));
-            cur_seg = seg;
-            cur_max = -INFINITY;
-        }
-        const bool valid = f0 + lane < n_frames;
-        float *Sout = S + (size_t)tile * (NCFA_N_MELS * kTileFrames) + lane;
-        float vmax = -INFINITY;
-        for (int m = mb0; m < mb1; ++m) {
-            const int g0 = __ldg(tb.mel_start4 + m), g1 = __ldg(tb.mel_start4 + m + 1);
-            const float4 *wq = tb.mel_w4 + g0;
-            const float *p = sm.P + __ldg(tb.mel_bin0 + m) * kPStride + lane;
-            float acc = 0.0f;
-            for (int g = 0; g < g1 - g0; ++g) {
-                const float4 wv = __ldg(wq + g);
-                acc = fmaf(wv.x, p[0], acc);
-                acc = fmaf(wv.y, p[kPStride], acc);
-                acc = fmaf(wv.z, p[2 * kPStride], acc);
-                acc = fmaf(wv.w, p[3 * kPStride], acc);
-                p += 4 * kPStride;
-            }
-            const float db = 10.0f * log10f(fmaxf(1e-10f, acc));
-            if (valid) {
-                Sout[m * kTileFrames] = db;
-                vmax = fmaxf(vmax, db);
-            }
-        }
-        cur_max = fmaxf(cur_max, warp_max(vmax));
-        __syncthreads();  // the next tile's FFT phase overwrites P
-    }
-    if (cur_seg >= 0 && lane == 0) atomicMax(seg_max + cur_seg, float_to_ordered(cur_max));
-}
-
-// flux over the tile-major scratch: one thread per output frame walks the 128 bands of frames j-pad and j-pad+1
-// (lanes = consecutive frames: coalesced), summing in the order of flux_kernel (4 bands per partial, xor tree).
-__global__ void __launch_bounds__(128) flux_tile_kernel(const float *__restrict__ S, const unsigned *__restrict__ seg_max,
-                                                        const int32_t *__restrict__ seg_len, int hop, int tiles_per_seg,
-                                                        int pad, float *__restrict__ onset,
-                                                        const int64_t *__restrict__ onset_off) {
-    const int seg = blockIdx.y;
-    const int n_frames = 1 + seg_len[seg] / hop;
-    const int j = blockIdx.x * 128 + threadIdx.x;
-    if (j >= n_frames) return;
-    float *out = onset + onset_off[seg];
-    if (j < pad) {
-        out[j] = 0.0f;
-        return;
-    }
-    const float floor_db = ordered_to_float(seg_max[seg]) - 80.0f;
-    const int ja = j - pad, jb = ja + 1;
-    const float *base = S + (size_t)seg * tiles_per_seg * (NCFA_N_MELS * kTileFrames);
-    const float *pa = base + (size_t)(ja >> 5) * (NCFA_N_MELS * kTileFrames) + (ja & 31);
-    const float *pb = base + (size_t)(jb >> 5) * (NCFA_N_MELS * kTileFrames) + (jb & 31);
-    float q[32];
-#pragma unroll
-    for (int l = 0; l < 32; ++l) {
-        float s = fmaxf(0.0f, fmaxf(pb[(4 * l) * kTileFrames], floor_db) - fmaxf(pa[(4 * l) * kTileFrames], floor_db));
-        s += fmaxf(0.0f, fmaxf(pb[(4 * l + 1) * kTileFrames], floor_db) - fmaxf(pa[(4 * l + 1) * kTileFrames], floor_db));
-        s += fmaxf(0.0f, fmaxf(pb[(4 * l + 2) * kTileFrames], floor_db) - fmaxf(pa[(4 * l + 2) * kTileFrames], floor_db));
-        s += fmaxf(0.0f, fmaxf(pb[(4 * l + 3) * kTileFrames], floor_db) - fmaxf(pa[(4 * l + 3) * kTileFrames], floor_db));
-        q[l] = s;
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1)
-#pragma unroll
-        for (int l = 0; l < o; ++l) q[l] = q[l] + q[l + o];
-    out[j] = q[0] * (1.0f / NCFA_N_MELS);
-}
-
-// measured on B200: the tile form was 7 % (hop 64) to 19 % (hop 512) SLOWER than the warp form when both were scalar
-// (profiles r1ai), and it gained nothing from the packed-FP32 FFT that sped the warp form up (109 vs 78 ms per 250 pairs,
-// r1bj): with 16 warps, two block barriers per tile and four shared round trips per transpose it is latency bound, not
-// issue bound.  The warp form stays the default; the tile form is kept as a cross-check (NCFA_STFT_IMPL=tile).
-static bool use_warp_form() {
-    static const bool v = [] {
-        const char *e = getenv("NCFA_STFT_IMPL");
-        return !(e && strcmp(e, "tile") == 0);
-    }();
-    return v;
-}
-// NCFA_STFT_IMPL=warp1: the one-frame-per-warp form (cross-check of the two-frame default)
-static bool use_one_frame_form() {
-    static const bool v = [] {
-        const char *e = getenv("NCFA_STFT_IMPL");
-        return e && strcmp(e, "warp1") == 0;
-    }();
-    return v;
-}
-
 }  // namespace ncfa
 
 using namespace ncfa;
@@ -397,55 +180,21 @@ extern "C" int ncfa_onset_strength_batched(const float *d_audio, const int64_t *
     if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     const int frames = 1 + max_seg_len / hop;
-    const int tiles_per_seg = (frames + kTileFrames - 1) / kTileFrames;
+    const int tiles_per_seg = (frames + 31) / 32;  // the workspace is sized in whole tiles of 32 frames
     float *S = (float *)d_workspace;
-    unsigned *seg_max =
-        (unsigned *)((char *)d_workspace + align_up((size_t)n_seg * tiles_per_seg * kTileFrames * NCFA_N_MELS * 4, 256));
+    unsigned *seg_max = (unsigned *)((char *)d_workspace + align_up((size_t)n_seg * tiles_per_seg * 32 * NCFA_N_MELS * 4, 256));
     NCFA_CUDA_OK(cudaMemsetAsync(seg_max, 0, (size_t)n_seg * 4, st));
     int n_sm = 0;
-    const int pad_t = 1 + NCFA_N_FFT / (2 * hop);
-    if (!use_warp_form()) {
-        NCFA_REQUIRE((int64_t)n_seg * tiles_per_seg < (int64_t)1 << 31, "too many frame tiles in one call");
-        if ((rc = ensure_dynamic_smem((const void *)stft_logmel_tile_kernel, sizeof(TileSmem)))) return rc;
-        if ((rc = sm_count(&n_sm))) return rc;
-        {
-            const int64_t tiles = (int64_t)n_seg * tiles_per_seg;
-            const int grid = (int)(tiles < n_sm ? tiles : n_sm);  // persistent: one CTA per SM
-            ProfScope _p(hop <= 128 ? "stft_logmel_kernel[hop<=128]" : "stft_logmel_kernel[hop>128]", st);
-            stft_logmel_tile_kernel<<<grid, kTileThreads, sizeof(TileSmem), st>>>(d_audio, d_seg_off, d_seg_len, n_seg, hop,
-                                                                                 tiles_per_seg, tb, S, seg_max);
-        }
-        NCFA_LAUNCH_OK("stft_logmel_tile_kernel");
-        dim3 g2((frames + 127) / 128, n_seg);
-        {
-            ProfScope _p("flux_kernel", st);
-            flux_tile_kernel<<<g2, 128, 0, st>>>(S, seg_max, d_seg_len, hop, tiles_per_seg, pad_t, d_onset, d_onset_off);
-        }
-        NCFA_LAUNCH_OK("flux_tile_kernel");
-        return NCFA_OK;
-    }
     if ((rc = sm_count(&n_sm))) return rc;
-    if (use_one_frame_form()) {
-        if ((rc = ensure_dynamic_smem((const void *)stft_logmel_kernel, sizeof(OnsetSmem)))) return rc;
-        const int64_t groups = ((int64_t)n_seg * frames + kWarps - 1) / kWarps;
-        const int grid = (int)(groups < n_sm ? groups : n_sm);  // persistent: one CTA per SM
-        ProfScope _p(hop <= 128 ? "stft_logmel_kernel[hop<=128]" : "stft_logmel_kernel[hop>128]", st);
-        stft_logmel_kernel<<<grid, kThreads, sizeof(OnsetSmem), st>>>(d_audio, d_seg_off, d_seg_len, n_seg, hop, frames, tb,
-                                                                  S, seg_max);
-    } else {
-        // as many warps as the 227 KB of shared memory hold (12 at 22 050 Hz: 95 mel-weight rows)
-        static const int env_warps = [] {
-            const char *e = getenv("NCFA_STFT_WARPS");
-            return e ? atoi(e) : 0;
-        }();
-        const size_t fixed = onset2_fixed_bytes(tb.mel_wt_rows);
-        int warps = (int)((232448 - fixed) / kScrBytes2);
-        if (warps > kWarps2Max) warps = kWarps2Max;
-        if (env_warps >= 1 && env_warps < warps) warps = env_warps;
-        NCFA_REQUIRE(warps >= 1, "mel table too large for shared memory");
-        const size_t smem = fixed + (size_t)warps * kScrBytes2;
-        const int64_t groups = ((int64_t)n_seg * ((frames + 1) / 2) + warps - 1) / warps;
-        const int grid = (int)(groups < n_sm ? groups : n_sm);  // persistent: one CTA per SM
+    // as many warps as the 227 KB of shared memory hold (12 at 22 050 Hz: 95 mel-weight rows)
+    const size_t fixed = onset2_fixed_bytes(tb.mel_wt_rows);
+    int warps = (int)((232448 - fixed) / kScrBytes2);
+    if (warps > kWarps2Max) warps = kWarps2Max;
+    NCFA_REQUIRE(warps >= 1, "mel table too large for shared memory");
+    const size_t smem = fixed + (size_t)warps * kScrBytes2;
+    const int64_t groups = ((int64_t)n_seg * ((frames + 1) / 2) + warps - 1) / warps;
+    const int grid = (int)(groups < n_sm ? groups : n_sm);  // persistent: one CTA per SM
+    {
         ProfScope _p(hop <= 128 ? "stft_logmel_kernel[hop<=128]" : "stft_logmel_kernel[hop>128]", st);
         if (hop == 64) {
             if ((rc = ensure_dynamic_smem((const void *)stft_logmel2_kernel<1>, smem))) return rc;

@@ -17,7 +17,6 @@
 // yields a best score s*; phase 2 evaluates only the remaining blocks that contain a lag with
 // prior_k > s* − log1p(1e6) − 1e-6 (the prior is unimodal, so that set is one interval).  Lags outside
 // cannot win, so the argmax is unchanged; typically ~80 % of the 2691 hop-64 lags are never touched.
-#include <stdlib.h>
 #include "ncfa_common.cuh"
 
 namespace ncfa {
@@ -431,14 +430,10 @@ __global__ void __launch_bounds__(256) tg_argmax_kernel(const float *__restrict_
     if (threadIdx.x == 0) lag_out[seg] = (s_idx[0] == 0x7fffffff) ? k_min : s_idx[0];
 }
 
+// frames per chunk of pass 2: short envelopes in one chunk, long ones in chunks of 4096 frames
 static int tempo_chunk(int max_env_len) {
     if (max_env_len <= 1024) return max_env_len < 1 ? 1 : max_env_len;
-    static const int long_chunk = [] {
-        const char *e = getenv("NCFA_TG_CHUNK");  // experiments only
-        const int v = e ? atoi(e) : 0;
-        return (v >= 1024 && v <= 16384) ? v : 4096;
-    }();
-    return long_chunk;
+    return 4096;
 }
 
 }  // namespace ncfa

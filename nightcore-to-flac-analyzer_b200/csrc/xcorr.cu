@@ -20,7 +20,6 @@
 // exact in float64; the reference's float32 BLAS sums differ from these by rounding only).
 // The general (win, stride) case of the C ABI — more than 4 blocks per window — keeps the direct
 // kernel (one CTA per (window, candidate)).
-#include <stdlib.h>
 #include "ncfa_common.cuh"
 #include "tc05.cuh"
 
@@ -508,21 +507,16 @@ __global__ void __launch_bounds__(kXcThreads) align_pick_kernel(const double *__
     }
 }
 
-// NCFA_XCORR_IMPL=ring4: four B blocks per CTA, 8 KB copies, 16 consumer warps (before/after of the eight-block default)
-static bool xcorr_g4() {
-    static const bool v = [] {
-        const char *e = getenv("NCFA_XCORR_IMPL");
-        return e && strcmp(e, "ring4") == 0;
-    }();
-    return v;
-}
-// NCFA_XCORR_IMPL=direct forces the one-CTA-per-candidate kernel (cross-check)
-static bool xcorr_force_direct() {
-    static const bool v = [] {
-        const char *e = getenv("NCFA_XCORR_IMPL");
-        return e && strcmp(e, "direct") == 0;
-    }();
-    return v;
+// launch shape of the block form (the last line of the table above): G = 8 B blocks per CTA, 1024-sample chunks (4 KB
+// copies), 4 stages, 8 consumer warps
+constexpr int kXrG = 8, kXrChunk = 1024, kXrStages = 4, kXrConsumers = 256;
+template <int NQ>
+using XrSmemT = XrSmem<NQ, kXrG, kXrChunk, kXrStages, kXrConsumers>;
+template <int NQ>
+static void xr_kernel_for(decltype(&xcorr_blocks_ring_kernel<1, kXrG, kXrChunk, kXrStages, kXrConsumers>) *kfn,
+                          size_t *smem) {
+    *kfn = xcorr_blocks_ring_kernel<NQ, kXrG, kXrChunk, kXrStages, kXrConsumers>;
+    *smem = sizeof(XrSmemT<NQ>);
 }
 
 }  // namespace ncfa
@@ -552,38 +546,23 @@ extern "C" int ncfa_xcorr_search_batched(const float *d_a, const float *d_b, con
     char *wp = (char *)d_workspace;
     const int nq = win / stride;
     // the tail (win − nq·stride samples per candidate) is summed by one lane in the pick kernel: keep it short
-    if (nq >= 1 && nq <= kMaxPieces && win - nq * stride <= 16 && !xcorr_force_direct()) {
+    if (nq >= 1 && nq <= kMaxPieces && win - nq * stride <= 16) {
         const int max_blocks = max_cand + kMaxPieces - 1;
         double *part = (double *)wp;
         double *na2b = (double *)(wp + align_up((size_t)n_windows * (kMaxPieces + 1) * max_blocks * 8, 256));
         {
             ProfScope _p("xcorr_blocks_kernel", st);
-            int rc = 0;
-#define NCFA_XR_LAUNCH(NQ_)                                                                                             \
-    do {                                                                                                                \
-        if (xcorr_g4()) {                                                                                               \
-            using Sm = XrSmem<NQ_, 4, 2048, 3, 512>;                                                                    \
-            auto kfn = xcorr_blocks_ring_kernel<NQ_, 4, 2048, 3, 512>;                                                  \
-            if ((rc = ensure_dynamic_smem((const void *)kfn, sizeof(Sm)))) return rc;                                   \
-            dim3 g4((max_cand + nq - 1 + 3) / 4, n_windows);                                                            \
-            kfn<<<g4, 512 + 32, sizeof(Sm), st>>>(d_a, d_b, d_a_pos, d_b_lo, d_n_cand, max_blocks, win, stride, part,   \
-                                                  na2b);                                                                \
-        } else {                                                                                                        \
-            using Sm = XrSmem<NQ_, 8, 1024, 4, 256>;                                                                    \
-            auto kfn = xcorr_blocks_ring_kernel<NQ_, 8, 1024, 4, 256>;                                                  \
-            if ((rc = ensure_dynamic_smem((const void *)kfn, sizeof(Sm)))) return rc;                                   \
-            dim3 g8((max_cand + nq - 1 + 7) / 8, n_windows);                                                            \
-            kfn<<<g8, 256 + 32, sizeof(Sm), st>>>(d_a, d_b, d_a_pos, d_b_lo, d_n_cand, max_blocks, win, stride, part,   \
-                                                  na2b);                                                                \
-        }                                                                                                               \
-    } while (0)
+            decltype(&xcorr_blocks_ring_kernel<1, kXrG, kXrChunk, kXrStages, kXrConsumers>) kfn;
+            size_t smem;
             switch (nq) {
-                case 1: NCFA_XR_LAUNCH(1); break;
-                case 2: NCFA_XR_LAUNCH(2); break;
-                case 3: NCFA_XR_LAUNCH(3); break;
-                default: NCFA_XR_LAUNCH(4); break;
+                case 1: xr_kernel_for<1>(&kfn, &smem); break;
+                case 2: xr_kernel_for<2>(&kfn, &smem); break;
+                case 3: xr_kernel_for<3>(&kfn, &smem); break;
+                default: xr_kernel_for<4>(&kfn, &smem); break;
             }
-#undef NCFA_XR_LAUNCH
+            if (int rc = ensure_dynamic_smem((const void *)kfn, smem)) return rc;
+            dim3 g((max_cand + nq - 1 + kXrG - 1) / kXrG, n_windows);
+            kfn<<<g, kXrConsumers + 32, smem, st>>>(d_a, d_b, d_a_pos, d_b_lo, d_n_cand, max_blocks, win, stride, part, na2b);
         }
         NCFA_LAUNCH_OK("xcorr_blocks_kernel");
         {

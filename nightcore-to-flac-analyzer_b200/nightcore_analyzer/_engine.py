@@ -7,7 +7,6 @@ tensors and never synchronises; the list-of-numpy convenience wrappers upload, r
 from __future__ import annotations
 
 import math
-import os
 import threading
 import weakref
 from typing import List, Optional, Sequence, Tuple
@@ -20,7 +19,7 @@ from ._native import check, lib
 
 # Intermediate log-mel tiles are sized to stay resident in the 126 MB L2 between the STFT kernel
 # and the flux kernel (DESIGN.md "onset front-end").
-ONSET_WS_TARGET_BYTES = int(os.environ.get("NCFA_ONSET_WS_MB", "96")) << 20
+ONSET_WS_TARGET_BYTES = 96 << 20
 MAX_SEGS_PER_CALL = 65535
 # tuning peak lists / decimation pyramids of one launch (HBM scratch, reused across sub-batches)
 CHROMA_WS_TARGET_BYTES = 4 << 30

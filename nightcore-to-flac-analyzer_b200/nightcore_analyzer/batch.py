@@ -334,22 +334,11 @@ def plan_subbatches(n_pairs: int, sub: int, workers: int = 2, first: int = 8, gr
     return sizes
 
 
-def _first_job_pairs(n_pairs: int, sub: int) -> int:
-    """Size of the first streamed job.  Its upload is the only one nothing hides, so it should be small; but jobs of a
-    few pairs are latency bound on the device (one CTA per envelope in the beat tracker, short grids), so it should not
-    be tiny either.  NCFA_E2E_FIRST overrides (experiments)."""
-    import os
-    env = os.environ.get("NCFA_E2E_FIRST")
-    if env:
-        return max(1, int(env))
-    return 8   # measured on B200, 1000 pairs (profiles/r2l): first = 8 → 1107 pairs/s end to end, 24 → 913, 48 → 891, 83 → 890
-
-
-def _job_growth() -> float:
-    """Growth factor of the streamed job sizes (NCFA_E2E_GROWTH overrides; experiments)."""
-    import os
-    env = os.environ.get("NCFA_E2E_GROWTH")
-    return float(env) if env else 1.5
+# Size of the first streamed job.  Its upload is the only one nothing hides, so it should be small; but jobs of a few
+# pairs are latency bound on the device (one CTA per envelope in the beat tracker, short grids), so it should not be tiny
+# either.  Measured on B200, 1000 pairs (profiles/r2l): first = 8 → 1107 pairs/s end to end, 24 → 913, 48 → 891, 83 → 890.
+FIRST_JOB_PAIRS = 8
+JOB_GROWTH = 1.5             # growth factor of the streamed job sizes
 
 
 # ------------------------------------------------------------------------------------------------ the batch scheduler
@@ -378,12 +367,11 @@ def _stage_pool():
     """Threads that copy pageable tracks into the pinned staging slot (np.copyto releases the GIL).  Unlike torch's
     copy_, whose parallelism follows OMP_NUM_THREADS (torchrun sets it to 1), the pool is ours.  Measured on the 16-core
     B200 box, 1000 pairs from pageable numpy arrays: 4 threads 751 pairs/s, 12 threads 858, torch copy_ with 16 OpenMP
-    threads 842 (profiles/r2z_*).  NCFA_STAGE_THREADS overrides the count."""
+    threads 842 (profiles/r2z_*)."""
     global _STAGE_POOL
     if _STAGE_POOL is None:
         import concurrent.futures as cf
-        env = os.environ.get("NCFA_STAGE_THREADS")
-        n = int(env) if env else max(2, min(12, len(os.sched_getaffinity(0)) * 3 // 4))
+        n = max(2, min(12, len(os.sched_getaffinity(0)) * 3 // 4))
         _STAGE_POOL = cf.ThreadPoolExecutor(max_workers=max(1, n), thread_name_prefix="ncfa-stage")
     return _STAGE_POOL
 
@@ -434,13 +422,9 @@ def analyse_batch(source, sr: int = SAMPLE_RATE, *, sub_batch: int = SUB_BATCH_P
         lengths = np.array([len(t) for t in tracks], dtype=np.int64)
     if P == 0:
         return []
-    if sizes is None and os.environ.get("NCFA_E2E_SIZES"):       # explicit plan (experiments): "8,12,18,..." must sum to P
-        sizes = [int(x) for x in os.environ["NCFA_E2E_SIZES"].split(",")]
-        if sum(sizes) != P:
-            sizes = None
     if sizes is None:
-        sizes = [P] if P <= INLINE_PAIRS else plan_subbatches(P, sub_batch, workers, first=_first_job_pairs(P, sub_batch),
-                                                              growth=_job_growth())
+        sizes = [P] if P <= INLINE_PAIRS else plan_subbatches(P, sub_batch, workers, first=FIRST_JOB_PAIRS,
+                                                              growth=JOB_GROWTH)
     sizes = [int(k) for k in sizes]
     if any(k <= 0 for k in sizes) or sum(sizes) != P:
         raise ValueError(f"sub-batch sizes {sizes} do not cover the {P} pairs of the batch exactly once")
@@ -467,7 +451,7 @@ def analyse_batch(source, sr: int = SAMPLE_RATE, *, sub_batch: int = SUB_BATCH_P
         # device slots: one per worker + TWO ahead.  With one ahead the copy of job j+3 cannot start before job j ends, and
         # a worker that finishes early finds nothing uploaded: measured 1036 pairs/s with 3 slots, 1218 with 4, 1227 with 6
         # (profiles/r3a_e2e_slots.log; 3.6 GB of HBM per slot at 125 pairs)
-        n_slots = int(os.environ.get("NCFA_E2E_SLOTS", 0)) or nw + 2
+        n_slots = nw + 2
         slots = _slots_for(device, n_slots, need, want_pinned=not pinned_in)
         free_q: "queue.Queue[_Slot]" = queue.Queue()
         for sl in slots:

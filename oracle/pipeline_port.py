@@ -223,16 +223,18 @@ ALIGN_HOP = 512
 
 
 def speed_xcorr_arrays(ya: np.ndarray, yb: np.ndarray, sr: int = 22050, n_windows: int = 20, window_sec: float = 3.0,
-                       search_range: float = 0.05, skip_edges: float = 0.10, return_indices: bool = False):
+                       search_range: float = 0.05, skip_edges: float = 0.10, return_indices: bool = False,
+                       stride: Optional[int] = None):
     """xcorr.py:95-162 from the point where both files are loaded at `sr`: edge trim, 20 reference
-    windows of A, strided float32 cosine search in B (stride = win//4, first strict maximum), polyfit
+    windows of A, strided float32 cosine search in B (stride = win//4 unless given, first strict maximum), polyfit
     slope + median quality.  Returns (slope, quality) [+ (a_pos, best_pb or -1 per window)]."""
     min_len = min(len(ya), len(yb))
     s, e = int(min_len * skip_edges), int(min_len * (1.0 - skip_edges))
     ya, yb = ya[s:e], yb[s:e]
     win = int(window_sec * sr)
     search = int(search_range * len(yb))
-    stride = max(1, win // 4)
+    if stride is None:
+        stride = max(1, win // 4)
     if len(ya) < win or len(yb) < win:
         return ((1.0, 0.0), (np.zeros(0, np.int64), np.zeros(0, np.int64))) if return_indices else (1.0, 0.0)
     a_positions = np.linspace(0, len(ya) - win, n_windows).astype(int)

@@ -45,35 +45,21 @@ def test_onset_strength_hop64_and_ragged(engine):
     assert np.all(got[2] == 0)
 
 
-@pytest.mark.parametrize("impl", ["tile", "warp1"])
-def test_onset_kernel_forms_are_bit_identical(engine, tmp_path, impl):
-    """The default STFT kernel (two frames per warp), the one-frame-per-warp form (NCFA_STFT_IMPL=warp1) and the tile
-    form (32-frame tiles, lane = frame in the mel phase; NCFA_STFT_IMPL=tile; the switch is read once per process) do the
-    same arithmetic in the same order: identical envelopes — ragged tails, odd frame counts, short segments and a hop that
-    is not a multiple of 64 included."""
-    import os
-    import subprocess
-    import sys
+@pytest.mark.parametrize("hop", [64, 512, 96])
+def test_onset_kernel_matches_oracle_at_each_hop_form(engine, hop):
+    """The STFT kernel has one instantiation per hop class: hop 64 and hop 512 (the two frames of a warp share register
+    loads) and any other even hop (two independent loads; hop 96 here).  Each matches the oracle — ragged tails, odd
+    frame counts and short segments included; an all-zero envelope must come out all zero."""
     ys = [synth.synth(7, 4.0, SR, bpm=101.0), synth.synth(8, 2.0, SR, bpm=133.0)[:40001], synth.synth(9, 1.0, SR)[:1500],
           synth.synth(10, 3.0, SR)[:64 * 700]]
-    for k, y in enumerate(ys):
-        np.save(tmp_path / f"y{k}.npy", y)
-    code = (
-        "import sys, numpy as np\n"
-        f"sys.path[:0] = {[p for p in sys.path if p]!r}\n"
-        "from nightcore_analyzer import _engine\n"
-        "e = _engine.get_engine()\n"
-        f"ys = [np.load(r'{tmp_path}/y%d.npy' % k) for k in range({len(ys)})]\n"
-        "for hop in (64, 512, 96):\n"
-        "    g = e.onset_strength(ys, hop=hop, sr=22050)\n"
-        f"    np.savez(r'{tmp_path}/other_%d.npz' % hop, *g)\n")
-    env = dict(os.environ, NCFA_STFT_IMPL=impl)
-    subprocess.run([sys.executable, "-c", code], check=True, env=env, timeout=600)
-    for hop in (64, 512, 96):
-        got = engine.onset_strength(ys, hop=hop, sr=SR)
-        ref = np.load(tmp_path / f"other_{hop}.npz")
-        for i, g in enumerate(got):
-            assert np.array_equal(g, ref[f"arr_{i}"]), (hop, i, float(np.max(np.abs(g - ref[f"arr_{i}"]))))
+    got = engine.onset_strength(ys, hop=hop, sr=SR)
+    for i, (y, g) in enumerate(zip(ys, got)):
+        want = lr.onset_strength(y, SR, hop)
+        assert g.shape == want.shape, (i, g.shape, want.shape)
+        if float(np.max(np.abs(want))) == 0.0:
+            assert np.all(g == 0), i
+        else:
+            assert rel_err(g, want) < 1e-4, (i, rel_err(g, want))
 
 
 def test_onset_top_db_clamp_active(engine):

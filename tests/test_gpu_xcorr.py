@@ -46,6 +46,38 @@ def test_speed_xcorr_44k_and_batch(engine):
     assert both[1][0] == w_same[0] and abs(both[1][1] - w_same[1]) <= 1e-5
 
 
+def test_xcorr_direct_path_matches_port(engine):
+    """stride = win // 8: a window spans 8 blocks, more than the block form takes, so the search runs the direct kernels
+    (one CTA per (window, candidate)) — the path of any (win, stride) outside the block form."""
+    from nightcore_analyzer import xcorr as nx
+    a, b = make_pair(4003, 60.0)
+    s, la, lb, win, _, a_pos, lo, _ = nx._search_tables(len(a), len(b), SR, nx.XCORR_N_WINDOWS, nx.XCORR_WINDOW_SEC,
+                                                         nx.XCORR_SEARCH_RANGE, nx.XCORR_SKIP_EDGES)
+    stride = win // 8
+    search = int(nx.XCORR_SEARCH_RANGE * lb)
+    n_cand = np.zeros(len(a_pos), dtype=np.int32)
+    for i, (pa, lo_b) in enumerate(zip(a_pos, lo)):
+        hi_b = min(lb - win, int(pa * lb / la) + search)
+        n_cand[i] = 0 if lo_b >= hi_b else len(range(lo_b, hi_b, stride))
+    audio, off, _ = engine.pack([a, b])
+    bj, bc = engine.xcorr_search_dev(audio, audio, off[0] + s + a_pos, off[1] + s + lo, n_cand, win, stride,
+                                     nx.XCORR_RMS_GATE)
+    bj, bc = engine.to_host(bj), engine.to_host(bc)
+    (w_slope, w_quality), (w_pos, w_pb) = port.speed_xcorr_arrays(a, b, SR, return_indices=True, stride=stride)
+    assert a_pos.tolist() == w_pos.tolist()
+    assert bj.tolist() == np.where(w_pb >= 0, (w_pb - lo) // stride, -1).tolist()
+    assert int((bj >= 0).sum()) >= 3
+    ya, yb = a[s:], b[s:]
+    for pa, lo_b, j, c in zip(a_pos, lo, bj, bc):
+        if j >= 0:
+            wa = ya[pa : pa + win].astype(np.float64)
+            wb = yb[lo_b + j * stride : lo_b + j * stride + win].astype(np.float64)
+            assert abs(c - float(np.dot(wa, wb) / (np.linalg.norm(wa) * np.linalg.norm(wb)))) <= 1e-5
+    slope, quality = nx._fit(a_pos, lo, stride, bj, bc)
+    assert slope == w_slope
+    assert abs(quality - w_quality) <= 1e-5
+
+
 def test_speed_xcorr_sentinels(engine):
     from nightcore_analyzer import xcorr as nx
     short = synth.synth(1, 3.0, SR, bpm=120.0)
