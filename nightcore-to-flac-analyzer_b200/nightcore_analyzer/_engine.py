@@ -99,7 +99,8 @@ class Engine:
     def pack(self, arrays: Sequence[np.ndarray]) -> Tuple[torch.Tensor, np.ndarray, np.ndarray]:
         """Concatenate float32 arrays into one device buffer → (audio, seg_off int64, seg_len int32) (host descriptors)."""
         lens = np.array([len(a) for a in arrays], dtype=np.int32)
-        # 4-sample (16 B) aligned starts keep the float4 loads of the kernels aligned
+        # 4-sample (16 B) aligned starts put the kernels on their vector-load fast paths; any other start gives the same
+        # results (tests/test_gpu_segment_placement.py)
         starts = np.zeros(len(arrays), dtype=np.int64)
         pos = 0
         for i, n in enumerate(lens):
