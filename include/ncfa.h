@@ -154,7 +154,9 @@ int ncfa_cyclic_xcorr_batched(const double *d_src, const double *d_nc, int n_pai
  * (the host applies xcorr.py:95-111,121-125 to produce these tables).  c = dot/(‖wa‖‖wb‖) with the
  * reference's float32 roundings of dot and norms; d_best_j[w] = first j with the largest c when it
  * is > 0 and the window passes the RMS gate (xcorr.py:118) and the 1e-10 norm gates, else −1;
- * d_best_c[w] = that c (0 when none). */
+ * d_best_c[w] = that c (0 when none).  (win, stride) picks the block form (win/stride <= 4 blocks and a tail of at
+ * most 16 samples) or the direct form; the workspace size is the larger of the two layouts, so it holds either.  Until
+ * the direct form was sized too, one window with max_cand <= 3 got 512 bytes instead of 768. */
 size_t ncfa_xcorr_workspace_bytes(int n_windows, int max_cand);
 int ncfa_xcorr_search_batched(const float *d_a, const float *d_b, const int64_t *d_a_pos, const int64_t *d_b_lo,
                               const int32_t *d_n_cand, int n_windows, int max_cand, int win, int stride,

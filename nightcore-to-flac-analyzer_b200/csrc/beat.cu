@@ -433,14 +433,29 @@ static size_t beat_f64_per_seg(int max_env_len, int max_fpb) {
     return 3 * (size_t)max_env_len + 2 * (2 * (size_t)max_fpb + 1) + 8;
 }
 
+// the per-segment BeatWs regions: float64 ones of all segments, then int32 ones
+struct BeatWorkspace {
+    double *f64;
+    int32_t *i32;
+    size_t bytes;
+};
+
+static BeatWorkspace beat_ws(int n_seg, int max_env_len, int max_lag, void *base) {
+    Carve c(base);
+    BeatWorkspace w;
+    w.f64 = c.take<double>((size_t)n_seg * beat_f64_per_seg(max_env_len, max_lag));
+    w.i32 = c.take<int32_t>((size_t)n_seg * 2 * max_env_len);
+    w.bytes = c.used;
+    return w;
+}
+
 }  // namespace ncfa
 
 using namespace ncfa;
 
 extern "C" size_t ncfa_beat_workspace_bytes(int n_seg, int max_env_len, int max_lag) {
     if (n_seg <= 0 || max_env_len <= 0 || max_lag <= 0) return 0;
-    return align_up((size_t)n_seg * beat_f64_per_seg(max_env_len, max_lag) * 8, 256) +
-           align_up((size_t)n_seg * 2 * max_env_len * 4, 256);
+    return beat_ws(n_seg, max_env_len, max_lag, nullptr).bytes;
 }
 
 extern "C" int ncfa_beat_track_batched(const float *d_onset, const int64_t *d_onset_off, const int32_t *d_env_len,
@@ -451,43 +466,26 @@ extern "C" int ncfa_beat_track_batched(const float *d_onset, const int64_t *d_on
     if (n_seg == 0) return NCFA_OK;
     NCFA_REQUIRE(d_onset && d_onset_off && d_env_len && d_lag && d_beats && d_n_beats && d_workspace, "null pointer");
     NCFA_REQUIRE(max_env_len > 0 && max_beats > 0 && max_lag > 0, "max_env_len/max_beats/max_lag");
-    if (workspace_bytes < ncfa_beat_workspace_bytes(n_seg, max_env_len, max_lag)) {
-        set_error("beat workspace too small");
-        return NCFA_E_WORKSPACE;
-    }
-    double *wf = (double *)d_workspace;
-    int32_t *wi = (int32_t *)((char *)d_workspace +
-                              align_up((size_t)n_seg * beat_f64_per_seg(max_env_len, max_lag) * 8, 256));
+    const BeatWorkspace w = beat_ws(n_seg, max_env_len, max_lag, d_workspace);
+    if (int rc = check_workspace("beat", workspace_bytes, w.bytes)) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
     // long envelopes: measured on B200, 9.9 ms (512 threads) vs 11.1 (1024) vs 12.5 (256) per 250 pairs
     const int threads = max_env_len <= 2048 ? 64 : 512;
     const int ring = beat_ring(max_lag);
     // reduction scratch | score ring | transition penalties | best predecessor per frame of a wavefront (ints)
     const size_t smem = ((size_t)threads + ring + (3 * (size_t)max_lag / 2 + 4) + ((size_t)max_lag / 4 + 4)) * sizeof(double);
-    int rc = ensure_dynamic_smem((const void *)beat_track_kernel, smem);
-    if (rc) return rc;
-    {
-        ProfScope _p("beat_prep_kernel", (cudaStream_t)stream);
-        beat_prep_kernel<<<n_seg, 256, 0, (cudaStream_t)stream>>>(d_onset, d_onset_off, d_env_len, max_env_len, d_lag, wf,
-                                                              max_lag);
-    }
-    NCFA_LAUNCH_OK("beat_prep_kernel");
-    {
-        dim3 g(n_seg, (max_env_len + 256 * kScoreFramesPerThread - 1) / (256 * kScoreFramesPerThread));
-        NCFA_REQUIRE(g.y <= 65535, "envelope too long for one call");
-        ProfScope _p("beat_score_kernel", (cudaStream_t)stream);
-        const size_t tile_elems = (size_t)256 * kScoreFramesPerThread + 2 * (size_t)max_lag + 1;
-        const size_t smem_score = (tile_elems + tile_elems / 16 + 2) * sizeof(double);
-        int rcs = ensure_dynamic_smem((const void *)beat_score_kernel, smem_score);
-        if (rcs) return rcs;
-        beat_score_kernel<<<g, 256, smem_score, (cudaStream_t)stream>>>(d_env_len, max_env_len, d_lag, wf, max_lag);
-    }
-    NCFA_LAUNCH_OK("beat_score_kernel");
-    {
-        ProfScope _p(max_env_len <= 2048 ? "beat_track_kernel" : "beat_track_kernel[long]", (cudaStream_t)stream);
-        beat_track_kernel<<<n_seg, threads, smem, (cudaStream_t)stream>>>(d_onset, d_onset_off, d_env_len, max_env_len,
-                                                                          d_lag, wf, wi, max_lag, d_beats, max_beats,
-                                                                          d_n_beats, ring);
-    }
-    NCFA_LAUNCH_OK("beat_track_kernel");
-    return NCFA_OK;
+    const dim3 gs(n_seg, (max_env_len + 256 * kScoreFramesPerThread - 1) / (256 * kScoreFramesPerThread));
+    NCFA_REQUIRE(gs.y <= 65535, "envelope too long for one call");
+    const size_t tile_elems = (size_t)256 * kScoreFramesPerThread + 2 * (size_t)max_lag + 1;
+    const size_t smem_score = (tile_elems + tile_elems / 16 + 2) * sizeof(double);
+    int rc;
+    if ((rc = launch("beat_prep_kernel", beat_prep_kernel, n_seg, 256, 0, st, d_onset, d_onset_off, d_env_len,
+                     max_env_len, d_lag, w.f64, max_lag)))
+        return rc;
+    if ((rc = launch("beat_score_kernel", beat_score_kernel, gs, 256, smem_score, st, d_env_len, max_env_len, d_lag,
+                     w.f64, max_lag)))
+        return rc;
+    return launch(max_env_len <= 2048 ? "beat_track_kernel" : "beat_track_kernel[long]", beat_track_kernel, n_seg,
+                  threads, smem, st, d_onset, d_onset_off, d_env_len, max_env_len, d_lag, w.f64, w.i32, max_lag,
+                  d_beats, max_beats, d_n_beats, ring);
 }

@@ -418,29 +418,30 @@ __global__ void __launch_bounds__(256) boot_finish_kernel(const int32_t *__restr
     }
 }
 
-struct BootLayout {
-    size_t tables, rank_a, rank_b, sorted_a, sorted_b, start, extra, boot, total;
+struct BootWs {
+    BootTables *tables;
+    int32_t *rank_a, *rank_b;
+    double *sorted_a, *sorted_b;
+    int64_t *start;
+    int32_t *extra;
+    double *boot;
+    size_t bytes;
 };
 
-static BootLayout boot_layout(int n_jobs, int max_a, int max_b, int n_boot) {
-    BootLayout L;
-    size_t p = 0;
-    auto take = [&](size_t bytes) {
-        size_t o = p;
-        p += align_up(bytes, 256);
-        return o;
-    };
+static BootWs boot_ws(int n_jobs, int max_a, int max_b, int n_boot, void *base) {
+    Carve c(base);
+    BootWs w;
     const size_t mb = max_b > 0 ? max_b : 1;
-    L.tables = take(sizeof(BootTables));
-    L.rank_a = take((size_t)n_jobs * max_a * 4);
-    L.rank_b = take((size_t)n_jobs * mb * 4);
-    L.sorted_a = take((size_t)n_jobs * max_a * 8);
-    L.sorted_b = take((size_t)n_jobs * mb * 8);
-    L.start = take((size_t)n_jobs * n_boot * 8);
-    L.extra = take((size_t)n_jobs * n_boot * 4);
-    L.boot = take((size_t)n_jobs * n_boot * 8);
-    L.total = p;
-    return L;
+    w.tables = c.take<BootTables>(1);
+    w.rank_a = c.take<int32_t>((size_t)n_jobs * max_a);
+    w.rank_b = c.take<int32_t>((size_t)n_jobs * mb);
+    w.sorted_a = c.take<double>((size_t)n_jobs * max_a);
+    w.sorted_b = c.take<double>((size_t)n_jobs * mb);
+    w.start = c.take<int64_t>((size_t)n_jobs * n_boot);
+    w.extra = c.take<int32_t>((size_t)n_jobs * n_boot);
+    w.boot = c.take<double>((size_t)n_jobs * n_boot);
+    w.bytes = c.used;
+    return w;
 }
 
 }  // namespace ncfa
@@ -449,7 +450,7 @@ using namespace ncfa;
 
 extern "C" size_t ncfa_bootstrap_workspace_bytes(int n_jobs, int max_a, int max_b, int n_boot) {
     if (n_jobs <= 0 || max_a <= 0 || max_b < 0 || n_boot <= 0) return 0;
-    return boot_layout(n_jobs, max_a, max_b, n_boot).total;
+    return boot_ws(n_jobs, max_a, max_b, n_boot, nullptr).bytes;
 }
 
 extern "C" int ncfa_bootstrap_ratio_batched(const double *d_a, const int64_t *d_a_off, const int32_t *d_a_len,
@@ -472,71 +473,35 @@ extern "C" int ncfa_bootstrap_ratio_batched(const double *d_a, const int64_t *d_
                   (size_t)max_a, (size_t)max_b);
         return NCFA_E_OVERFLOW;
     }
-    const BootLayout L = boot_layout(n_jobs, max_a, max_b, n_boot);
-    if (workspace_bytes < L.total) {
-        set_error("bootstrap workspace too small: %zu < %zu", workspace_bytes, L.total);
-        return NCFA_E_WORKSPACE;
-    }
+    const BootWs w = boot_ws(n_jobs, max_a, max_b, n_boot, d_workspace);
+    if (int rc = check_workspace("bootstrap", workspace_bytes, w.bytes)) return rc;
     cudaStream_t st = (cudaStream_t)stream;
-    char *wp = (char *)d_workspace;
-    BootTables *tb = (BootTables *)(wp + L.tables);
-    int32_t *rank_a = (int32_t *)(wp + L.rank_a), *rank_b = (int32_t *)(wp + L.rank_b);
-    double *sorted_a = (double *)(wp + L.sorted_a), *sorted_b = (double *)(wp + L.sorted_b);
-    int64_t *start = (int64_t *)(wp + L.start);
-    int32_t *extra = (int32_t *)(wp + L.extra);
-    double *boot = d_boot ? d_boot : (double *)(wp + L.boot);
+    double *boot = d_boot ? d_boot : w.boot;
     const u128 state0 = ((u128)h_pcg_state[0] << 64) | h_pcg_state[1];
     const u128 inc = ((u128)h_pcg_state[2] << 64) | h_pcg_state[3];
-
-    {
-        ProfScope _p("boot_tables_kernel", st);
-        boot_tables_kernel<<<1, 32, 0, st>>>(inc, tb);
-    }
-    NCFA_LAUNCH_OK("boot_tables_kernel");
-    {
-        dim3 g(n_jobs, d_b ? 2 : 1);
-        {
-            ProfScope _p("boot_rank_kernel", st);
-            boot_rank_kernel<<<g, 256, 0, st>>>(d_a, d_a_off, d_a_len, d_b, d_b_off, d_b_len, max_a, max_b > 0 ? max_b : 1,
-                                            rank_a, rank_b, sorted_a, sorted_b);
-        }
-        NCFA_LAUNCH_OK("boot_rank_kernel");
-    }
-    {
-        int threads = n_boot >= 1024 ? 1024 : ((n_boot + 31) / 32) * 32;
-        {
-            ProfScope _p("boot_offsets_kernel", st);
-            boot_offsets_kernel<<<n_jobs, threads, 0, st>>>(d_a_len, d_b ? d_b_len : nullptr, n_boot, state0, inc, tb,
-                                                        start, extra);
-        }
-        NCFA_LAUNCH_OK("boot_offsets_kernel");
-    }
-    {
-        // warps per CTA bounded by the shared-memory histogram; stride padded to avoid lock-step banks
-        const int hist_stride = (int)((hist_ints + 1) | 1);
-        int warps = (int)((200 * 1024) / ((size_t)hist_stride * 4));
-        warps = warps > 8 ? 8 : (warps < 1 ? 1 : warps);
-        const size_t sh = (size_t)warps * hist_stride * 4;
-        if (sh > 48 * 1024) {
-            int rc = ensure_dynamic_smem((const void *)boot_median_kernel, 200 * 1024 + 64);
-            if (rc) return rc;
-        }
-        const long long total = (long long)n_jobs * n_boot;
-        long long blocks = (total + warps - 1) / warps;
-        if (blocks > 148LL * 64) blocks = 148LL * 64;
-        {
-            ProfScope _p("boot_median_kernel", st);
-            boot_median_kernel<<<(unsigned)blocks, warps * 32, sh, st>>>(
-            d_a_len, d_b ? d_b_len : nullptr, max_a, max_b > 0 ? max_b : 1, n_boot, n_jobs, state0, inc, tb, start,
-            extra, rank_a, rank_b, sorted_a, sorted_b, boot, d_idx, hist_stride);
-        }
-        NCFA_LAUNCH_OK("boot_median_kernel");
-    }
-    {
-        ProfScope _p("boot_finish_kernel", st);
-        boot_finish_kernel<<<n_jobs, 256, n_boot <= kBootFinishMaxStaged ? (size_t)n_boot * 8 : 0, st>>>(d_a_len, d_b ? d_b_len : nullptr, max_a, max_b > 0 ? max_b : 1, n_boot,
-                                               sorted_a, sorted_b, boot, q_lo, q_hi, d_out);
-    }
-    NCFA_LAUNCH_OK("boot_finish_kernel");
-    return NCFA_OK;
+    const int mb = max_b > 0 ? max_b : 1;
+    const int32_t *b_len = d_b ? d_b_len : nullptr;
+    int rc;
+    if ((rc = launch("boot_tables_kernel", boot_tables_kernel, 1, 32, 0, st, inc, w.tables))) return rc;
+    if ((rc = launch("boot_rank_kernel", boot_rank_kernel, dim3(n_jobs, d_b ? 2 : 1), 256, 0, st, d_a, d_a_off, d_a_len,
+                     d_b, d_b_off, d_b_len, max_a, mb, w.rank_a, w.rank_b, w.sorted_a, w.sorted_b)))
+        return rc;
+    const int threads = n_boot >= 1024 ? 1024 : ((n_boot + 31) / 32) * 32;
+    if ((rc = launch("boot_offsets_kernel", boot_offsets_kernel, n_jobs, threads, 0, st, d_a_len, b_len, n_boot,
+                     state0, inc, w.tables, w.start, w.extra)))
+        return rc;
+    // warps per CTA bounded by the shared-memory histogram; stride padded to avoid lock-step banks
+    const int hist_stride = (int)((hist_ints + 1) | 1);
+    int warps = (int)((200 * 1024) / ((size_t)hist_stride * 4));
+    warps = warps > 8 ? 8 : (warps < 1 ? 1 : warps);
+    const long long total = (long long)n_jobs * n_boot;
+    long long blocks = (total + warps - 1) / warps;
+    if (blocks > 148LL * 64) blocks = 148LL * 64;
+    if ((rc = launch("boot_median_kernel", boot_median_kernel, (unsigned)blocks, warps * 32,
+                     (size_t)warps * hist_stride * 4, st, d_a_len, b_len, max_a, mb, n_boot, n_jobs, state0, inc,
+                     w.tables, w.start, w.extra, w.rank_a, w.rank_b, w.sorted_a, w.sorted_b, boot, d_idx, hist_stride)))
+        return rc;
+    return launch("boot_finish_kernel", boot_finish_kernel, n_jobs, 256,
+                  n_boot <= kBootFinishMaxStaged ? (size_t)n_boot * 8 : 0, st, d_a_len, b_len, max_a, mb, n_boot,
+                  w.sorted_a, w.sorted_b, boot, q_lo, q_hi, d_out);
 }

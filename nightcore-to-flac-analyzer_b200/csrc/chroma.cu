@@ -988,10 +988,28 @@ using namespace ncfa;
 
 static size_t tuning_frames(int max_seg_len) { return 1 + (size_t)max_seg_len / 512; }
 
+// per frame kPeakStride candidate peaks (magnitude, bin) and their count
+struct TuningWs {
+    float *pk_mag;
+    uint8_t *pk_bin;
+    int32_t *pk_cnt;
+    size_t bytes;
+};
+
+static TuningWs tuning_ws(int n_seg, int max_seg_len, void *base) {
+    const size_t frames = (size_t)n_seg * tuning_frames(max_seg_len);
+    Carve c(base);
+    TuningWs w;
+    w.pk_mag = c.take<float>(frames * kPeakStride);
+    w.pk_bin = c.take<uint8_t>(frames * kPeakStride);
+    w.pk_cnt = c.take<int32_t>(frames);
+    w.bytes = c.used;
+    return w;
+}
+
 extern "C" size_t ncfa_tuning_workspace_bytes(int n_seg, int max_seg_len) {
     if (n_seg <= 0 || max_seg_len < 0) return 0;
-    const size_t slots = (size_t)n_seg * tuning_frames(max_seg_len) * kPeakStride;
-    return align_up(slots * 4, 256) + align_up(slots, 256) + align_up((size_t)n_seg * tuning_frames(max_seg_len) * 4, 256);
+    return tuning_ws(n_seg, max_seg_len, nullptr).bytes;
 }
 
 extern "C" int ncfa_tuning_estimate_batched(const float *d_audio, const int64_t *d_seg_off, const int32_t *d_seg_len,
@@ -1001,13 +1019,11 @@ extern "C" int ncfa_tuning_estimate_batched(const float *d_audio, const int64_t 
     if (n_seg == 0) return NCFA_OK;
     NCFA_REQUIRE(d_audio && d_seg_off && d_seg_len && d_tuning_idx && d_workspace, "null pointer");
     NCFA_REQUIRE(max_seg_len >= 0 && sr > 0, "max_seg_len/sr");
-    if (workspace_bytes < ncfa_tuning_workspace_bytes(n_seg, max_seg_len)) {
-        set_error("tuning workspace too small");
-        return NCFA_E_WORKSPACE;
-    }
-    Tables tb;
-    int rc = get_tables(sr, &tb);
+    const TuningWs w = tuning_ws(n_seg, max_seg_len, d_workspace);
+    int rc = check_workspace("tuning", workspace_bytes, w.bytes);
     if (rc) return rc;
+    Tables tb;
+    if ((rc = get_tables(sr, &tb))) return rc;
     // piptrack frequency mask: fmin=150 <= fft_freq < min(4000, sr/2), fft_freq[k] = k · (1 / (n_fft · (1/sr)))
     const double val = 1.0 / (2048.0 * (1.0 / (double)sr));
     const double fmax = fmin(4000.0, (double)sr / 2.0);
@@ -1016,42 +1032,42 @@ extern "C" int ncfa_tuning_estimate_batched(const float *d_audio, const int64_t 
     while (kmax > 0 && !((double)kmax * val < fmax)) --kmax;
     NCFA_REQUIRE(kmin <= kmax && (kmax - kmin + 2) / 2 <= kPeakStride, "piptrack band does not fit the peak buffer");
     cudaStream_t st = (cudaStream_t)stream;
-    const size_t frames = tuning_frames(max_seg_len);
-    const size_t slots = (size_t)n_seg * frames * kPeakStride;
-    char *wp = (char *)d_workspace;
-    float *pk_mag = (float *)wp;
-    wp += align_up(slots * 4, 256);
-    uint8_t *pk_bin = (uint8_t *)wp;
-    wp += align_up(slots, 256);
-    int32_t *pk_cnt = (int32_t *)wp;
-    if ((rc = ensure_dynamic_smem((const void *)tuning_peaks_kernel, sizeof(TuningSmem)))) return rc;
-    {
-        int n_sm = 0;
-        if ((rc = sm_count(&n_sm))) return rc;
-        const int64_t groups = ((int64_t)n_seg * (int64_t)frames + kTunWarps - 1) / kTunWarps;
-        const int grid = (int)(groups < n_sm ? groups : n_sm);
-        ProfScope _p("tuning_peaks_kernel", st);
-        tuning_peaks_kernel<<<grid, kTunThreads, sizeof(TuningSmem), st>>>(d_audio, d_seg_off, d_seg_len, n_seg, (int)frames,
-                                                                           kmin, kmax, (double)sr / 2048.0, tb, pk_mag,
-                                                                           pk_bin, pk_cnt);
-    }
-    NCFA_LAUNCH_OK("tuning_peaks_kernel");
-    {
-        ProfScope _p("tuning_pick_kernel", st);
-        tuning_pick_kernel<<<n_seg, 256, 0, st>>>(d_seg_len, (int)frames, pk_mag, pk_bin, pk_cnt, d_tuning_idx);
-    }
-    NCFA_LAUNCH_OK("tuning_pick_kernel");
-    return NCFA_OK;
+    const int frames = (int)tuning_frames(max_seg_len);
+    int n_sm = 0;
+    if ((rc = sm_count(&n_sm))) return rc;
+    const int64_t groups = ((int64_t)n_seg * frames + kTunWarps - 1) / kTunWarps;
+    const int grid = (int)(groups < n_sm ? groups : n_sm);
+    if ((rc = launch("tuning_peaks_kernel", tuning_peaks_kernel, grid, kTunThreads, sizeof(TuningSmem), st, d_audio,
+                     d_seg_off, d_seg_len, n_seg, frames, kmin, kmax, (double)sr / 2048.0, tb, w.pk_mag, w.pk_bin,
+                     w.pk_cnt)))
+        return rc;
+    return launch("tuning_pick_kernel", tuning_pick_kernel, n_seg, 256, 0, st, d_seg_len, frames, w.pk_mag, w.pk_bin,
+                  w.pk_cnt, d_tuning_idx);
 }
 
 static int chroma_tiles(int max_seg_len) { return (cqt_frames(max_seg_len) + kPartialTF - 1) / kPartialTF; }
 
+// the decimated pyramid of every segment (plus 16 bytes), then kChroma float64 partial sums per tile of frames
+struct ChromaWs {
+    float *pyr;
+    double *partial;
+    size_t bytes;
+};
+
+static ChromaWs chroma_ws(int n_seg, int max_seg_len, const PyrOffsets &po, void *base) {
+    Carve c(base);
+    ChromaWs w;
+    w.pyr = c.take<float>((size_t)n_seg * po.off[kOctaves] + 4);
+    w.partial = c.take<double>((size_t)n_seg * chroma_tiles(max_seg_len) * kChroma);
+    w.bytes = c.used;
+    return w;
+}
+
 extern "C" size_t ncfa_chroma_workspace_bytes(int n_seg, int max_seg_len) {
     if (n_seg <= 0 || max_seg_len < 0) return 0;
-    size_t off[kOctaves + 1];
-    pyramid_layout(max_seg_len, off);
-    return align_up((size_t)n_seg * off[kOctaves] * 4 + 16, 256) +
-           align_up((size_t)n_seg * chroma_tiles(max_seg_len) * kChroma * 8, 256);
+    PyrOffsets po;
+    pyramid_layout(max_seg_len, po.off);
+    return chroma_ws(n_seg, max_seg_len, po, nullptr).bytes;
 }
 
 extern "C" int ncfa_chroma_mean_batched(const float *d_audio, const int64_t *d_seg_off, const int32_t *d_seg_len,
@@ -1062,43 +1078,30 @@ extern "C" int ncfa_chroma_mean_batched(const float *d_audio, const int64_t *d_s
     NCFA_REQUIRE(d_audio && d_seg_off && d_seg_len && d_tuning_idx && d_chroma && d_workspace, "null pointer");
     NCFA_REQUIRE(max_seg_len >= 0, "max_seg_len");
     NCFA_REQUIRE(sr == 22050, "the CQT path is laid out for sr = 22050 (7 octaves from C1, n_fft 1024, no early downsampling)");
-    if (workspace_bytes < ncfa_chroma_workspace_bytes(n_seg, max_seg_len)) {
-        set_error("chroma workspace too small");
-        return NCFA_E_WORKSPACE;
-    }
-    ChromaTables ct;
-    int rc = get_chroma_tables(sr, &ct);
-    if (rc) return rc;
-    cudaStream_t st = (cudaStream_t)stream;
     PyrOffsets po;
     pyramid_layout(max_seg_len, po.off);
+    const ChromaWs w = chroma_ws(n_seg, max_seg_len, po, d_workspace);
+    int rc = check_workspace("chroma", workspace_bytes, w.bytes);
+    if (rc) return rc;
+    ChromaTables ct;
+    if ((rc = get_chroma_tables(sr, &ct))) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
     const size_t stride = po.off[kOctaves];
-    float *pyr = (float *)d_workspace;
-    double *partial = (double *)((char *)d_workspace + align_up((size_t)n_seg * stride * 4 + 16, 256));
     for (int level = 1; level < kOctaves; ++level) {
         const int n_out = level_len(max_seg_len, level);
         if (n_out <= 0) continue;
-        ProfScope _p("decimate2_kernel", st);
-        dim3 g((n_out + kDecOutPerCta - 1) / kDecOutPerCta, n_seg);
-        decimate2_kernel<<<g, 256, 0, st>>>(d_audio, d_seg_off, d_seg_len, level, pyr, stride,
-                                            level >= 2 ? po.off[level - 1] : 0, po.off[level], ct.hb);
-        NCFA_LAUNCH_OK("decimate2_kernel");
+        if ((rc = launch("decimate2_kernel", decimate2_kernel, dim3((n_out + kDecOutPerCta - 1) / kDecOutPerCta, n_seg),
+                         256, 0, st, d_audio, d_seg_off, d_seg_len, level, w.pyr, stride,
+                         level >= 2 ? po.off[level - 1] : 0, po.off[level], ct.hb)))
+            return rc;
     }
-    if ((rc = ensure_dynamic_smem((const void *)cqt_tc_kernel, sizeof(TcSmem) + 1024))) return rc;
     const int tiles = chroma_tiles(max_seg_len);  // partial[] stride
-    {
-        ProfScope _p("cqt_tc_kernel", st);
-        dim3 g((cqt_frames(max_seg_len) + kTcFrames - 1) / kTcFrames, n_seg);
-        cqt_tc_kernel<<<g, kTcThreads, sizeof(TcSmem) + 1024, st>>>(d_audio, d_seg_off, d_seg_len, pyr, po, d_tuning_idx,
-                                                                   ct.Bimg, tiles, partial);
-    }
-    NCFA_LAUNCH_OK("cqt_tc_kernel");
-    {
-        ProfScope _p("chroma_mean_kernel", st);
-        chroma_mean_kernel<<<n_seg, 32, 0, st>>>(d_seg_len, tiles, kTcFrames, partial, d_chroma);
-    }
-    NCFA_LAUNCH_OK("chroma_mean_kernel");
-    return NCFA_OK;
+    if ((rc = launch("cqt_tc_kernel", cqt_tc_kernel, dim3((cqt_frames(max_seg_len) + kTcFrames - 1) / kTcFrames, n_seg),
+                     kTcThreads, sizeof(TcSmem) + 1024, st, d_audio, d_seg_off, d_seg_len, w.pyr, po, d_tuning_idx,
+                     ct.Bimg, tiles, w.partial)))
+        return rc;
+    return launch("chroma_mean_kernel", chroma_mean_kernel, n_seg, 32, 0, st, d_seg_len, tiles, kTcFrames, w.partial,
+                  d_chroma);
 }
 
 extern "C" int ncfa_cyclic_xcorr_batched(const double *d_src, const double *d_nc, int n_pairs, int n_bins,
@@ -1106,12 +1109,8 @@ extern "C" int ncfa_cyclic_xcorr_batched(const double *d_src, const double *d_nc
     NCFA_REQUIRE(n_pairs >= 0 && n_bins > 0, "n_pairs/n_bins");
     if (n_pairs == 0) return NCFA_OK;
     NCFA_REQUIRE(d_src && d_nc && d_lag, "null pointer");
-    {
-        ProfScope _p("cyclic_xcorr_kernel", (cudaStream_t)stream);
-        cyclic_xcorr_kernel<<<(n_pairs + 63) / 64, 64, 0, (cudaStream_t)stream>>>(d_src, d_nc, n_pairs, n_bins, d_lag);
-    }
-    NCFA_LAUNCH_OK("cyclic_xcorr_kernel");
-    return NCFA_OK;
+    return launch("cyclic_xcorr_kernel", cyclic_xcorr_kernel, (n_pairs + 63) / 64, 64, 0, (cudaStream_t)stream, d_src,
+                  d_nc, n_pairs, n_bins, d_lag);
 }
 
 // Host-side table builders, exported so that the CPU test-suite can check them without a GPU.

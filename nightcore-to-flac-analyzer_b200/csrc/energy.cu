@@ -141,6 +141,22 @@ __global__ void __launch_bounds__(256) trim_bounds_kernel(const int32_t *__restr
     }
 }
 
+// one float64 sum per 512-sample block, `stride` blocks (3 spare) per segment
+struct TrimWs {
+    int stride;
+    double *bsum;
+    size_t bytes;
+};
+
+static TrimWs trim_ws(int n_seg, int max_seg_len, void *base) {
+    Carve c(base);
+    TrimWs w;
+    w.stride = max_seg_len / 512 + 4;
+    w.bsum = c.take<double>((size_t)n_seg * w.stride);
+    w.bytes = c.used;
+    return w;
+}
+
 }  // namespace ncfa
 
 using namespace ncfa;
@@ -150,12 +166,8 @@ extern "C" int ncfa_window_energy(const float *d_audio, const int64_t *d_seg_off
     NCFA_REQUIRE(n_seg >= 0, "n_seg");
     if (n_seg == 0) return NCFA_OK;
     NCFA_REQUIRE(d_audio && d_seg_off && d_seg_len && d_meansq, "null pointer");
-    {
-        ProfScope _p("window_energy_kernel", (cudaStream_t)stream);
-        window_energy_kernel<<<n_seg, 256, 0, (cudaStream_t)stream>>>(d_audio, d_seg_off, d_seg_len, d_meansq);
-    }
-    NCFA_LAUNCH_OK("window_energy_kernel");
-    return NCFA_OK;
+    return launch("window_energy_kernel", window_energy_kernel, n_seg, 256, 0, (cudaStream_t)stream, d_audio, d_seg_off,
+                  d_seg_len, d_meansq);
 }
 
 extern "C" int ncfa_rms_frames(const float *d_audio, int64_t n, int frame_length, int hop, float *d_rms, void *stream) {
@@ -163,18 +175,13 @@ extern "C" int ncfa_rms_frames(const float *d_audio, int64_t n, int frame_length
     NCFA_REQUIRE(n >= 0 && frame_length > 0 && hop > 0, "n/frame_length/hop");
     const int64_t n_frames = 1 + n / hop;
     NCFA_REQUIRE((n_frames + 7) / 8 < 2147483647LL, "too many frames");
-    {
-        ProfScope _p("rms_frames_kernel", (cudaStream_t)stream);
-        rms_frames_kernel<<<(unsigned)((n_frames + 7) / 8), 256, 0, (cudaStream_t)stream>>>(d_audio, n, frame_length, hop,
-                                                                                       n_frames, d_rms);
-    }
-    NCFA_LAUNCH_OK("rms_frames_kernel");
-    return NCFA_OK;
+    return launch("rms_frames_kernel", rms_frames_kernel, (unsigned)((n_frames + 7) / 8), 256, 0, (cudaStream_t)stream,
+                  d_audio, n, frame_length, hop, n_frames, d_rms);
 }
 
 extern "C" size_t ncfa_trim_workspace_bytes(int n_seg, int max_seg_len) {
     if (n_seg <= 0 || max_seg_len < 0) return 0;
-    return align_up((size_t)n_seg * ((size_t)max_seg_len / 512 + 4) * 8, 256);
+    return trim_ws(n_seg, max_seg_len, nullptr).bytes;
 }
 
 extern "C" int ncfa_trim_bounds_batched(const float *d_audio, const int64_t *d_seg_off, const int32_t *d_seg_len,
@@ -184,23 +191,12 @@ extern "C" int ncfa_trim_bounds_batched(const float *d_audio, const int64_t *d_s
     if (n_seg == 0) return NCFA_OK;
     NCFA_REQUIRE(d_audio && d_seg_off && d_seg_len && d_bounds && d_workspace, "null pointer");
     NCFA_REQUIRE(max_seg_len >= 0, "max_seg_len");
-    if (workspace_bytes < ncfa_trim_workspace_bytes(n_seg, max_seg_len)) {
-        set_error("trim workspace too small");
-        return NCFA_E_WORKSPACE;
-    }
+    const TrimWs w = trim_ws(n_seg, max_seg_len, d_workspace);
+    if (int rc = check_workspace("trim", workspace_bytes, w.bytes)) return rc;
     cudaStream_t st = (cudaStream_t)stream;
-    const int stride = max_seg_len / 512 + 4;
-    double *bsum = (double *)d_workspace;
-    {
-        ProfScope _p("trim_blocksum_kernel", st);
-        dim3 g((stride + 7) / 8, n_seg);
-        trim_blocksum_kernel<<<g, 256, 0, st>>>(d_audio, d_seg_off, d_seg_len, stride, bsum);
-    }
-    NCFA_LAUNCH_OK("trim_blocksum_kernel");
-    {
-        ProfScope _p("trim_bounds_kernel", st);
-        trim_bounds_kernel<<<n_seg, 256, 0, st>>>(d_seg_len, stride, bsum, (float)top_db, d_bounds);
-    }
-    NCFA_LAUNCH_OK("trim_bounds_kernel");
-    return NCFA_OK;
+    if (int rc = launch("trim_blocksum_kernel", trim_blocksum_kernel, dim3((w.stride + 7) / 8, n_seg), 256, 0, st,
+                        d_audio, d_seg_off, d_seg_len, w.stride, w.bsum))
+        return rc;
+    return launch("trim_bounds_kernel", trim_bounds_kernel, n_seg, 256, 0, st, d_seg_len, w.stride, w.bsum,
+                  (float)top_db, d_bounds);
 }

@@ -360,13 +360,8 @@ extern "C" int ncfa_param_upload(void *d_dst, const void *h_pinned_src, size_t n
     }
     const size_t vecs = (nbytes + 15) / 16;
     const int grid = (int)std::min<size_t>(64, (vecs + 255) / 256);
-    {
-        ProfScope _p("param_upload_kernel", (cudaStream_t)stream);
-        param_upload_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>((unsigned char *)d_dst, (const unsigned char *)dsrc,
-                                                                nbytes);
-    }
-    NCFA_LAUNCH_OK("param_upload_kernel");
-    return NCFA_OK;
+    return launch("param_upload_kernel", param_upload_kernel, grid, 256, 0, (cudaStream_t)stream,
+                  (unsigned char *)d_dst, (const unsigned char *)dsrc, nbytes);
 }
 
 // Host-only view of the lane-transposed mel bank (tests/test_host_tables.py): h_lane_bin0 int32[128] ((q, lane) order),

@@ -20,15 +20,6 @@ void set_error(const char *fmt, ...);
         }                                                                                           \
     } while (0)
 
-#define NCFA_LAUNCH_OK(name)                                                                        \
-    do {                                                                                            \
-        cudaError_t _e = cudaGetLastError();                                                        \
-        if (_e != cudaSuccess) {                                                                    \
-            ncfa::set_error("launch of %s failed: %s", name, cudaGetErrorString(_e));                \
-            return NCFA_E_CUDA;                                                                     \
-        }                                                                                           \
-    } while (0)
-
 #define NCFA_REQUIRE(cond, msg)                                                                     \
     do {                                                                                            \
         if (!(cond)) {                                                                              \
@@ -39,14 +30,34 @@ void set_error(const char *fmt, ...);
 
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
+// Bump allocator over a workspace: every region starts on a 256-byte boundary.  With base == nullptr it only measures,
+// so one layout function per family serves both its ncfa_*_workspace_bytes query and its entry point.
+struct Carve {
+    char *base;
+    size_t used = 0;
+    explicit Carve(void *b) : base((char *)b) {}
+    template <class T>
+    T *take(size_t n) {
+        T *p = base ? (T *)(base + used) : nullptr;
+        used += align_up(n * sizeof(T), 256);
+        return p;
+    }
+};
+
+inline int check_workspace(const char *family, size_t have, size_t need) {
+    if (have >= need) return NCFA_OK;
+    set_error("%s workspace too small: %zu < %zu", family, have, need);
+    return NCFA_E_WORKSPACE;
+}
+
 // Thread-safe, monotonic cudaFuncAttributeMaxDynamicSharedMemorySize (host threads on different streams share kernels).
 int ensure_dynamic_smem(const void *func, size_t bytes);
 // SM count of the current device (cached)
 int sm_count(int *out);
 
-// Every launch site sits in a ProfScope.  It always opens an NVTX range named after the kernel family (header-only
-// NVTX3: a no-op costing one predicted branch unless a tool such as ncu / nsys injected itself), and —
-// optional per-kernel timing (ncfa_profile_enable) — a ProfScope around a launch records two CUDA events on the launch
+// Every launch goes through launch() below, so it sits in a ProfScope.  A ProfScope always opens an NVTX range named
+// after the kernel family (header-only NVTX3: a no-op costing one predicted branch unless a tool such as ncu / nsys
+// injected itself), and — optional per-kernel timing (ncfa_profile_enable) — records two CUDA events on the launch
 // stream (it owns both, so scopes of concurrent host threads never pair up with each other) and hands them to the
 // registry when it closes; ncfa_profile_report() synchronises them and sums per kernel name.
 bool prof_enabled();
@@ -68,6 +79,26 @@ struct ProfScope {
         nvtxRangePop();
     }
 };
+
+// Launches k<<<grid, block, smem, st>>>(args...) under ProfScope(name).  Any dynamic shared memory first raises the
+// kernel's limit to smem: the default limit is 48 KB less the kernel's static shared memory, so smem just under 48 KB
+// can need it too.  Returns NCFA_E_CUDA (the message names `name`) if the launch was rejected.
+template <class... P, class... A>
+int launch(const char *name, void (*k)(P...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, A &&...args) {
+    if (smem > 0) {
+        if (int rc = ensure_dynamic_smem((const void *)k, smem)) return rc;
+    }
+    {
+        ProfScope _p(name, st);
+        k<<<grid, block, smem, st>>>(static_cast<A &&>(args)...);
+    }
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) {
+        set_error("launch of %s failed: %s", name, cudaGetErrorString(e));
+        return NCFA_E_CUDA;
+    }
+    return NCFA_OK;
+}
 
 // Constant tables that live in device global memory, one set per device (see ncfa_api.cu).
 struct Tables {

@@ -186,10 +186,26 @@ static int spectral_ctas(int n_seg) {
     return c < 1 ? 1 : c;
 }
 
+// per segment `ctas` CTAs, each with kSpSlots pass-1 partial sums and kSpBins pass-2 per-bin partial sums
+struct SpectralWs {
+    int ctas;
+    double *partial, *bin_partial;
+    size_t bytes;
+};
+
+static SpectralWs spectral_ws(int n_seg, void *base) {
+    Carve c(base);
+    SpectralWs w;
+    w.ctas = spectral_ctas(n_seg);
+    w.partial = c.take<double>((size_t)n_seg * w.ctas * kSpSlots);
+    w.bin_partial = c.take<double>((size_t)n_seg * w.ctas * kSpBins);
+    w.bytes = c.used;
+    return w;
+}
+
 extern "C" size_t ncfa_spectral_workspace_bytes(int n_seg) {
     if (n_seg <= 0) return 0;
-    const size_t ctas = (size_t)spectral_ctas(n_seg);
-    return align_up((size_t)n_seg * ctas * kSpSlots * 8, 256) + align_up((size_t)n_seg * ctas * kSpBins * 8, 256);
+    return spectral_ws(n_seg, nullptr).bytes;
 }
 
 extern "C" int ncfa_spectral_stats_batched(const float *d_audio, const int64_t *d_seg_off, const int32_t *d_seg_len,
@@ -199,13 +215,11 @@ extern "C" int ncfa_spectral_stats_batched(const float *d_audio, const int64_t *
     if (n_seg == 0) return NCFA_OK;
     NCFA_REQUIRE(d_audio && d_seg_off && d_seg_len && d_stats && d_bin_db_mean && d_workspace, "null pointer");
     NCFA_REQUIRE(sr > 0, "sr");
-    if (workspace_bytes < ncfa_spectral_workspace_bytes(n_seg)) {
-        set_error("spectral workspace too small");
-        return NCFA_E_WORKSPACE;
-    }
-    Tables tb;
-    int rc = get_tables(sr, &tb);
+    const SpectralWs w = spectral_ws(n_seg, d_workspace);
+    int rc = check_workspace("spectral", workspace_bytes, w.bytes);
     if (rc) return rc;
+    Tables tb;
+    if ((rc = get_tables(sr, &tb))) return rc;
     // band masks of spectral.py:70-78: (freqs >= lo) & (freqs < hi) with freqs = k · (1 / (n_fft · (1/sr)))
     const double val = 1.0 / (2048.0 * (1.0 / (double)sr));
     const double edges[5][2] = {{20, 80}, {80, 250}, {250, 2000}, {2000, 6000}, {6000, 20000}};
@@ -219,28 +233,15 @@ extern "C" int ncfa_spectral_stats_batched(const float *d_audio, const int64_t *
         bands.hi[b] = hi;
     }
     cudaStream_t st = (cudaStream_t)stream;
-    const int ctas = spectral_ctas(n_seg);
-    double *partial = (double *)d_workspace;
-    double *bin_partial = (double *)((char *)d_workspace + align_up((size_t)n_seg * ctas * kSpSlots * 8, 256));
-    if ((rc = ensure_dynamic_smem((const void *)spectral_pass1_kernel, sizeof(SpectralSmem)))) return rc;
-    if ((rc = ensure_dynamic_smem((const void *)spectral_pass2_kernel, sizeof(SpectralSmem)))) return rc;
-    dim3 g(ctas, n_seg);
-    {
-        ProfScope _p("spectral_pass1_kernel", st);
-        spectral_pass1_kernel<<<g, kSpThreads, sizeof(SpectralSmem), st>>>(d_audio, d_seg_off, d_seg_len, (double)sr / 2048.0,
-                                                                           bands, tb, partial);
-    }
-    NCFA_LAUNCH_OK("spectral_pass1_kernel");
-    spectral_reduce1_kernel<<<n_seg, 32, 0, st>>>(partial, ctas, d_stats);
-    NCFA_LAUNCH_OK("spectral_reduce1_kernel");
-    {
-        ProfScope _p("spectral_pass2_kernel", st);
-        spectral_pass2_kernel<<<g, kSpThreads, sizeof(SpectralSmem), st>>>(d_audio, d_seg_off, d_seg_len, tb, d_stats,
-                                                                           bin_partial);
-    }
-    NCFA_LAUNCH_OK("spectral_pass2_kernel");
-    dim3 g2((kSpBins + 255) / 256, n_seg);
-    spectral_reduce2_kernel<<<g2, 256, 0, st>>>(bin_partial, ctas, d_seg_len, d_bin_db_mean);
-    NCFA_LAUNCH_OK("spectral_reduce2_kernel");
-    return NCFA_OK;
+    const dim3 g(w.ctas, n_seg);
+    if ((rc = launch("spectral_pass1_kernel", spectral_pass1_kernel, g, kSpThreads, sizeof(SpectralSmem), st, d_audio,
+                     d_seg_off, d_seg_len, (double)sr / 2048.0, bands, tb, w.partial)))
+        return rc;
+    if ((rc = launch("spectral_reduce1_kernel", spectral_reduce1_kernel, n_seg, 32, 0, st, w.partial, w.ctas, d_stats)))
+        return rc;
+    if ((rc = launch("spectral_pass2_kernel", spectral_pass2_kernel, g, kSpThreads, sizeof(SpectralSmem), st, d_audio,
+                     d_seg_off, d_seg_len, tb, d_stats, w.bin_partial)))
+        return rc;
+    return launch("spectral_reduce2_kernel", spectral_reduce2_kernel, dim3((kSpBins + 255) / 256, n_seg), 256, 0, st,
+                  w.bin_partial, w.ctas, d_seg_len, d_bin_db_mean);
 }

@@ -151,14 +151,30 @@ __global__ void __launch_bounds__(256) flux_kernel(const float *__restrict__ S, 
     }
 }
 
+// log-mel spectrogram S in whole tiles of 32 frames per segment, then one ordered-uint maximum per segment
+struct OnsetWs {
+    float *S;
+    unsigned *seg_max;
+    size_t bytes;
+};
+
+static OnsetWs onset_ws(int n_seg, int max_seg_len, int hop, void *base) {
+    Carve c(base);
+    OnsetWs w;
+    const size_t frames = (1 + (size_t)max_seg_len / hop + 31) / 32 * 32;
+    w.S = c.take<float>((size_t)n_seg * frames * NCFA_N_MELS);
+    w.seg_max = c.take<unsigned>(n_seg);
+    w.bytes = c.used;
+    return w;
+}
+
 }  // namespace ncfa
 
 using namespace ncfa;
 
 extern "C" size_t ncfa_onset_workspace_bytes(int n_seg, int max_seg_len, int hop) {
     if (n_seg <= 0 || hop <= 0 || max_seg_len < 0) return 0;
-    size_t frames = (1 + (size_t)max_seg_len / hop + 31) / 32 * 32;  // whole tiles of 32 frames
-    return align_up((size_t)n_seg * frames * NCFA_N_MELS * sizeof(float), 256) + align_up((size_t)n_seg * 4, 256);
+    return onset_ws(n_seg, max_seg_len, hop, nullptr).bytes;
 }
 
 extern "C" int ncfa_onset_strength_batched(const float *d_audio, const int64_t *d_seg_off, const int32_t *d_seg_len,
@@ -170,20 +186,14 @@ extern "C" int ncfa_onset_strength_batched(const float *d_audio, const int64_t *
     NCFA_REQUIRE(d_audio && d_seg_off && d_seg_len && d_onset && d_onset_off && d_workspace, "null pointer");
     NCFA_REQUIRE(hop >= 16 && hop <= 1024 && (hop % 2) == 0, "hop must be even and in [16, 1024]");
     NCFA_REQUIRE(max_seg_len >= 0, "max_seg_len");
-    if (workspace_bytes < ncfa_onset_workspace_bytes(n_seg, max_seg_len, hop)) {
-        set_error("onset workspace too small: %zu < %zu", workspace_bytes,
-                  ncfa_onset_workspace_bytes(n_seg, max_seg_len, hop));
-        return NCFA_E_WORKSPACE;
-    }
-    Tables tb;
-    int rc = get_tables(sr, &tb);
+    const OnsetWs w = onset_ws(n_seg, max_seg_len, hop, d_workspace);
+    int rc = check_workspace("onset", workspace_bytes, w.bytes);
     if (rc) return rc;
+    Tables tb;
+    if ((rc = get_tables(sr, &tb))) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     const int frames = 1 + max_seg_len / hop;
-    const int tiles_per_seg = (frames + 31) / 32;  // the workspace is sized in whole tiles of 32 frames
-    float *S = (float *)d_workspace;
-    unsigned *seg_max = (unsigned *)((char *)d_workspace + align_up((size_t)n_seg * tiles_per_seg * 32 * NCFA_N_MELS * 4, 256));
-    NCFA_CUDA_OK(cudaMemsetAsync(seg_max, 0, (size_t)n_seg * 4, st));
+    NCFA_CUDA_OK(cudaMemsetAsync(w.seg_max, 0, (size_t)n_seg * 4, st));
     int n_sm = 0;
     if ((rc = sm_count(&n_sm))) return rc;
     // as many warps as the 227 KB of shared memory hold (12 at 22 050 Hz: 95 mel-weight rows)
@@ -194,29 +204,11 @@ extern "C" int ncfa_onset_strength_batched(const float *d_audio, const int64_t *
     const size_t smem = fixed + (size_t)warps * kScrBytes2;
     const int64_t groups = ((int64_t)n_seg * ((frames + 1) / 2) + warps - 1) / warps;
     const int grid = (int)(groups < n_sm ? groups : n_sm);  // persistent: one CTA per SM
-    {
-        ProfScope _p(hop <= 128 ? "stft_logmel_kernel[hop<=128]" : "stft_logmel_kernel[hop>128]", st);
-        if (hop == 64) {
-            if ((rc = ensure_dynamic_smem((const void *)stft_logmel2_kernel<1>, smem))) return rc;
-            stft_logmel2_kernel<1><<<grid, warps * 32, smem, st>>>(d_audio, d_seg_off, d_seg_len, n_seg, hop, frames, tb, S,
-                                                                 seg_max);
-        } else if (hop == 512) {
-            if ((rc = ensure_dynamic_smem((const void *)stft_logmel2_kernel<8>, smem))) return rc;
-            stft_logmel2_kernel<8><<<grid, warps * 32, smem, st>>>(d_audio, d_seg_off, d_seg_len, n_seg, hop, frames, tb, S,
-                                                                 seg_max);
-        } else {
-            if ((rc = ensure_dynamic_smem((const void *)stft_logmel2_kernel<0>, smem))) return rc;
-            stft_logmel2_kernel<0><<<grid, warps * 32, smem, st>>>(d_audio, d_seg_off, d_seg_len, n_seg, hop, frames, tb, S,
-                                                                 seg_max);
-        }
-    }
-    NCFA_LAUNCH_OK("stft_logmel_kernel");
+    auto logmel = hop == 64 ? stft_logmel2_kernel<1> : (hop == 512 ? stft_logmel2_kernel<8> : stft_logmel2_kernel<0>);
+    if ((rc = launch(hop <= 128 ? "stft_logmel_kernel[hop<=128]" : "stft_logmel_kernel[hop>128]", logmel, grid,
+                     warps * 32, smem, st, d_audio, d_seg_off, d_seg_len, n_seg, hop, frames, tb, w.S, w.seg_max)))
+        return rc;
     const int pad = 1 + NCFA_N_FFT / (2 * hop);
-    dim3 g2((frames + 8 * kFluxRun - 1) / (8 * kFluxRun), n_seg);
-    {
-        ProfScope _p("flux_kernel", st);
-        flux_kernel<<<g2, 256, 0, st>>>(S, seg_max, d_seg_len, hop, frames, pad, d_onset, d_onset_off);
-    }
-    NCFA_LAUNCH_OK("flux_kernel");
-    return NCFA_OK;
+    return launch("flux_kernel", flux_kernel, dim3((frames + 8 * kFluxRun - 1) / (8 * kFluxRun), n_seg), 256, 0, st,
+                  w.S, w.seg_max, d_seg_len, hop, frames, pad, d_onset, d_onset_off);
 }

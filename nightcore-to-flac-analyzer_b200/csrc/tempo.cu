@@ -436,17 +436,37 @@ static int tempo_chunk(int max_env_len) {
     return 4096;
 }
 
+struct TempoWs {
+    double2 *trig;
+    double *w2, *r0, *r0inv, *partial;
+    int2 *range1, *range2, *hull;
+    size_t bytes;
+};
+
+static TempoWs tempo_ws(int n_seg, int max_env_len, int W, void *base) {
+    const int chunk = tempo_chunk(max_env_len);
+    const size_t n_chunks = (max_env_len + chunk - 1) / chunk;
+    Carve c(base);
+    TempoWs w;
+    w.trig = c.take<double2>(W);
+    w.w2 = c.take<double>(W);
+    w.r0 = c.take<double>((size_t)n_seg * max_env_len);
+    w.r0inv = c.take<double>((size_t)n_seg * max_env_len);
+    w.partial = c.take<double>((size_t)n_seg * n_chunks * W);
+    w.range1 = c.take<int2>(n_seg);
+    w.range2 = c.take<int2>(n_seg);
+    w.hull = c.take<int2>(n_seg);
+    w.bytes = c.used;
+    return w;
+}
+
 }  // namespace ncfa
 
 using namespace ncfa;
 
 extern "C" size_t ncfa_tempo_workspace_bytes(int n_seg, int max_env_len, int win_length) {
     if (n_seg <= 0 || max_env_len <= 0 || win_length <= 0) return 0;
-    const int chunk = tempo_chunk(max_env_len);
-    const size_t n_chunks = (max_env_len + chunk - 1) / chunk;
-    return align_up((size_t)win_length * sizeof(double2), 256) + align_up((size_t)win_length * 8, 256) +
-           2 * align_up((size_t)n_seg * max_env_len * 8, 256) + align_up((size_t)n_seg * n_chunks * win_length * 8, 256) +
-           3 * align_up((size_t)n_seg * sizeof(int2), 256);
+    return tempo_ws(n_seg, max_env_len, win_length, nullptr).bytes;
 }
 
 extern "C" int ncfa_tempo_lag_batched(const float *d_onset, const int64_t *d_onset_off, const int32_t *d_env_len,
@@ -458,40 +478,19 @@ extern "C" int ncfa_tempo_lag_batched(const float *d_onset, const int64_t *d_ons
     NCFA_REQUIRE(hop > 0 && sr > 0 && max_env_len > 0, "hop/sr/max_env_len");
     const int W = (int)floor(8.0 * (double)sr / (double)hop);  // time_to_frames(ac_size=8.0)
     NCFA_REQUIRE(W >= 4 && W <= 5000, "win_length out of the supported range [4, 5000]");
-    if (workspace_bytes < ncfa_tempo_workspace_bytes(n_seg, max_env_len, W)) {
-        set_error("tempo workspace too small");
-        return NCFA_E_WORKSPACE;
-    }
+    const TempoWs w = tempo_ws(n_seg, max_env_len, W, d_workspace);
+    int rc = check_workspace("tempo", workspace_bytes, w.bytes);
+    if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     const int chunk = tempo_chunk(max_env_len);
     const int n_chunks = (max_env_len + chunk - 1) / chunk;
-    char *wp = (char *)d_workspace;
-    double2 *trig = (double2 *)wp;
-    wp += align_up((size_t)W * sizeof(double2), 256);
-    double *w2 = (double *)wp;
-    wp += align_up((size_t)W * 8, 256);
-    double *r0 = (double *)wp;
-    wp += align_up((size_t)n_seg * max_env_len * 8, 256);
-    double *r0inv = (double *)wp;
-    wp += align_up((size_t)n_seg * max_env_len * 8, 256);
-    double *partial = (double *)wp;
-    wp += align_up((size_t)n_seg * n_chunks * W * 8, 256);
-    int2 *range1 = (int2 *)wp;
-    wp += align_up((size_t)n_seg * sizeof(int2), 256);
-    int2 *range2 = (int2 *)wp;
-    wp += align_up((size_t)n_seg * sizeof(int2), 256);
-    int2 *hull = (int2 *)wp;
 
     // first lag whose bpm is below max_tempo = 320 (logprior[:max_idx] = -inf)
     int k_min = 1;
     while (k_min < W && !((60.0 * (double)sr) / ((double)hop * (double)k_min) < 320.0)) ++k_min;
     NCFA_REQUIRE(k_min < W, "no admissible lag");
 
-    {
-        ProfScope _p("tg_tables_kernel", st);
-        tg_tables_kernel<<<(W + 255) / 256, 256, 0, st>>>(W, trig, w2);
-    }
-    NCFA_LAUNCH_OK("tg_tables_kernel");
+    if ((rc = launch("tg_tables_kernel", tg_tables_kernel, (W + 255) / 256, 256, 0, st, W, w.trig, w.w2))) return rc;
     {
         // frames per CTA: 8192 for whole tracks, one warp's worth of 32-frame blocks for short envelopes
         int threads = ((max_env_len + kR0Block - 1) / kR0Block + 31) / 32 * 32;
@@ -501,60 +500,30 @@ extern "C" int ncfa_tempo_lag_batched(const float *d_onset, const int64_t *d_ons
         const int span_cap = per_cta + W;
         const int n_blocks = (span_cap + 31) / 32;
         size_t sh = (size_t)(span_cap + 32 + ((span_cap + 32) >> 5) + 2 + 5 * n_blocks) * 8;
-        if (sh > 48 * 1024) {
-            int rc = ensure_dynamic_smem((const void *)tg_r0_kernel, sh);
-            if (rc) return rc;
-        }
-        {
-            ProfScope _p("tg_r0_kernel", st);
-            tg_r0_kernel<<<g, threads, sh, st>>>(d_onset, d_onset_off, d_env_len, max_env_len, W, trig, w2, r0, r0inv,
-                                                 per_cta);
-        }
-        NCFA_LAUNCH_OK("tg_r0_kernel");
+        if ((rc = launch("tg_r0_kernel", tg_r0_kernel, g, threads, sh, st, d_onset, d_onset_off, d_env_len, max_env_len,
+                         W, w.trig, w.w2, w.r0, w.r0inv, per_cta)))
+            return rc;
     }
-    {
-        ProfScope _p("tg_range_kernel", st);
-        tg_range_kernel<<<(n_seg + 127) / 128, 128, 0, st>>>(n_seg, W, k_min, hop, sr, d_start_bpm, range1);
-    }
-    NCFA_LAUNCH_OK("tg_range_kernel");
-    {
-        size_t sh = (size_t)(chunk + W) * 4;
-        if (sh > 48 * 1024) {
-            int rc = ensure_dynamic_smem((const void *)tg_lag_kernel, sh);
-            if (rc) return rc;
-        }
-        {
-            const int warps = n_seg * n_chunks;
-            ProfScope _p("tg_flags_kernel", st);
-            tg_flags_kernel<<<(warps + 3) / 4, 128, 0, st>>>(d_env_len, max_env_len, chunk, n_chunks, n_seg, r0, r0inv);
-        }
-        NCFA_LAUNCH_OK("tg_flags_kernel");
-        const int lag_blocks = (W - k_min + kLagThreads - 1) / kLagThreads;
-        dim3 g(lag_blocks < 2 ? lag_blocks : 2, n_chunks, n_seg);   // a CTA strides over the lag blocks (see the kernel)
-        {
-            ProfScope _p(n_chunks > 1 ? "tg_lag_kernel[long]" : "tg_lag_kernel", st);
-            tg_lag_kernel<<<g, kLagThreads, sh, st>>>(d_onset, d_onset_off, d_env_len, max_env_len, W, chunk, n_chunks, trig,
-                                                  r0inv, range1, nullptr, partial);
-        }
-        NCFA_LAUNCH_OK("tg_lag_kernel");
-        {
-            ProfScope _p("tg_bound_kernel", st);
-            tg_bound_kernel<<<n_seg, 256, 0, st>>>(d_env_len, W, n_chunks, chunk, k_min, hop, sr, d_start_bpm, partial,
-                                               range1, range2, hull);
-        }
-        NCFA_LAUNCH_OK("tg_bound_kernel");
-        {
-            ProfScope _p(n_chunks > 1 ? "tg_lag_kernel[long]" : "tg_lag_kernel", st);
-            tg_lag_kernel<<<g, kLagThreads, sh, st>>>(d_onset, d_onset_off, d_env_len, max_env_len, W, chunk, n_chunks, trig,
-                                                  r0inv, range2, range1, partial);
-        }
-        NCFA_LAUNCH_OK("tg_lag_kernel");
-    }
-    {
-        ProfScope _p("tg_argmax_kernel", st);
-        tg_argmax_kernel<<<n_seg, 256, 0, st>>>(d_onset, d_onset_off, d_env_len, W, n_chunks, chunk, k_min, hop, sr,
-                                            d_start_bpm, partial, hull, d_lag);
-    }
-    NCFA_LAUNCH_OK("tg_argmax_kernel");
-    return NCFA_OK;
+    if ((rc = launch("tg_range_kernel", tg_range_kernel, (n_seg + 127) / 128, 128, 0, st, n_seg, W, k_min, hop, sr,
+                     d_start_bpm, w.range1)))
+        return rc;
+    const int warps = n_seg * n_chunks;
+    if ((rc = launch("tg_flags_kernel", tg_flags_kernel, (warps + 3) / 4, 128, 0, st, d_env_len, max_env_len, chunk,
+                     n_chunks, n_seg, w.r0, w.r0inv)))
+        return rc;
+    const char *lag_name = n_chunks > 1 ? "tg_lag_kernel[long]" : "tg_lag_kernel";
+    const int lag_blocks = (W - k_min + kLagThreads - 1) / kLagThreads;
+    const dim3 g(lag_blocks < 2 ? lag_blocks : 2, n_chunks, n_seg);  // a CTA strides over the lag blocks (the kernel)
+    const size_t sh = (size_t)(chunk + W) * 4;
+    if ((rc = launch(lag_name, tg_lag_kernel, g, kLagThreads, sh, st, d_onset, d_onset_off, d_env_len, max_env_len, W,
+                     chunk, n_chunks, w.trig, w.r0inv, w.range1, nullptr, w.partial)))
+        return rc;
+    if ((rc = launch("tg_bound_kernel", tg_bound_kernel, n_seg, 256, 0, st, d_env_len, W, n_chunks, chunk, k_min, hop,
+                     sr, d_start_bpm, w.partial, w.range1, w.range2, w.hull)))
+        return rc;
+    if ((rc = launch(lag_name, tg_lag_kernel, g, kLagThreads, sh, st, d_onset, d_onset_off, d_env_len, max_env_len, W,
+                     chunk, n_chunks, w.trig, w.r0inv, w.range2, w.range1, w.partial)))
+        return rc;
+    return launch("tg_argmax_kernel", tg_argmax_kernel, n_seg, 256, 0, st, d_onset, d_onset_off, d_env_len, W, n_chunks,
+                  chunk, k_min, hop, sr, d_start_bpm, w.partial, w.hull, d_lag);
 }

@@ -519,15 +519,46 @@ static void xr_kernel_for(decltype(&xcorr_blocks_ring_kernel<1, kXrG, kXrChunk, 
     *smem = sizeof(XrSmemT<NQ>);
 }
 
+// block form: (kMaxPieces + 1) partial tables of max_cand + kMaxPieces − 1 blocks per window, then ‖a‖² per window
+struct XcorrBlockWs {
+    double *part, *na2;
+    size_t bytes;
+};
+
+static XcorrBlockWs xcorr_block_ws(int n_windows, int max_cand, void *base) {
+    Carve c(base);
+    XcorrBlockWs w;
+    w.part = c.take<double>((size_t)n_windows * (kMaxPieces + 1) * (max_cand + kMaxPieces - 1));
+    w.na2 = c.take<double>(n_windows);
+    w.bytes = c.used;
+    return w;
+}
+
+// direct form: dot product and ‖b‖² per candidate, then ‖a‖² per window
+struct XcorrDirectWs {
+    double *dots, *nb2, *na2;
+    size_t bytes;
+};
+
+static XcorrDirectWs xcorr_direct_ws(int n_windows, int max_cand, void *base) {
+    Carve c(base);
+    XcorrDirectWs w;
+    w.dots = c.take<double>((size_t)n_windows * max_cand);
+    w.nb2 = c.take<double>((size_t)n_windows * max_cand);
+    w.na2 = c.take<double>(n_windows);
+    w.bytes = c.used;
+    return w;
+}
+
 }  // namespace ncfa
 
 using namespace ncfa;
 
 extern "C" size_t ncfa_xcorr_workspace_bytes(int n_windows, int max_cand) {
     if (n_windows <= 0 || max_cand <= 0) return 0;
-    // block form: (kMaxPieces + 1) partial tables of max_cand + kMaxPieces − 1 blocks per window; direct form: 2 tables
-    const size_t blocks = (size_t)max_cand + kMaxPieces - 1;
-    return align_up((size_t)n_windows * (kMaxPieces + 1) * blocks * 8, 256) + align_up((size_t)n_windows * 8, 256);
+    const size_t block = xcorr_block_ws(n_windows, max_cand, nullptr).bytes;
+    const size_t direct = xcorr_direct_ws(n_windows, max_cand, nullptr).bytes;
+    return block > direct ? block : direct;
 }
 
 extern "C" int ncfa_xcorr_search_batched(const float *d_a, const float *d_b, const int64_t *d_a_pos,
@@ -538,59 +569,35 @@ extern "C" int ncfa_xcorr_search_batched(const float *d_a, const float *d_b, con
     if (n_windows == 0) return NCFA_OK;
     NCFA_REQUIRE(d_a && d_b && d_a_pos && d_b_lo && d_n_cand && d_best_j && d_best_c && d_workspace, "null pointer");
     NCFA_REQUIRE(win > 0 && stride > 0 && max_cand > 0, "win/stride/max_cand");
-    if (workspace_bytes < ncfa_xcorr_workspace_bytes(n_windows, max_cand)) {
-        set_error("xcorr workspace too small");
-        return NCFA_E_WORKSPACE;
-    }
+    int rc = check_workspace("xcorr", workspace_bytes, ncfa_xcorr_workspace_bytes(n_windows, max_cand));
+    if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
-    char *wp = (char *)d_workspace;
     const int nq = win / stride;
     // the tail (win − nq·stride samples per candidate) is summed by one lane in the pick kernel: keep it short
     if (nq >= 1 && nq <= kMaxPieces && win - nq * stride <= 16) {
+        const XcorrBlockWs w = xcorr_block_ws(n_windows, max_cand, d_workspace);
         const int max_blocks = max_cand + kMaxPieces - 1;
-        double *part = (double *)wp;
-        double *na2b = (double *)(wp + align_up((size_t)n_windows * (kMaxPieces + 1) * max_blocks * 8, 256));
-        {
-            ProfScope _p("xcorr_blocks_kernel", st);
-            decltype(&xcorr_blocks_ring_kernel<1, kXrG, kXrChunk, kXrStages, kXrConsumers>) kfn;
-            size_t smem;
-            switch (nq) {
-                case 1: xr_kernel_for<1>(&kfn, &smem); break;
-                case 2: xr_kernel_for<2>(&kfn, &smem); break;
-                case 3: xr_kernel_for<3>(&kfn, &smem); break;
-                default: xr_kernel_for<4>(&kfn, &smem); break;
-            }
-            if (int rc = ensure_dynamic_smem((const void *)kfn, smem)) return rc;
-            dim3 g((max_cand + nq - 1 + kXrG - 1) / kXrG, n_windows);
-            kfn<<<g, kXrConsumers + 32, smem, st>>>(d_a, d_b, d_a_pos, d_b_lo, d_n_cand, max_blocks, win, stride, part, na2b);
+        decltype(&xcorr_blocks_ring_kernel<1, kXrG, kXrChunk, kXrStages, kXrConsumers>) kfn;
+        size_t smem;
+        switch (nq) {
+            case 1: xr_kernel_for<1>(&kfn, &smem); break;
+            case 2: xr_kernel_for<2>(&kfn, &smem); break;
+            case 3: xr_kernel_for<3>(&kfn, &smem); break;
+            default: xr_kernel_for<4>(&kfn, &smem); break;
         }
-        NCFA_LAUNCH_OK("xcorr_blocks_kernel");
-        {
-            ProfScope _p("xcorr_pick_kernel", st);
-            xcorr_pick_blocks_kernel<<<n_windows, 32, 0, st>>>(d_a, d_b, d_a_pos, d_b_lo, d_n_cand, max_blocks, nq, win, stride,
-                                                            rms_gate, part, na2b, d_best_j, d_best_c);
-        }
-        NCFA_LAUNCH_OK("xcorr_pick_blocks_kernel");
-        return NCFA_OK;
+        if ((rc = launch("xcorr_blocks_kernel", kfn, dim3((max_cand + nq - 1 + kXrG - 1) / kXrG, n_windows),
+                         kXrConsumers + 32, smem, st, d_a, d_b, d_a_pos, d_b_lo, d_n_cand, max_blocks, win, stride,
+                         w.part, w.na2)))
+            return rc;
+        return launch("xcorr_pick_kernel", xcorr_pick_blocks_kernel, n_windows, 32, 0, st, d_a, d_b, d_a_pos, d_b_lo,
+                      d_n_cand, max_blocks, nq, win, stride, rms_gate, w.part, w.na2, d_best_j, d_best_c);
     }
-    double *dots = (double *)wp;
-    wp += align_up((size_t)n_windows * max_cand * 8, 256);
-    double *nb2 = (double *)wp;
-    wp += align_up((size_t)n_windows * max_cand * 8, 256);
-    double *na2 = (double *)wp;
-    {
-        ProfScope _p("xcorr_dots_kernel", st);
-        dim3 g(max_cand + 1, n_windows);
-        xcorr_dots_kernel<<<g, kXcThreads, 0, st>>>(d_a, d_b, d_a_pos, d_b_lo, d_n_cand, max_cand, win, stride, dots, nb2,
-                                                na2);
-    }
-    NCFA_LAUNCH_OK("xcorr_dots_kernel");
-    {
-        ProfScope _p("xcorr_pick_kernel", st);
-        xcorr_pick_kernel<<<n_windows, 32, 0, st>>>(d_n_cand, max_cand, win, rms_gate, dots, nb2, na2, d_best_j, d_best_c);
-    }
-    NCFA_LAUNCH_OK("xcorr_pick_kernel");
-    return NCFA_OK;
+    const XcorrDirectWs w = xcorr_direct_ws(n_windows, max_cand, d_workspace);
+    if ((rc = launch("xcorr_dots_kernel", xcorr_dots_kernel, dim3(max_cand + 1, n_windows), kXcThreads, 0, st, d_a, d_b,
+                     d_a_pos, d_b_lo, d_n_cand, max_cand, win, stride, w.dots, w.nb2, w.na2)))
+        return rc;
+    return launch("xcorr_pick_kernel", xcorr_pick_kernel, n_windows, 32, 0, st, d_n_cand, max_cand, win, rms_gate,
+                  w.dots, w.nb2, w.na2, d_best_j, d_best_c);
 }
 
 extern "C" int ncfa_decimate2(const float *d_in, int64_t n_in, float *d_out, void *stream) {
@@ -600,25 +607,35 @@ extern "C" int ncfa_decimate2(const float *d_in, int64_t n_in, float *d_out, voi
     const double *hb = nullptr;
     int rc = ncfa::get_halfband_device(&hb);
     if (rc) return rc;
-    {
-        ProfScope _p("align_decimate2_kernel", (cudaStream_t)stream);
-        align_decimate2_kernel<<<(unsigned)((n_out + 255) / 256), 256, 0, (cudaStream_t)stream>>>(d_in, n_in, d_out, n_out, hb);
-    }
-    NCFA_LAUNCH_OK("align_decimate2_kernel");
-    return NCFA_OK;
+    return launch("align_decimate2_kernel", align_decimate2_kernel, (unsigned)((n_out + 255) / 256), 256, 0,
+                  (cudaStream_t)stream, d_in, n_in, d_out, n_out, hb);
 }
 
 extern "C" int ncfa_f32_to_f64(const float *d_in, int64_t n, double *d_out, void *stream) {
     NCFA_REQUIRE(d_in && d_out && n >= 0, "d_in/d_out/n");
     if (n == 0) return NCFA_OK;
-    f32_to_f64_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(d_in, n, d_out);
-    NCFA_LAUNCH_OK("f32_to_f64_kernel");
-    return NCFA_OK;
+    return launch("f32_to_f64_kernel", f32_to_f64_kernel, (unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream,
+                  d_in, n, d_out);
+}
+
+// the stretched nc envelope of every speed, then its correlation at every lag
+struct AlignWs {
+    double *stretched, *corr;
+    size_t bytes;
+};
+
+static AlignWs align_ws(int n_speeds, int max_stretched, int max_lags, void *base) {
+    Carve c(base);
+    AlignWs w;
+    w.stretched = c.take<double>((size_t)n_speeds * max_stretched);
+    w.corr = c.take<double>((size_t)n_speeds * max_lags);
+    w.bytes = c.used;
+    return w;
 }
 
 extern "C" size_t ncfa_align_workspace_bytes(int n_speeds, int max_stretched, int max_lags) {
     if (n_speeds <= 0 || max_stretched <= 0 || max_lags <= 0) return 0;
-    return align_up((size_t)n_speeds * max_stretched * 8, 256) + align_up((size_t)n_speeds * max_lags * 8, 256);
+    return align_ws(n_speeds, max_stretched, max_lags, nullptr).bytes;
 }
 
 extern "C" int ncfa_align_search(const double *d_src_env, int n_src, const double *d_nc_env, int n_nc,
@@ -630,31 +647,16 @@ extern "C" int ncfa_align_search(const double *d_src_env, int n_src, const doubl
     NCFA_REQUIRE(d_src_env && d_nc_env && d_n_stretched && d_n_lags && d_peak_idx && d_score && d_workspace, "null pointer");
     NCFA_REQUIRE(n_src > 0 && n_nc > 1 && max_stretched >= 2 && max_lags > 0, "n_src/n_nc/max_stretched/max_lags");
     // per speed n_stretched[s] + n_lags[s] − 1 <= n_src by construction (xcorr.py:232: search_len <= n_src − n_stretched)
-    if (workspace_bytes < ncfa_align_workspace_bytes(n_speeds, max_stretched, max_lags)) {
-        set_error("align workspace too small");
-        return NCFA_E_WORKSPACE;
-    }
+    const AlignWs w = align_ws(n_speeds, max_stretched, max_lags, d_workspace);
+    int rc = check_workspace("align", workspace_bytes, w.bytes);
+    if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
-    double *stretched = (double *)d_workspace;
-    double *corr = (double *)((char *)d_workspace + align_up((size_t)n_speeds * max_stretched * 8, 256));
-    {
-        ProfScope _p("align_stretch_kernel", st);
-        dim3 g((max_stretched + 255) / 256, n_speeds);
-        align_stretch_kernel<<<g, 256, 0, st>>>(d_nc_env, n_nc, d_n_stretched, max_stretched, stretched);
-    }
-    NCFA_LAUNCH_OK("align_stretch_kernel");
-    {
-        ProfScope _p("align_corr_kernel", st);
-        dim3 g(max_lags, n_speeds);
-        align_corr_kernel<<<g, kXcThreads, 0, st>>>(d_src_env, stretched, max_stretched, d_n_stretched, d_n_lags, max_lags,
-                                                corr);
-    }
-    NCFA_LAUNCH_OK("align_corr_kernel");
-    {
-        ProfScope _p("align_pick_kernel", st);
-        align_pick_kernel<<<n_speeds, kXcThreads, 0, st>>>(d_src_env, stretched, max_stretched, d_n_stretched, d_n_lags,
-                                                       max_lags, corr, d_peak_idx, d_score);
-    }
-    NCFA_LAUNCH_OK("align_pick_kernel");
-    return NCFA_OK;
+    if ((rc = launch("align_stretch_kernel", align_stretch_kernel, dim3((max_stretched + 255) / 256, n_speeds), 256, 0,
+                     st, d_nc_env, n_nc, d_n_stretched, max_stretched, w.stretched)))
+        return rc;
+    if ((rc = launch("align_corr_kernel", align_corr_kernel, dim3(max_lags, n_speeds), kXcThreads, 0, st, d_src_env,
+                     w.stretched, max_stretched, d_n_stretched, d_n_lags, max_lags, w.corr)))
+        return rc;
+    return launch("align_pick_kernel", align_pick_kernel, n_speeds, kXcThreads, 0, st, d_src_env, w.stretched,
+                  max_stretched, d_n_stretched, d_n_lags, max_lags, w.corr, d_peak_idx, d_score);
 }

@@ -31,6 +31,16 @@ def _ptr(t: Optional[torch.Tensor]) -> int:
     return 0 if t is None else t.data_ptr()
 
 
+def aligned_layout(lengths) -> Tuple[np.ndarray, int]:
+    """Offsets (int64) of arrays of the given lengths laid end to end in one buffer, each starting on a 4-sample (16 B)
+    boundary, and the buffer's total length.  Aligned starts put the kernels on their vector-load fast paths; any other
+    start gives the same results (tests/test_gpu_segment_placement.py)."""
+    padded = (np.asarray(lengths, dtype=np.int64) + 3) // 4 * 4
+    off = np.zeros(len(padded), dtype=np.int64)
+    np.cumsum(padded[:-1], out=off[1:])
+    return off, int(padded.sum())
+
+
 class Engine:
     def __init__(self, device: Optional[torch.device] = None):
         if not torch.cuda.is_available():
@@ -99,13 +109,7 @@ class Engine:
     def pack(self, arrays: Sequence[np.ndarray]) -> Tuple[torch.Tensor, np.ndarray, np.ndarray]:
         """Concatenate float32 arrays into one device buffer → (audio, seg_off int64, seg_len int32) (host descriptors)."""
         lens = np.array([len(a) for a in arrays], dtype=np.int32)
-        # 4-sample (16 B) aligned starts put the kernels on their vector-load fast paths; any other start gives the same
-        # results (tests/test_gpu_segment_placement.py)
-        starts = np.zeros(len(arrays), dtype=np.int64)
-        pos = 0
-        for i, n in enumerate(lens):
-            starts[i] = pos
-            pos += (int(n) + 3) // 4 * 4
+        starts, pos = aligned_layout(lens)
         host = torch.zeros(max(pos, 4), dtype=torch.float32)
         hn = host.numpy()
         for a, s, n in zip(arrays, starts, lens):
@@ -154,12 +158,7 @@ class Engine:
     @staticmethod
     def env_layout(seg_len: np.ndarray, hop: int) -> Tuple[np.ndarray, np.ndarray, int]:
         env_len = (1 + seg_len.astype(np.int64) // hop).astype(np.int32)
-        padded = (env_len.astype(np.int64) + 3) // 4 * 4
-        off = np.zeros(len(seg_len), dtype=np.int64)
-        if len(seg_len) > 1:
-            off[1:] = np.cumsum(padded)[:-1]
-        total = int(padded.sum()) if len(seg_len) else 0
-        return env_len, off, total
+        return (env_len, *aligned_layout(env_len))
 
     def onset_strength_dev(self, audio: torch.Tensor, seg_off: np.ndarray, seg_len: np.ndarray, hop: int, sr: int,
                            d_seg_off: Optional[torch.Tensor] = None, d_seg_len: Optional[torch.Tensor] = None):

@@ -65,11 +65,7 @@ def pin_pairs(pairs: Sequence[Tuple[np.ndarray, np.ndarray]], sr: int = SAMPLE_R
     """Lay [(nc_audio, src_audio), ...] out in one pinned host buffer (4-sample aligned track starts)."""
     tracks = [np.asarray(t, dtype=np.float32) for p in pairs for t in p]
     length = np.array([len(t) for t in tracks], dtype=np.int64)
-    padded = (length + 3) // 4 * 4
-    off = np.zeros(len(tracks), dtype=np.int64)
-    if len(tracks) > 1:
-        off[1:] = np.cumsum(padded)[:-1]
-    total = int(padded.sum()) if len(tracks) else 0
+    off, total = _engine.aligned_layout(length)
     if pinned is None or pinned.numel() < max(total, 4):
         pinned = torch.empty(max(total, 4), dtype=torch.float32, pin_memory=True)
     dst = pinned.numpy()
@@ -91,7 +87,7 @@ def upload(pb: PinnedBatch, n_pairs: Optional[int] = None, out: Optional[torch.T
         raise ValueError(f"pairs [{s}, {s + k}) outside the pinned batch of {pb.n_pairs} pairs")
     off, length = pb.off[2 * s : 2 * (s + k)], pb.length[2 * s : 2 * (s + k)]
     base = int(off[0]) if k else 0
-    total = int(off[-1] + (length[-1] + 3) // 4 * 4) - base if k else 0
+    total = _engine.aligned_layout(length)[1]
     n = max(total, 4)
     src = pb.pinned[base : base + n] if base + n <= pb.pinned.numel() else pb.pinned[base:]
     if out is not None and out.numel() >= n:
@@ -397,14 +393,6 @@ def release_buffers() -> None:
         _SLOTS.clear()
 
 
-def _layout(lengths: np.ndarray) -> Tuple[np.ndarray, int]:
-    padded = (lengths + 3) // 4 * 4
-    off = np.zeros(len(lengths), dtype=np.int64)
-    if len(lengths) > 1:
-        off[1:] = np.cumsum(padded)[:-1]
-    return off, int(padded.sum()) if len(lengths) else 0
-
-
 def analyse_batch(source, sr: int = SAMPLE_RATE, *, sub_batch: int = SUB_BATCH_PAIRS, workers: int = 2,
                   sizes: Optional[Sequence[int]] = None, stats: Optional[dict] = None, **kwargs):
     """Analyse every pair of ``source`` — a ``PinnedBatch`` (pin_pairs) or a sequence of ``(nc_audio, src_audio)``
@@ -446,7 +434,7 @@ def analyse_batch(source, sr: int = SAMPLE_RATE, *, sub_batch: int = SUB_BATCH_P
     device = eng.device
     main = torch.cuda.current_stream(device)
     nw = max(1, min(int(workers), len(sizes)))
-    need = max(_layout(lengths[2 * s : 2 * (s + k)])[1] for s, k in zip(starts, sizes))
+    need = max(_engine.aligned_layout(lengths[2 * s : 2 * (s + k)])[1] for s, k in zip(starts, sizes))
     with _SCHED_LOCK:       # one scheduled batch per process at a time (the slots are shared)
         # device slots: one per worker + TWO ahead.  With one ahead the copy of job j+3 cannot start before job j ends, and
         # a worker that finishes early finds nothing uploaded: measured 1036 pairs/s with 3 slots, 1218 with 4, 1227 with 6
@@ -475,10 +463,10 @@ def analyse_batch(source, sr: int = SAMPLE_RATE, *, sub_batch: int = SUB_BATCH_P
                     if pinned_in:
                         base = int(source.off[2 * s])
                         off = source.off[2 * s : 2 * (s + k)] - base
-                        total = int(off[-1] + (ln[-1] + 3) // 4 * 4)
+                        total = _engine.aligned_layout(ln)[1]
                         src = source.pinned[base : base + total]
                     else:
-                        off, total = _layout(ln)
+                        off, total = _engine.aligned_layout(ln)
                         dst = sl.pinned.numpy()       # pageable → pinned: one memcpy per track on a small thread pool
                         list(_stage_pool().map(lambda a: np.copyto(dst[a[1] : a[1] + len(a[0])], a[0]),
                                                zip(tracks[2 * s : 2 * (s + k)], off.tolist())))

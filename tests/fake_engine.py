@@ -12,6 +12,7 @@ from typing import List, Optional, Sequence, Tuple
 import numpy as np
 import torch
 
+from nightcore_analyzer._engine import aligned_layout
 from oracle import librosa_restated as lr
 from oracle import native
 
@@ -35,11 +36,7 @@ class FakeEngine:
 
     def pack(self, arrays: Sequence[np.ndarray]) -> Tuple[torch.Tensor, np.ndarray, np.ndarray]:
         lens = np.array([len(a) for a in arrays], dtype=np.int32)
-        starts = np.zeros(len(arrays), dtype=np.int64)
-        pos = 0
-        for i, n in enumerate(lens):
-            starts[i] = pos
-            pos += (int(n) + 3) // 4 * 4
+        starts, pos = aligned_layout(lens)
         host = torch.zeros(max(pos, 4), dtype=torch.float32)
         for a, s, n in zip(arrays, starts, lens):
             host.numpy()[s : s + n] = np.asarray(a, dtype=np.float32)

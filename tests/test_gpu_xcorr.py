@@ -78,6 +78,34 @@ def test_xcorr_direct_path_matches_port(engine):
     assert abs(quality - w_quality) <= 1e-5
 
 
+def test_xcorr_direct_form_stays_inside_its_workspace(engine):
+    """One window with one candidate in the direct form (win / stride = 8), given exactly ncfa_xcorr_workspace_bytes at
+    the start of a larger buffer: the bytes after it keep their pattern, and the pick is the cosine of the two
+    windows."""
+    import torch
+    from nightcore_analyzer._native import check, lib
+    win, stride = 4096, 512
+    rng = np.random.default_rng(21)
+    a = rng.standard_normal(win).astype(np.float32)
+    b = (a + 0.1 * rng.standard_normal(win)).astype(np.float32)
+    audio, off, _ = engine.pack([a, b])
+    d_pos, d_lo = engine.to_dev(off[:1]), engine.to_dev(off[1:])
+    d_n = engine.to_dev(np.array([1], np.int32))
+    need = lib.ncfa_xcorr_workspace_bytes(1, 1)
+    ws = torch.full((need + 4096,), 0xA5, dtype=torch.uint8, device=engine.device)
+    best_j = torch.empty(1, dtype=torch.int32, device=engine.device)
+    best_c = torch.empty(1, dtype=torch.float64, device=engine.device)
+    check(lib.ncfa_xcorr_search_batched(audio.data_ptr(), audio.data_ptr(), d_pos.data_ptr(), d_lo.data_ptr(),
+                                        d_n.data_ptr(), 1, 1, win, stride, 0.0, best_j.data_ptr(), best_c.data_ptr(),
+                                        ws.data_ptr(), need, torch.cuda.current_stream().cuda_stream),
+          "ncfa_xcorr_search_batched")
+    torch.cuda.synchronize()
+    assert bool((ws[need:] == 0xA5).all())
+    a64, b64 = a.astype(np.float64), b.astype(np.float64)
+    want = float(np.dot(a64, b64) / (np.linalg.norm(a64) * np.linalg.norm(b64)))
+    assert best_j.item() == 0
+    assert abs(best_c.item() - want) <= 1e-5
+
 def test_speed_xcorr_sentinels(engine):
     from nightcore_analyzer import xcorr as nx
     short = synth.synth(1, 3.0, SR, bpm=120.0)
