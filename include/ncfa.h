@@ -189,10 +189,33 @@ int ncfa_spectral_stats_batched(const float *d_audio, const int64_t *d_seg_off, 
                                 double *d_stats, float *d_bin_db_mean, void *d_workspace, size_t workspace_bytes,
                                 void *stream);
 
+/* ---- workflow.py:117 `sox SRC HQNC speed X`: band-limited speed change (the HQNC render) -------------------------
+ * Output m of segment i is the segment evaluated at input time t = m·R, R = ratio[i] (sox `speed R`: pitch and tempo
+ * both × R at the same sample rate), through a Kaiser-windowed sinc table T of Z zero crossings × L entries each:
+ *   T[j] = sinc(j/L)·I0(β·sqrt(1 − (j/(Z·L))²))/I0(β), j < Z·L;  T[Z·L] = 0   (float64, built on the host)
+ *   c = ρ/max(1, R), half = Z/c (input samples), n_out = ncfa_render_out_len(len, R) = len ? floor((len−1)/R) + 1 : 0
+ *   per output, in float64 and in this order: t = (double)m·R; n0 = floor(t − half) + 1; for k = 0 .. ceil(2·half),
+ *   n = n0 + k: d = (|t − n|·c)·L, i = floor(d), f = d − i; if i < Z·L and 0 <= n < len:
+ *   acc += (T[i] + f·(T[i+1] − T[i]))·(double)x[n];  y[m] = (float)(acc·c).
+ * Samples outside the segment count as zero.  Output i goes to d_out[d_out_off[i] ..  + n_out).  The ratios are passed
+ * twice: d_ratio is what the kernel reads, h_ratio (host memory, the same values) is checked before the launch (finite,
+ * in [0.25, 4]) so that a bad ratio is an NCFA_E_INVALID rather than a device-side condition.  max_seg_len bounds every
+ * d_seg_len[i] and sizes the grid; n_seg <= 65535 per call.  No workspace. */
+#define NCFA_RENDER_ZEROS 32
+#define NCFA_RENDER_PHASES 512
+#define NCFA_RENDER_BETA 10.0
+#define NCFA_RENDER_ROLLOFF 0.95
+int64_t ncfa_render_out_len(int32_t len, double ratio);
+int ncfa_render_batched(const float *d_audio, const int64_t *d_seg_off, const int32_t *d_seg_len, const double *d_ratio,
+                        const double *h_ratio, int n_seg, int max_seg_len, const int64_t *d_out_off, float *d_out,
+                        void *stream);
+
 /* Host-side constant-table builders (no GPU needed; used by the CPU test-suite):
  * h_K[1024][72] = the CQT contraction matrix of tuning index j; h_taps[127] = the half-band FIR. */
 int ncfa_host_cqt_matrix(int sr, int tuning_index, float *h_K);
 int ncfa_host_halfband_taps(double *h_taps);
+/* h_table[Z·L + 1] = the float64 sinc table ncfa_render_batched reads (see above). */
+int ncfa_host_render_table(double *h_table);
 /* Lane-transposed Slaney mel bank of the STFT kernels: h_lane_bin0 int32[4][32] first bin read by lane l of
  * group q (bands l, 63-l, 64+l, 127-l), h_qw int32[4] rows per group, h_wt float32[128][32] weights
  * (row = group offset + i, column = lane; zero outside a band's support). */

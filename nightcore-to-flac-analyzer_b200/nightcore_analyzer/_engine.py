@@ -457,6 +457,35 @@ class Engine:
         self.launches += 4
         return stats[:n_seg], bins[:n_seg]
 
+    # ------------------------------------------------------------------ render: band-limited speed change (sox speed)
+    @staticmethod
+    def render_layout(seg_len: np.ndarray, ratio: np.ndarray) -> Tuple[np.ndarray, np.ndarray, int]:
+        """(out_len int64, out_off int64, total) of the rendered segments; the length rule is the library's."""
+        out_len = np.array([lib.ncfa_render_out_len(int(n), float(r)) for n, r in zip(seg_len, ratio)], dtype=np.int64)
+        return (out_len, *aligned_layout(out_len))
+
+    def render_dev(self, audio: torch.Tensor, seg_off: np.ndarray, seg_len: np.ndarray, ratio) -> Tuple[torch.Tensor, np.ndarray]:
+        """Segment i played ratio[i] times faster (sox ``speed``, include/ncfa.h) → (out float32 packed on the device,
+        out_off int64 on the host); segment i's output is out[out_off[i] : out_off[i] + render_layout(...)[0][i]]."""
+        n_seg = len(seg_len)
+        ratio = np.broadcast_to(np.asarray(ratio, dtype=np.float64), (n_seg,)).copy()
+        _, out_off, total = self.render_layout(seg_len, ratio)
+        out = torch.empty(max(total, 4), dtype=torch.float32, device=self.device)
+        if n_seg == 0:
+            return out, out_off
+        d_off, d_len = self.to_dev(seg_off.astype(np.int64)), self.to_dev(seg_len.astype(np.int32))
+        d_ratio, d_out_off = self.to_dev(ratio), self.to_dev(out_off)
+        with torch.cuda.device(self.device):
+            st = self._stream()
+            for s in range(0, n_seg, MAX_SEGS_PER_CALL):
+                e = min(n_seg, s + MAX_SEGS_PER_CALL)
+                check(lib.ncfa_render_batched(_ptr(audio), d_off.data_ptr() + 8 * s, d_len.data_ptr() + 4 * s,
+                                              d_ratio.data_ptr() + 8 * s, ratio[s:].ctypes.data, e - s,
+                                              int(seg_len[s:e].max()), d_out_off.data_ptr() + 8 * s, _ptr(out), st),
+                      "ncfa_render_batched")
+                self.launches += 1
+        return out, out_off
+
     # ------------------------------------------------------------------ host conveniences
     def onset_strength(self, arrays: Sequence[np.ndarray], hop: int, sr: int) -> List[np.ndarray]:
         audio, off, ln = self.pack(arrays)

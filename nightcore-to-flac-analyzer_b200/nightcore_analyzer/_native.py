@@ -68,6 +68,9 @@ _SIGNATURES = {
     "ncfa_align_search": (c_int, [_P, c_int, _P, c_int, _P, _P, c_int, c_int, c_int, _P, _P, _P, c_size_t, _P]),
     "ncfa_spectral_workspace_bytes": (c_size_t, [c_int]),
     "ncfa_spectral_stats_batched": (c_int, [_P, _P, _P, c_int, c_int, _P, _P, _P, c_size_t, _P]),
+    "ncfa_render_out_len": (c_int64, [c_int32, c_double]),
+    "ncfa_render_batched": (c_int, [_P, _P, _P, _P, _P, c_int, c_int, _P, _P, _P]),
+    "ncfa_host_render_table": (c_int, [_P]),
     "ncfa_host_cqt_matrix": (c_int, [c_int, c_int, _P]),
     "ncfa_host_halfband_taps": (c_int, [_P]),
     "ncfa_host_mel_lanes": (c_int, [c_int, _P, _P, _P]),

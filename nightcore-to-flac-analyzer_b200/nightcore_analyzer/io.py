@@ -69,26 +69,60 @@ def _rms_db(audio: np.ndarray) -> float:
     return _db_from_meansq(float(ms.cpu().numpy()[0]))
 
 
-def load_audio(path: str, sr: int = SAMPLE_RATE) -> tuple[np.ndarray, int]:
-    """io.py:44-55.  Decoding is out of scope (no librosa/soundfile on the box): accepts ``.npy``
-    (float mono already at *sr*) and PCM ``.wav``; a WAV at another rate is resampled with
-    scipy's polyphase filter (NOT soxr_hq — documented deviation)."""
-    path = str(path)
-    if path.endswith(".npy"):
-        return np.load(path).astype(np.float32), (sr or SAMPLE_RATE)
-    with wave.open(path, "rb") as w:
+def read_wav(path: str) -> tuple[np.ndarray, int, int]:
+    """PCM ``.wav`` → (frames float32 [n, channels], sample rate, sample width in bytes).  8-bit (unsigned), 16-, 24- and
+    32-bit (signed) samples are scaled by 2^(bits−1) into [−1, 1)."""
+    with wave.open(str(path), "rb") as w:
         n, ch, sw, fr = w.getnframes(), w.getnchannels(), w.getsampwidth(), w.getframerate()
         raw = w.readframes(n)
     if sw == 2:
         y = np.frombuffer(raw, dtype="<i2").astype(np.float32) / 32768.0
+    elif sw == 3:
+        b = np.frombuffer(raw, dtype=np.uint8).reshape(-1, 3).astype(np.int32)
+        v = b[:, 0] | (b[:, 1] << 8) | (b[:, 2] << 16)
+        y = (v - ((v & 0x800000) << 1)).astype(np.float32) / 8388608.0
     elif sw == 4:
         y = np.frombuffer(raw, dtype="<i4").astype(np.float32) / 2147483648.0
     elif sw == 1:
         y = (np.frombuffer(raw, dtype=np.uint8).astype(np.float32) - 128.0) / 128.0
     else:
         raise ValueError(f"unsupported WAV sample width {sw}")
-    if ch > 1:
-        y = y.reshape(-1, ch).mean(axis=1).astype(np.float32)
+    return y.reshape(-1, ch), fr, sw
+
+
+def write_wav(path: str, frames: np.ndarray, rate: int, sample_width: int = 2) -> None:
+    """frames ([n] or [n, channels], float, full scale ±1) → PCM ``.wav`` of `sample_width` bytes (1, 2, 3 or 4): scaled
+    by 2^(bits−1), rounded half to even and clipped to the integer range, without dither.  Writing what ``read_wav``
+    returned reproduces a 8-, 16- or 24-bit file's samples exactly."""
+    if sample_width not in (1, 2, 3, 4):
+        raise ValueError(f"unsupported WAV sample width {sample_width}")
+    y = np.asarray(frames, dtype=np.float64)
+    y = y.reshape(len(y), -1)
+    full = float(1 << (8 * sample_width - 1))
+    q = np.clip(np.rint(y * full), -full, full - 1).astype(np.int64)
+    if sample_width == 1:
+        raw = (q + 128).astype(np.uint8).tobytes()
+    elif sample_width == 3:
+        raw = (q.reshape(-1, 1) >> np.array([0, 8, 16])).astype(np.uint8).tobytes()
+    else:
+        raw = q.astype(f"<i{sample_width}").tobytes()
+    with wave.open(str(path), "wb") as w:
+        w.setnchannels(y.shape[1])
+        w.setsampwidth(sample_width)
+        w.setframerate(int(rate))
+        w.writeframes(raw)
+
+
+def load_audio(path: str, sr: int = SAMPLE_RATE) -> tuple[np.ndarray, int]:
+    """io.py:44-55.  Decoding is out of scope (no librosa/soundfile on the box): accepts ``.npy``
+    (float mono already at *sr*) and PCM ``.wav`` read by ``read_wav`` (8-, 16-, 24- or 32-bit; 24-bit files load since
+    ``read_wav`` was added, before that they raised ``ValueError``), averaged to mono; a WAV at another rate is
+    resampled with scipy's polyphase filter (NOT soxr_hq — documented deviation)."""
+    path = str(path)
+    if path.endswith(".npy"):
+        return np.load(path).astype(np.float32), (sr or SAMPLE_RATE)
+    frames, fr, _ = read_wav(path)
+    y = frames.mean(axis=1).astype(np.float32) if frames.shape[1] > 1 else frames[:, 0]
     if sr is not None and fr != sr:
         from fractions import Fraction
         import scipy.signal
