@@ -170,7 +170,10 @@ int ncfa_xcorr_search_batched(const float *d_a, const float *d_b, const int64_t 
  * ncfa_align_search: for each candidate speed s: stretched = np.interp(linspace(0,1,n_stretched[s]),
  *   linspace(0,1,n_nc), nc_env); corr = np.correlate(src_env, stretched, 'valid')[:n_lags[s]];
  *   d_peak_idx[s] = first argmax; d_score[s] = corr[peak]/sqrt(Σ src_env[peak:peak+n]²·Σ stretched²)
- *   (0 when the denominator is <= 1e-12).  n_lags[s] <= 0 marks a speed the reference skips. */
+ *   (0 when the denominator is <= 1e-12).  n_lags[s] <= 0 marks a speed the reference skips: its d_peak_idx is −1,
+ *   its d_score 0, and its n_stretched is ignored (it may exceed max_stretched).  Every other speed needs
+ *   1 <= n_stretched[s] <= max_stretched, n_lags[s] <= max_lags and n_stretched[s] + n_lags[s] − 1 <= n_src;
+ *   n_stretched = 1 is the single point np.linspace(0, 1, 1) = [0], i.e. nc_env[0]. */
 int ncfa_decimate2(const float *d_in, int64_t n_in, float *d_out, void *stream);
 int ncfa_f32_to_f64(const float *d_in, int64_t n, double *d_out, void *stream);
 size_t ncfa_align_workspace_bytes(int n_speeds, int max_stretched, int max_lags);

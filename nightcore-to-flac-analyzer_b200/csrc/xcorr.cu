@@ -398,14 +398,19 @@ __global__ void __launch_bounds__(256) f32_to_f64_kernel(const float *__restrict
     if (i < n) out[i] = (double)in[i];
 }
 
-// np.linspace(0, 1, n)[i]
-__device__ __forceinline__ double lin01(int i, int n, double step) { return (i == n - 1) ? 1.0 : __dmul_rn((double)i, step); }
+// np.linspace(0, 1, n)[i]: the one point of np.linspace(0, 1, 1) is the start, 0
+__device__ __forceinline__ double lin01(int i, int n, double step) {
+    return n == 1 ? 0.0 : (i == n - 1) ? 1.0 : __dmul_rn((double)i, step);
+}
 
-// stretched[s][i] = np.interp(linspace(0,1,ns)[i], linspace(0,1,n_nc), nc_env)
+// stretched[s][i] = np.interp(linspace(0,1,ns)[i], linspace(0,1,n_nc), nc_env).  A skipped speed (n_lag <= 0) writes
+// nothing: its n_str is not bounded by str_stride.
 __global__ void __launch_bounds__(256) align_stretch_kernel(const double *__restrict__ nc_env, int n_nc,
-                                                            const int32_t *__restrict__ n_str, int str_stride,
+                                                            const int32_t *__restrict__ n_str,
+                                                            const int32_t *__restrict__ n_lag, int str_stride,
                                                             double *__restrict__ stretched) {
     const int sp = blockIdx.y;
+    if (n_lag[sp] <= 0) return;
     const int ns = n_str[sp];
     const int i = blockIdx.x * 256 + threadIdx.x;
     if (i >= ns) return;
@@ -652,7 +657,7 @@ extern "C" int ncfa_align_search(const double *d_src_env, int n_src, const doubl
     if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     if ((rc = launch("align_stretch_kernel", align_stretch_kernel, dim3((max_stretched + 255) / 256, n_speeds), 256, 0,
-                     st, d_nc_env, n_nc, d_n_stretched, max_stretched, w.stretched)))
+                     st, d_nc_env, n_nc, d_n_stretched, d_n_lags, max_stretched, w.stretched)))
         return rc;
     if ((rc = launch("align_corr_kernel", align_corr_kernel, dim3(max_lags, n_speeds), kXcThreads, 0, st, d_src_env,
                      w.stretched, max_stretched, d_n_stretched, d_n_lags, max_lags, w.corr)))
