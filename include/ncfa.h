@@ -102,7 +102,9 @@ int ncfa_tempo_lag_batched(const float *d_onset, const int64_t *d_onset_off, con
  * Dynamic-programming beat tracker with frames-per-beat = d_lag[i] <= max_lag (tightness 100, trim=True;
  * max_lag = the tempogram win_length floor(8·sr/hop) bounds every lag ncfa_tempo_lag_batched returns).
  * d_beats holds max_beats int32 frames per segment (ascending); d_n_beats[i] the count
- * (NCFA_E_OVERFLOW is flagged in d_n_beats[i] = -1 if max_beats is too small). */
+ * (NCFA_E_OVERFLOW is flagged in d_n_beats[i] = -1 if max_beats is too small; the row then holds the first max_beats
+ * beats).  A segment with d_lag[i] < 2, d_lag[i] > max_lag or d_env_len[i] < 2 gets d_n_beats[i] = 0 and its row of
+ * d_beats is not written. */
 size_t ncfa_beat_workspace_bytes(int n_seg, int max_env_len, int max_lag);
 int ncfa_beat_track_batched(const float *d_onset, const int64_t *d_onset_off, const int32_t *d_env_len, int n_seg,
                             int max_env_len, const int32_t *d_lag, int max_lag, int32_t *d_beats, int max_beats,

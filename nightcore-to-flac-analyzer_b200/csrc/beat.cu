@@ -78,7 +78,8 @@ __device__ double select_localmax(const double *cum, int n, int rank, int *hist,
 }
 
 // Workspace of one segment (doubles): onorm[env_stride] | ls[env_stride] | cum[env_stride] | window[2·max_fpb+1] |
-// (2·max_fpb+1 unused) | 8 spare — spare[0] holds max(ls) as an order-preserving 64-bit key.
+// pen[2·max_fpb+1] (the DP's transition penalties for d = near .. 2·fpb, copied from shared memory) | 8 spare —
+// spare[0] holds max(ls) as an order-preserving 64-bit key.
 __device__ __forceinline__ double *beat_seg_base(double *ws_f64, int seg, int env_stride, int max_fpb) {
     const size_t K = 2 * (size_t)max_fpb + 1;
     return ws_f64 + (size_t)seg * (3 * (size_t)env_stride + 2 * K + 8);
@@ -238,7 +239,9 @@ __global__ void beat_track_kernel(const float *__restrict__ onset, const int64_t
     const double logf = log(dfpb);
     for (int d = near + tid; d <= far; d += nt) {
         double x = log((double)d) - logf;
-        pen[d - near] = 100.0 * (x * x);
+        const double p = 100.0 * (x * x);
+        pen[d - near] = p;
+        window[K + (d - near)] = p;  // the workspace copy lets a host check run the DP on this device's log
     }
     __syncthreads();
 

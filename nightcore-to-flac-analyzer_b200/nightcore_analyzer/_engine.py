@@ -41,6 +41,15 @@ def aligned_layout(lengths) -> Tuple[np.ndarray, int]:
     return off, int(padded.sum())
 
 
+def check_beat_counts(n_beats: np.ndarray) -> np.ndarray:
+    """Host copy of the beat counts of ncfa_beat_track_batched, returned as is.  A count of −1 marks a segment whose
+    beats did not fit its max_beats slots (Engine.max_beats_for rules that out for every lag the tempogram returns):
+    it raises here rather than being read as "too few beats"."""
+    if (np.asarray(n_beats) < 0).any():
+        raise _native.NcfaError("beat buffer overflow")
+    return n_beats
+
+
 class Engine:
     def __init__(self, device: Optional[torch.device] = None):
         if not torch.cuda.is_available():
@@ -506,9 +515,7 @@ class Engine:
         d_off, d_len = self.to_dev(off), self.to_dev(ln)
         d_lag = self.to_dev(np.asarray(lags, dtype=np.int32))
         beats, n_beats = self.beat_track_dev(onset, d_off, d_len, ln, d_lag, hop, sr)
-        hb, hn = beats.cpu().numpy(), n_beats.cpu().numpy()
-        if (hn < 0).any():
-            raise _native.NcfaError("beat buffer overflow")
+        hb, hn = beats.cpu().numpy(), check_beat_counts(n_beats.cpu().numpy())
         return [hb[i, : hn[i]].copy() for i in range(len(envelopes))]
 
     def tempo_and_beats(self, arrays: Sequence[np.ndarray], start_bpm: Sequence[float], hop: int, sr: int,
@@ -516,9 +523,7 @@ class Engine:
         """onset → tempo → beat DP for each array → (lags int32[n], list of beat-frame arrays | counts)."""
         audio, off, ln = self.pack(arrays)
         _, _, _, lag, beats, n_beats = self.tempo_segments_dev(audio, off, ln, np.asarray(start_bpm, np.float64), hop, sr)
-        hl, hn = lag.cpu().numpy(), n_beats.cpu().numpy()
-        if (hn < 0).any():
-            raise _native.NcfaError("beat buffer overflow")
+        hl, hn = lag.cpu().numpy(), check_beat_counts(n_beats.cpu().numpy())
         if not want_beats:
             return hl, hn
         hb = beats.cpu().numpy()

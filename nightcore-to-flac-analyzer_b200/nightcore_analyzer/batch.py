@@ -182,7 +182,7 @@ def analyse_staged(batch: StagedBatch, *, window_sec: float = WINDOW_SEC, hop_se
             return np.zeros(0, np.int32), np.zeros(0, np.int32)
         _, _, _, lag, _, n_beats = eng.tempo_segments_dev(batch.audio, seg_off[sel], seg_len[sel], bpm,
                                                           _tempo.HOP_LENGTH, sr)
-        return eng.to_host(lag), eng.to_host(n_beats)
+        return eng.to_host(lag), _engine.check_beat_counts(eng.to_host(n_beats))
 
     is_src = (seg_track % 2) == 1
     pair_of = seg_track // 2
@@ -228,7 +228,7 @@ def analyse_staged(batch: StagedBatch, *, window_sec: float = WINDOW_SEC, hop_se
         bpm = np.array([prior[k // 2] if k % 2 == 0 else 120.0 for k in tr])
         _, _, _, lag64, beats64, nb64 = eng.tempo_segments_dev(batch.audio, t_off[tr], t_len[tr].astype(np.int32), bpm,
                                                                _tempo.IBI_HOP_LENGTH, sr)
-        hn = eng.to_host(nb64)
+        hn = _engine.check_beat_counts(eng.to_host(nb64))
         mb = int(hn.max()) if len(hn) else 0
         hb = eng.to_host(beats64[:, : max(mb, 1)])
         per_track = {}

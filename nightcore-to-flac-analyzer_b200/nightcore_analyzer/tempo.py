@@ -65,7 +65,7 @@ def _tempo_windows(windows: List[AudioWindow], start_bpm: float) -> List[Optiona
             audio, seg_off, seg_len = eng.pack([w.audio for w in ws])
         bpm = np.full(len(ws), float(start_bpm), dtype=np.float64)
         _, _, _, lag, _, n_beats = eng.tempo_segments_dev(audio, seg_off, seg_len, bpm, HOP_LENGTH, sr)
-        hl, hn = lag.cpu().numpy(), n_beats.cpu().numpy()
+        hl, hn = lag.cpu().numpy(), _engine.check_beat_counts(n_beats.cpu().numpy())
         for j, i in enumerate(idxs):
             results[i] = _consensus(int(hl[j]), int(hn[j]), sr, HOP_LENGTH)
     return results

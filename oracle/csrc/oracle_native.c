@@ -5,6 +5,7 @@
  *
  *  orc_local_score  : librosa.beat.__beat_local_score, static tempo  (SURVEY Appendix A.4; tempo.py:45,159)
  *  orc_beat_dp      : librosa.beat.__beat_track_dp                    (SURVEY Appendix A.4)
+ *  orc_beat_dp_pen  : the same DP on a given penalty table, with per-frame predecessor margins
  *  orc_bootstrap    : numpy Generator(PCG64).choice(..., replace=True) + median, the loop of
  *                     consensus.py:259-262 / :304-307 / pitch.py:145-148 (SURVEY §4 RNG KATs)
  */
@@ -27,7 +28,12 @@ void orc_local_score(const double *onset, int64_t N, const double *window, int64
     }
 }
 
-void orc_beat_dp(const double *ls, int64_t N, double fpb, double tightness, int64_t *backlink, double *cumscore) {
+/* pen == NULL: the transition penalty is tightness·(log(d) − log(fpb))², as librosa computes it; otherwise it is read
+ * from the table pen[d − near], d = near .. far (a caller that wants another machine's log).  margin != NULL receives,
+ * per frame, (best − second best) / max(|best|, |second best|) over its candidate predecessors (+inf with fewer than
+ * two candidates, 0 on an exact tie). */
+static void beat_dp(const double *ls, int64_t N, double fpb, double tightness, const double *pen, int64_t *backlink,
+                    double *cumscore, double *margin) {
     double mx = ls[0];
     for (int64_t i = 1; i < N; ++i)
         if (ls[i] > mx) mx = ls[i];
@@ -39,15 +45,31 @@ void orc_beat_dp(const double *ls, int64_t N, double fpb, double tightness, int6
     const int64_t far = (int64_t)(2.0 * fpb);
     const double logf = log(fpb);
     for (int64_t i = 0; i < N; ++i) {
-        double best = -INFINITY;
+        double best = -INFINITY, second = -INFINITY;
         int64_t bl = -1;
         for (int64_t loc = i - near; loc > i - far - 1; --loc) {
             if (loc < 0) break;
-            double d = log((double)(i - loc)) - logf;
-            double score = cumscore[loc] - tightness * (d * d);
+            double score;
+            if (pen) {
+                score = cumscore[loc] - pen[i - loc - near];
+            } else {
+                double d = log((double)(i - loc)) - logf;
+                score = cumscore[loc] - tightness * (d * d);
+            }
             if (score > best) {
+                second = best;
                 best = score;
                 bl = loc;
+            } else if (score > second) {
+                second = score;
+            }
+        }
+        if (margin) {
+            if (second == -INFINITY) {
+                margin[i] = INFINITY;
+            } else {
+                double s = fabs(best) > fabs(second) ? fabs(best) : fabs(second);
+                margin[i] = (best == second) ? 0.0 : (best - second) / s;
             }
         }
         cumscore[i] = (bl >= 0) ? ls[i] + best : ls[i];
@@ -58,6 +80,16 @@ void orc_beat_dp(const double *ls, int64_t N, double fpb, double tightness, int6
             first_beat = 0;
         }
     }
+}
+
+void orc_beat_dp(const double *ls, int64_t N, double fpb, double tightness, int64_t *backlink, double *cumscore) {
+    beat_dp(ls, N, fpb, tightness, NULL, backlink, cumscore, NULL);
+}
+
+/* orc_beat_dp with the penalty table pen[d − near] (NULL: librosa's log form) and the optional per-frame margin */
+void orc_beat_dp_pen(const double *ls, int64_t N, double fpb, double tightness, const double *pen, int64_t *backlink,
+                     double *cumscore, double *margin) {
+    beat_dp(ls, N, fpb, tightness, pen, backlink, cumscore, margin);
 }
 
 /* ---- PCG64 (numpy): 128-bit LCG step, then XSL-RR output of the new state ---- */

@@ -277,13 +277,33 @@ def _beat_local_score(onset_norm: np.ndarray, fpb: float) -> np.ndarray:
 def beat_track_frames(onset_envelope: np.ndarray, bpm: float, sr: float = 22050, hop_length: int = 512,
                       tightness: float = 100.0, trim: bool = True, return_debug: bool = False):
     """librosa.beat.__beat_tracker with a given bpm (Appendix A.4): frames of the detected beats."""
-    from . import native
     onset = np.asarray(onset_envelope, dtype=np.float64)
     fpb = float(np.round((float(sr) / hop_length) * 60.0 / bpm))
     norm = onset.std(ddof=1)
     onset_norm = onset / (norm + tiny(np.float64(0)))
-    localscore = _beat_local_score(onset_norm, fpb)
-    backlink, cumscore = native.beat_dp(localscore, fpb, tightness)
+    out, debug = beat_track_from_norm(onset_norm, fpb, tightness=tightness, trim=trim)
+    return (out, debug) if return_debug else out
+
+
+def beat_track_from_norm(onset_norm: np.ndarray, fpb: float, window=None, pen=None, tightness: float = 100.0,
+                         trim: bool = True):
+    """The chain of beat_track_frames after the normalisation: local score → DP → last beat → backtrack → trim.
+
+    ``window`` (2·fpb + 1 taps) and ``pen`` (the transition penalty tightness·ln²(d / fpb) for d = round(fpb/2) .. 2·fpb)
+    replace the values this module would compute, so that the chain can run on another machine's float64 exp and log.
+    → (beat frames, debug dict: localscore, cumscore, backlink, tail, threshold, fpb, median of the local-maximum
+    scores, margin = each frame's best-versus-second predecessor score gap, relative, pen = the penalty table used)."""
+    from . import native
+    fpb = float(fpb)
+    if window is None:
+        localscore = _beat_local_score(onset_norm, fpb)
+    else:
+        localscore = native.local_score(onset_norm, window, len(window))
+    backlink, cumscore, margin = native.beat_dp_pen(localscore, fpb, tightness, pen)
+    if pen is None:           # the table the C DP computed: tightness·(log(d) − log(fpb))² with the same C library log
+        logf = math.log(fpb)
+        pen = np.array([tightness * ((math.log(d) - logf) * (math.log(d) - logf))
+                        for d in range(int(np.round(fpb / 2.0)), int(2.0 * fpb) + 1)])
     # last beat
     mask = localmax(cumscore)
     if mask.any():
@@ -298,7 +318,7 @@ def beat_track_frames(onset_envelope: np.ndarray, bpm: float, sr: float = 22050,
             tail = n
             break
         n -= 1
-    beats = np.zeros(len(onset), dtype=bool)
+    beats = np.zeros(len(onset_norm), dtype=bool)
     n = tail
     while n >= 0:
         beats[n] = True
@@ -316,10 +336,8 @@ def beat_track_frames(onset_envelope: np.ndarray, bpm: float, sr: float = 22050,
         beats[n] = False
         n -= 1
     out = np.flatnonzero(beats)
-    if return_debug:
-        return out, dict(localscore=localscore, cumscore=cumscore, backlink=backlink, tail=tail,
-                         threshold=threshold, fpb=fpb)
-    return out
+    return out, dict(localscore=localscore, cumscore=cumscore, backlink=backlink, tail=tail, threshold=threshold,
+                     fpb=fpb, median=med, margin=margin, pen=pen)
 
 
 def beat_track(onset_envelope: np.ndarray, sr: float = 22050, hop_length: int = 512, start_bpm: float = 120.0):

@@ -34,10 +34,11 @@ def lib():
         ip = ctypes.POINTER(ctypes.c_int64)
         _lib.orc_local_score.argtypes = [dp, ctypes.c_int64, dp, ctypes.c_int64, dp]
         _lib.orc_beat_dp.argtypes = [dp, ctypes.c_int64, ctypes.c_double, ctypes.c_double, ip, dp]
+        _lib.orc_beat_dp_pen.argtypes = [dp, ctypes.c_int64, ctypes.c_double, ctypes.c_double, dp, ip, dp, dp]
         _lib.orc_bootstrap.argtypes = [dp, ctypes.c_int, dp, ctypes.c_int, ctypes.c_int] + [ctypes.c_uint64] * 4 + [
             dp, ctypes.POINTER(ctypes.c_int32)]
         _lib.orc_pcg64_raw.argtypes = [ctypes.c_uint64] * 4 + [ctypes.c_int, ctypes.POINTER(ctypes.c_uint64)]
-        for f in (_lib.orc_local_score, _lib.orc_beat_dp, _lib.orc_bootstrap, _lib.orc_pcg64_raw):
+        for f in (_lib.orc_local_score, _lib.orc_beat_dp, _lib.orc_beat_dp_pen, _lib.orc_bootstrap, _lib.orc_pcg64_raw):
             f.restype = None
     return _lib
 
@@ -62,6 +63,24 @@ def beat_dp(localscore: np.ndarray, fpb: float, tightness: float):
     lib().orc_beat_dp(_dp(localscore), n, float(fpb), float(tightness),
                       backlink.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), _dp(cumscore))
     return backlink, cumscore
+
+
+def beat_dp_pen(localscore: np.ndarray, fpb: float, tightness: float, pen=None):
+    """beat_dp with the transition penalty read from pen[d − near], d = near .. far (None: librosa's log form)
+    → (backlink, cumscore, margin): margin[i] = (best − second best) / max(|best|, |second|) over frame i's candidate
+    predecessors, +inf with fewer than two, 0 on an exact tie."""
+    localscore = np.ascontiguousarray(localscore, dtype=np.float64)
+    n = len(localscore)
+    backlink = np.empty(n, dtype=np.int64)
+    cumscore = np.empty(n, dtype=np.float64)
+    margin = np.empty(n, dtype=np.float64)
+    if pen is not None:
+        near, far = int(np.round(fpb / 2.0)), int(2.0 * fpb)
+        pen = np.ascontiguousarray(pen, dtype=np.float64)
+        assert len(pen) == far - near + 1, (len(pen), near, far)
+    lib().orc_beat_dp_pen(_dp(localscore), n, float(fpb), float(tightness), None if pen is None else _dp(pen),
+                          backlink.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), _dp(cumscore), _dp(margin))
+    return backlink, cumscore, margin
 
 
 def pcg64_state(seed: int):

@@ -170,6 +170,32 @@ def test_beat_dp_monotone_argmax_equals_full_scan():
     assert total_mono < 0.6 * total_full                  # and it is much less work (≈ 5x at hop-64 sizes)
 
 
+def test_beat_spacing_bounds_the_beat_count():
+    """Every predecessor lies at least round(lag / 2) frames back, so consecutive beats are at least that far apart and
+    an envelope of N frames has at most N // round(k_min / 2) + 2 beats for every lag >= k_min, the smallest lag the
+    tempogram can return (bpm < 320).  That is Engine.max_beats_for, the row size of the beat buffer: with it the
+    kernel's overflow flag (a count of −1) cannot be reached from the pipeline.  Checked on the oracle for every lag
+    from k_min to k_min + 40 and a geometric sample up to the tempogram's largest lag, at hops 64, 96 and 512."""
+    import os
+    import __graft_entry__ as ge
+    if not os.path.exists(ge.LIB):
+        ge._build_native()
+    from nightcore_analyzer._engine import Engine
+    from oracle import librosa_restated as lr
+    sr = 22050
+    for hop in (64, 96, 512):
+        W = int(np.floor(8.0 * sr / hop))
+        k_min = next(k for k in range(1, W) if 60.0 * sr / (hop * k) < 320.0)
+        lags = sorted(set(range(k_min, k_min + 41)) | {int(v) for v in np.geomspace(k_min + 41, W, 8)})
+        assert lags[-1] == W
+        for lag in lags:
+            n = 3000 + lag % 7
+            env = np.random.default_rng(hop + lag).exponential(1.0, n).astype(np.float32)
+            beats = lr.beat_track_frames(env, 60.0 * sr / (hop * float(lag)), sr, hop)
+            assert len(beats) >= 2 and np.all(np.diff(beats) >= int(np.round(lag / 2.0))), (hop, lag)
+            assert len(beats) <= Engine.max_beats_for(n, hop, sr), (hop, lag, len(beats))
+
+
 def test_xcorr_block_decomposition_identity():
     """xcorr.cu: with stride = win // 4 the candidate at position j·stride is B blocks j..j+3 (+ a tail of win − 4·stride
     samples): dot(wa, wb_j) = D[0][j] + D[1][j+1] + D[2][j+2] + D[3][j+3] + tail, ‖wb_j‖² = S[j] + … + S[j+3] + tail."""
